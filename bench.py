@@ -2,6 +2,7 @@
 """bench.py -- samples/sec of fwd + bwd (+ fused Adagrad update) of the embedding + FM / cross layer.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2|cfg3|cfg5] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic Criteo-shaped input
 (BASELINE.json configs[1] by default: 26 sparse + 13 dense fields, 10 M rows, K = 16, B = 65 536,
@@ -17,6 +18,11 @@ embeddings emitted to / upstream gradients consumed from the DNN side):
   cpu_baseline / --impl reference
             the PyTorch-CPU op-by-op restatement of the reference's TF graph
             (oracle/torch_restatement.py; TF 1.x itself cannot be installed here) on the host cores.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step handed its caller (logits, first-order
+and FM terms, embeddings, the cross output) and a sample of the table state it left behind, one DIR/<name>.npy
+per array (see dump_outputs).  Inputs and initial tables depend on the arguments only, so two builds run with
+the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -38,7 +44,7 @@ LR = 0.05
 def parse_args():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=200)
+    p.add_argument("--steps", type=int, default=200, help="timed steps (each timed loop runs exactly this many)")
     p.add_argument("--warmup", type=int, default=10)
     p.add_argument("--impl", default="b200", choices=["b200", "reference"])
     p.add_argument("--workload", default="cfg2", choices=["cfg2", "cfg3", "cfg4", "cfg5"],
@@ -63,7 +69,15 @@ def parse_args():
     p.add_argument("--feed", default="columns", choices=["columns", "resolved"],
                    help="e2e host format: one column per feature (the reference's input_fn form) or the [B,F] pair")
     p.add_argument("--cpu-seconds", type=float, default=12.0)
+    p.add_argument("--dump-outputs", default="", metavar="DIR",
+                   help="after the timed steps, write the last timed step's outputs as DIR/<name>.npy "
+                        "(float32, at most 64 MB in all; large arrays as a fixed-seed sample), replacing "
+                        "any .npy files DIR held")
     args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        p.error("--dump-outputs writes what the B200 path computed: it needs --impl b200")
     if args.strong:                        # per-GPU batch = global batch / ranks; everything below sees a per-GPU batch
         full = args.batch or dir_synth_batch(args.workload)
         if full % max(args.gpus, 1):
@@ -337,6 +351,12 @@ def run_b200(args):
         else:
             layer.presort(devs[nxt][0], devs[nxt][1], handle=handles[nxt], fork=False, after=ready_events.get(nxt))
 
+    # --dump-outputs: the outputs of the latest step of each (captured?, slot, micro-batch).  A graph replay rewrites
+    # the tensors its capture produced, so those are kept apart from the ones an eager step of the same slot makes.
+    # They are kept detached: holding a step's autograd graph would keep its AccumulateGrad nodes, bound to the
+    # stream they were created on, alive into the next capture and invalidate it.
+    produced = {} if args.dump_outputs else None
+
     def model(slot, x=None):
         if x is None:
             idx, val, y = devs[slot]
@@ -348,11 +368,18 @@ def run_b200(args):
         with torch.no_grad():
             logits = first + fm
             g = torch.sigmoid(logits).sub_(y.unsqueeze(1))          # SUM-reduced CE: no 1/B (deepFM.py:72)
+        if produced is not None:
+            produced[(getattr(layer, "capturing", False), slot, x)] = {
+                "logits": logits, "first_order": first.detach(), "fm": fm.detach(), "embeddings": emb.detach()}
         return first, fm, emb, g, up, logits
 
     def backward(first, fm, emb, g, up):
         if cross is not None:
             xL = cross(emb)
+            if produced is not None:
+                for out in produced.values():        # the step whose embeddings these are (same storage)
+                    if out["embeddings"].data_ptr() == emb.data_ptr():
+                        out["cross_out"] = xL.detach()
             torch.autograd.backward((first, fm, xL), (g, g, up))
         elif emit:
             torch.autograd.backward((first, fm, emb), (g, g, up))
@@ -524,6 +551,12 @@ def run_b200(args):
     ms = float(t.item())
     ms_per_step = ms / args.steps
     value = B * world * args.steps / (ms * 1e-3)
+    if args.dump_outputs:
+        if rank == 0:
+            last = (cursor[0] - 1) % R             # the slot the last timed step ran on
+            halves = [None] if micro == 1 else [0, 1]
+            dump_outputs(args.dump_outputs, [produced[(use_graph, last, x)] for x in halves], layer, cross)
+        barrier()                                  # the other ranks' next steps hold the device-side rows barrier
 
     # ---------------- e2e: pinned host inputs, H2D + D2H inside the timed region ---------------
     e2e = None
@@ -733,6 +766,69 @@ def run_b200(args):
     if rank == 0:
         sys.stdout.flush()
         print(json.dumps(line), flush=True)
+
+
+DUMP_SEED = 1239
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, outs, layer, cross):
+    """Write one step's outputs (`outs`: the step's micro-batches in order, dicts of device tensors) and the layer's
+    state after it as path/<name>.npy, float32; sampled positions as float64 `*_index` arrays.
+
+    Per sample: logits, first_order, fm on up to 65 536 samples; embeddings and cross_out (the DCN cross output) on up
+    to 4 MB worth of samples.  State: table, accumulator, linear, linear_accumulator on up to 262 144 rows of this
+    rank's table, bias, and cross_w_grad_sum / cross_b_grad_sum: the cross parameters' .grad, which nothing zeroes,
+    so the sum over every step run so far (warm-up and capture included).  Samples are drawn from a fixed seed, so two
+    runs with the same arguments write the same positions.  .npy files already in `path` are removed first: the
+    directory holds this run's arrays only."""
+    import numpy as np
+    import torch
+
+    rng = np.random.default_rng(DUMP_SEED)
+
+    def pick(n, k):
+        return np.sort(rng.choice(n, size=min(n, k), replace=False))
+
+    def rows_of(t, index):
+        return t.index_select(0, torch.as_tensor(index, device=t.device)).cpu().numpy().astype(np.float32)
+
+    step = {k: torch.cat([o[k] for o in outs]) for k in outs[0]}
+    B = step["logits"].shape[0]
+    arrays = {}
+    s = pick(B, 1 << 16)
+    arrays["sample_index"] = s.astype(np.float64)
+    for k in ("logits", "first_order", "fm"):
+        arrays[k] = rows_of(step[k].reshape(B), s)
+    if step["embeddings"].numel():
+        e = pick(B, max(1, (4 << 20) // (4 * step["embeddings"].shape[1])))
+        arrays["embedding_sample_index"] = e.astype(np.float64)
+        for k in ("embeddings", "cross_out"):
+            if k in step:
+                arrays[k] = rows_of(step[k].reshape(B, -1), e)
+    n = layer.plan.n_local if hasattr(layer, "plan") else layer.n_rows
+    r = pick(n, 1 << 18)
+    arrays["table_row_index"] = r.astype(np.float64)
+    for k, t in (("table", layer.table), ("accumulator", layer.accum), ("linear", layer.w1),
+                 ("linear_accumulator", layer.w1_accum)):
+        if t is not None:
+            arrays[k] = rows_of(t, r)
+    arrays["bias"] = layer.bias.detach().cpu().numpy().astype(np.float32)
+    if cross is not None:
+        for k in ("cross_w", "cross_b"):
+            grad = getattr(cross, k).grad
+            if grad is not None:
+                arrays[k + "_grad_sum"] = grad.cpu().numpy().astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes (limit %d)" % (total, DUMP_MAX_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for f in os.listdir(path):
+        if f.endswith(".npy"):
+            os.remove(os.path.join(path, f))
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+    print("bench.py: wrote %d arrays (%.1f MB) to %s" % (len(arrays), total / 1e6, path), file=sys.stderr)
 
 
 def time_sharded_calls(pkg, layer, dev_set, up, B, barrier, iters=20):
