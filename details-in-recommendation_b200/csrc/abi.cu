@@ -1,18 +1,9 @@
 // Library-wide state of libdir_b200.so: version, thread-local error text, launch counter.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace dir {
 thread_local char g_err[512] = "";
 std::atomic<uint64_t> g_launches{0};
-int tune() {
-  static const int t = [] {
-    const char* e = getenv("DIR_B200_TUNE");
-    return e ? atoi(e) : 0;
-  }();
-  return t;
-}
 }  // namespace dir
 
 extern "C" int dir_version(void) { return 100; }  // 0.1.0

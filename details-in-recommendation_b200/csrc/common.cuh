@@ -31,8 +31,6 @@ inline int launched(const char* what, int n = 1) {
   return 0;
 }
 
-int tune();  // DIR_B200_TUNE experiment bits, read once
-
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
@@ -65,18 +63,6 @@ __device__ __forceinline__ uint64_t policy_evict_last() {
 __device__ __forceinline__ float4 ldg_hint(const float* p, uint64_t pol) {
   float4 r;
   asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
-               : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w)
-               : "l"(p), "l"(pol));
-  return r;
-}
-// The same with the L2 fill limited to the 64 bytes around the address (.L2::64B).  By default a miss brings the whole
-// 128-byte line in from HBM, so a random gather of a 64-byte piece moves twice its bytes; with the hint the traffic
-// halves (tools/gather_probe.cu: 120 -> 60 bytes of DRAM traffic per 64-byte lookup) -- and the time does not
-// (86.6 -> 82.9 us for 4.2 M lookups): HBM serves about 50 random accesses per nanosecond whatever their size.
-// Experiment only (DIR_B200_TUNE bit 2048).
-__device__ __forceinline__ float4 ldg_hint64(const float* p, uint64_t pol) {
-  float4 r;
-  asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.L2::64B.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
                : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w)
                : "l"(p), "l"(pol));
   return r;

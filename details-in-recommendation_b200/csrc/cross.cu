@@ -427,39 +427,6 @@ cross_bwd_dw_kernel(const float* __restrict__ x0g, const float* __restrict__ alp
   }
 }
 
-// pass 3: fixed-order combine.  thread = one column c.
-__global__ void __launch_bounds__(256)
-cross_bwd_finish_kernel(const float* __restrict__ wg, const float* __restrict__ bg,
-                        const float* __restrict__ Dpart, const float* __restrict__ dypart,
-                        const float* __restrict__ dwpart, int G1, int G2, int d, int L,
-                        float* __restrict__ dw, float* __restrict__ db) {
-  extern __shared__ float sDl[];  // [L] sum_b ds_l
-  if (threadIdx.x < L) {
-    float t = 0.f;
-    for (int g = 0; g < G1; ++g) t += Dpart[(int64_t)g * L + threadIdx.x];
-    sDl[threadIdx.x] = t;
-  }
-  __syncthreads();
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c >= d) return;
-  float sumdy = 0.f;
-  for (int g = 0; g < G1; ++g) sumdy += dypart[(int64_t)g * d + c];
-  // db_l = sum dy + sum_{j>l} w_j D_j ; walk l downwards carrying the tail
-  float tail = 0.f;
-  for (int l = L - 1; l >= 0; --l) {
-    db[l * d + c] = sumdy + tail;
-    tail = fmaf(wg[l * d + c], sDl[l], tail);
-  }
-  // dw_l = sum alpha_l x0 + beta_l D_l ; beta_l = sum_{j<l} b_j
-  float beta = 0.f;
-  for (int l = 0; l < L; ++l) {
-    float t = 0.f;
-    for (int g = 0; g < G2; ++g) t += dwpart[((int64_t)g * L + l) * d + c];
-    dw[l * d + c] = fmaf(beta, sDl[l], t);
-    beta += bg[l * d + c];
-  }
-}
-
 // ------------------------------------------------------------------------------ fused backward (L <= 8)
 // One pass over x0 and dy.  A CTA walks tiles of kTS samples:
 //   phase A  one warp per sample: a = dy . x0, p_l (saved by the forward, or recomputed), the two
@@ -1070,7 +1037,7 @@ extern "C" int dir_cross_bwd(const float* x0, const float* cross_w, const float*
     return fail(DIR_EINVAL, "cross_bwd: 16-byte alignment required when d % 4 == 0");
   CrossBwdWs w = cross_carve(workspace, B, d, L);
   if (workspace_bytes < w.total) return fail(DIR_ENOMEM, "cross_bwd: workspace too small");
-  if (L <= 8 && !(tune() & 1024) && sh.vec == 4) {  // DIR_B200_TUNE bit 1024: the tiled kernel, for A/B runs
+  if (L <= 8 && sh.vec == 4) {
     // per-warp rings: needs the batch sums of one warp in registers and at least a two-slot ring in shared memory
     const int LT = (L + 1) & ~1;
     const size_t fixed = ((size_t)L * (4 * sh.npl * 32) + kCrossWarps * 32 + 32 + kCrossWarps) * 4;

@@ -16,8 +16,7 @@
 //
 // Reference: TF autodiff + optimizer.minimize behind models/DeepFM/deepFM.py:230-241
 // (SURVEY.md rows A8/A9).
-#include <cub/device/device_radix_sort.cuh>
-#include <cub/device/dispatch/dispatch_radix_sort.cuh>
+#include <type_traits>
 
 #include "common.cuh"
 #include "keys.cuh"
@@ -35,10 +34,8 @@ constexpr int kOneRowCtasMax = 444;  // CTAs of the one-row column-sum kernel (t
 struct BwdWorkspace {
   uint32_t* keys;      // [n] sorted global rows
   uint32_t* pos;       // [n] lookup position b*F+f of each sorted entry
-  uint32_t* pos_in;    // [n] iota
-  void* cub_temp;
-  size_t cub_bytes;
-  uint32_t* alt_keys;   // [n] the other half of the radix sort's ping-pong (pos_in is the values' other half)
+  uint32_t* pos_in;    // [n] the other half of the radix sort's ping-pong for the values
+  uint32_t* alt_keys;  // [n] the other half of the radix sort's ping-pong for the keys
   uint32_t* radix_hist; // radix_hist_bytes(n)
   float* part;         // [nchunks][2][K]
   float* part1;        // [nchunks][2]
@@ -49,60 +46,6 @@ struct BwdWorkspace {
   double* onerow_part; // [296][64][K + 4] fp64 partial column sums
   size_t total;
 };
-
-// cub's onesweep with a smaller tile than its sm_90+ default (384 threads x 23 items = 8832 pairs):
-// at 2.5 M pairs the default gives 290 tiles, < 2 per SM, and each pass is latency-bound.
-template <int THREADS, int ITEMS>
-struct SmallTileHub {
-  using Base = cub::detail::radix::policy_hub<uint32_t, uint32_t, int>;
-  struct Policy300 : cub::ChainedPolicy<300, Policy300, Policy300> {
-    static constexpr bool ONESWEEP = true;
-    static constexpr int ONESWEEP_RADIX_BITS = 8;
-    using HistogramPolicy = typename Base::Policy900::HistogramPolicy;
-    using ExclusiveSumPolicy = typename Base::Policy900::ExclusiveSumPolicy;
-    using OnesweepPolicy =
-        cub::AgentRadixSortOnesweepPolicy<THREADS, ITEMS, uint32_t, 1, cub::RADIX_RANK_MATCH_EARLY_COUNTS_ANY,
-                                          cub::BLOCK_SCAN_RAKING_MEMOIZE, cub::RADIX_SORT_STORE_DIRECT, 8>;
-    using ScanPolicy = typename Base::Policy900::ScanPolicy;
-    using DownsweepPolicy = typename Base::Policy900::DownsweepPolicy;
-    using AltDownsweepPolicy = typename Base::Policy900::AltDownsweepPolicy;
-    using UpsweepPolicy = typename Base::Policy900::UpsweepPolicy;
-    using AltUpsweepPolicy = typename Base::Policy900::AltUpsweepPolicy;
-    using SingleTilePolicy = typename Base::Policy900::SingleTilePolicy;
-    using SegmentedPolicy = typename Base::Policy900::SegmentedPolicy;
-    using AltSegmentedPolicy = typename Base::Policy900::AltSegmentedPolicy;
-  };
-  using MaxPolicy = Policy300;
-};
-
-template <class Hub>
-static cudaError_t sort_pairs_hub(void* temp, size_t& bytes, const uint32_t* kin, uint32_t* kout,
-                                  const uint32_t* vin, uint32_t* vout, int n, int end_bit, cudaStream_t st) {
-  cub::DoubleBuffer<uint32_t> dk(const_cast<uint32_t*>(kin), kout);
-  cub::DoubleBuffer<uint32_t> dv(const_cast<uint32_t*>(vin), vout);
-  return cub::DispatchRadixSort<false, uint32_t, uint32_t, int, Hub>::Dispatch(temp, bytes, dk, dv, n, 0, end_bit,
-                                                                              false, st);
-}
-
-static cudaError_t sort_pairs(void* temp, size_t& bytes, const uint32_t* kin, uint32_t* kout,
-                              const uint32_t* vin, uint32_t* vout, int n, int end_bit, cudaStream_t st,
-                              int variant) {
-  if (variant == 1) return sort_pairs_hub<SmallTileHub<256, 8>>(temp, bytes, kin, kout, vin, vout, n, end_bit, st);
-  if (variant == 2) return sort_pairs_hub<SmallTileHub<384, 12>>(temp, bytes, kin, kout, vin, vout, n, end_bit, st);
-  if (variant == 3) return sort_pairs_hub<SmallTileHub<512, 8>>(temp, bytes, kin, kout, vin, vout, n, end_bit, st);
-  return cub::DeviceRadixSort::SortPairs(temp, bytes, kin, kout, vin, vout, n, 0, end_bit, st);
-}
-
-static int sort_variant() { return (tune() >> 5) & 3; }  // DIR_B200_TUNE bits 32, 64
-
-static size_t cub_temp_bytes(int64_t n) {
-  size_t bytes = 0;
-  sort_pairs(nullptr, bytes, nullptr, nullptr, nullptr, nullptr, (int)n, 32, (cudaStream_t)0, sort_variant());
-  cudaGetLastError();  // a size query on a box without a GPU leaves an error behind
-  // onesweep needs ~ (n/ (items per tile) + digits*passes) counters; keep a generous floor
-  const size_t floor_bytes = (size_t)n / 8 + (1u << 20);
-  return bytes > floor_bytes ? bytes : floor_bytes;
-}
 
 static BwdWorkspace carve(void* base, int64_t n, int K) {
   BwdWorkspace w;
@@ -117,8 +60,6 @@ static BwdWorkspace carve(void* base, int64_t n, int K) {
   w.keys = reinterpret_cast<uint32_t*>(take((size_t)n * 4));
   w.pos = reinterpret_cast<uint32_t*>(take((size_t)n * 4));
   w.pos_in = reinterpret_cast<uint32_t*>(take((size_t)n * 4));
-  w.cub_bytes = cub_temp_bytes(n);
-  w.cub_temp = take(w.cub_bytes);
   w.alt_keys = reinterpret_cast<uint32_t*>(take((size_t)n * 4));
   w.radix_hist = reinterpret_cast<uint32_t*>(take(radix_hist_bytes(n)));
   // everything whose size does not depend on K comes first: the sort step carves with a dummy K
@@ -133,73 +74,64 @@ static BwdWorkspace carve(void* base, int64_t n, int K) {
   return w;
 }
 
-__global__ void iota_kernel(uint32_t* out, int64_t n, uint32_t* zero2, unsigned long long* zero1) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = (uint32_t)i;
-  if (i == 0) {
-    *zero2 = 0;
-    *zero1 = 0ull;
-  }
-}
-
+// Every field has a default, so each entry point names only the fields of its own mode.
 struct BwdArgs {
-  float* table;
-  float* accum;
-  int64_t row_stride;
-  float* lin;
-  float* lin_accum;
-  int64_t lin_stride;
-  const float* val;
-  const float* g_first;
-  const float* g_fm;
-  const float* S;
-  const float* u;
-  const uint32_t* keys;
-  const uint32_t* pos;
-  float* part;
-  float* part1;
-  uint32_t* long_list;
-  uint32_t* long_count;
-  unsigned long long* n_unique;
-  int64_t n;
-  int F;
-  uint32_t pruned_key;  // = n_rows
-  int opt;
-  float lr;
-  uint32_t div_magic;   // position / F == (position * div_magic) >> div_shift for position < 2^31
-  int div_shift;
-  int tune;             // DIR_B200_TUNE experiment bits
-  const int32_t* field_sel;  // sorted entries index the compact [B, n_sel] list of these fields (or NULL)
-  int n_sel;
+  float* table = nullptr;
+  float* accum = nullptr;
+  int64_t row_stride = 0;
+  float* lin = nullptr;
+  float* lin_accum = nullptr;
+  int64_t lin_stride = 0;
+  const float* val = nullptr;
+  const float* g_first = nullptr;
+  const float* g_fm = nullptr;
+  const float* S = nullptr;
+  const float* u = nullptr;
+  const uint32_t* keys = nullptr;
+  const uint32_t* pos = nullptr;
+  float* part = nullptr;
+  float* part1 = nullptr;
+  uint32_t* long_list = nullptr;
+  uint32_t* long_count = nullptr;
+  unsigned long long* n_unique = nullptr;
+  int64_t n = 0;
+  int F = 0;
+  uint32_t pruned_key = 0;  // = n_rows
+  int opt = DIR_OPT_SGD;
+  float lr = 0.f;
+  uint32_t div_magic = 0;   // position / F == (position * div_magic) >> div_shift for position < 2^31
+  int div_shift = 0;
+  const int32_t* field_sel = nullptr;  // sorted entries index the compact [B, n_sel] list of these fields (or NULL)
+  int n_sel = 0;
   // sharded-table modes (see kMode*)
-  int mode;
-  const uint32_t* rowidx;  // kModeEmit: row of `table` (the exchanged unique-row buffer) per sorted entry
-  float* emit;             // kModeEmit: [n_unique, emit_stride] receives (G[K], g1) per run
-  int64_t emit_stride;
-  const float* gbuf;       // kModeGiven: [n, gbuf_stride] per-lookup (G[K], g1), indexed by position
-  int64_t gbuf_stride;
+  int mode = 0;
+  const uint32_t* rowidx = nullptr;  // kModeEmit: row of `table` (the exchanged unique-row buffer) per sorted entry
+  float* emit = nullptr;             // kModeEmit: [n_unique, emit_stride] receives (G[K], g1) per run
+  int64_t emit_stride = 0;
+  const float* gbuf = nullptr;       // kModeGiven: [n, gbuf_stride] per-lookup (G[K], g1), indexed by position
+  int64_t gbuf_stride = 0;
   // kModeEmit straight into the owners' buffers over NVLink (emit_peers != NULL; csrc/shard_peer.cu): distinct
   // row u of segment q (emit_seg[q] <= u < emit_seg[q+1]) is row emit_dst_row + u - emit_seg[q] of the gradient
   // region (emit_byte_off) of the buffer at the peer-mapped address emit_peers[q]; its g1 goes to emit_g1[u]
-  const int64_t* emit_seg;
-  const int64_t* emit_peers;
-  int64_t emit_byte_off;
-  int64_t emit_dst_row;
-  int64_t emit_seg_cap;
-  float* emit_g1;
-  int emit_G;
-  int perm_G, perm_rank;  // > 1: warps take the chunks in an owner-interleaved, rank-rotated order (see chunk_of)
-  int64_t perm_M;
-  int emit_read_key;  // kModeEmit over the table itself: rows are read at the key, sums still go to row uidx of `emit`
+  const int64_t* emit_seg = nullptr;
+  const int64_t* emit_peers = nullptr;
+  int64_t emit_byte_off = 0;
+  int64_t emit_dst_row = 0;
+  int64_t emit_seg_cap = 0;
+  float* emit_g1 = nullptr;
+  int emit_G = 0;
+  int perm_G = 0, perm_rank = 0;  // > 1: warps take the chunks in an owner-interleaved, rank-rotated order (see chunk_of)
+  int64_t perm_M = 0;
+  int emit_read_key = 0;  // kModeEmit over the table itself: rows are read at the key, sums still go to row uidx of `emit`
   // entries actually in the sorted list, read on the device (NULL: n).  `n` then only bounds the launch
   // and lays out the workspace, so a step whose sizes are known on the device alone needs no host read.
-  const int64_t* n_dev;
-  LinOpt lo;
+  const int64_t* n_dev = nullptr;
+  LinOpt lo{};
   // kModeBag (multi-hot bags, embed_bag.cu): sorted payload = entry index j
-  const uint32_t* entry_slot;  // [nnz] slot b*F+f of entry j
-  const float* entry_x;        // [nnz] effective scale w_j / norm(bag)
-  const float* emb;            // [B*F, K] combined embeddings e_s saved by the forward
-  float l1, l2;                // ProximalAdagrad strengths of the table rows
+  const uint32_t* entry_slot = nullptr;  // [nnz] slot b*F+f of entry j
+  const float* entry_x = nullptr;        // [nnz] effective scale w_j / norm(bag)
+  const float* emb = nullptr;            // [B*F, K] combined embeddings e_s saved by the forward
+  float l1 = 0.f, l2 = 0.f;              // ProximalAdagrad strengths of the table rows
 };
 
 __device__ __forceinline__ int64_t entries(const BwdArgs& a) {
@@ -293,8 +225,8 @@ __device__ __forceinline__ void apply_loaded(const BwdArgs& a, uint32_t key, int
 //                           running sum carried from the previous pass.
 //   At the last lookup of a run: the run lies inside the chunk -> update the row right here with the
 //   row / accumulator already in registers; otherwise leave a partial for phase 2 / 3.
-template <int LPR, int MODE, int MINB = 3>
-__global__ void __launch_bounds__(256, MINB) embed_bwd_reduce_kernel(const BwdArgs a) {
+template <int LPR, int MODE>
+__global__ void __launch_bounds__(256, 3) embed_bwd_reduce_kernel(const BwdArgs a) {
   constexpr int K = LPR * 4;
   constexpr int SLOTS = 32 / LPR;             // lookups per pass
   constexpr int PASSES = LPR;                 // passes per tile of 32 lookups
@@ -322,8 +254,7 @@ __global__ void __launch_bounds__(256, MINB) embed_bwd_reduce_kernel(const BwdAr
   // tools/gather_probe.cu); the other half of a `u` line belongs to the neighbouring field of the
   // same sample and is wanted later by some other warp, so `u` lines are asked to stay (evict_last)
   // while row / accumulator lines, read and rewritten exactly once, are asked to leave first.
-  const int tune = a.tune;
-  const uint64_t pol_once = (tune & 8) ? policy_evict_first() : policy_evict_last();
+  const uint64_t pol_once = policy_evict_last();
   const uint64_t pol_row = policy_evict_first();
 
   uint32_t carry_key = kNoKey, last_key = prev_key;
@@ -423,17 +354,15 @@ __global__ void __launch_bounds__(256, MINB) embed_bwd_reduce_kernel(const BwdAr
           if (MODE == kModeGiven) {  // the per-lookup gradient was formed by the requester
             ub[j] = ldg_hint(a.gbuf + (int64_t)p * a.gbuf_stride + sub * 4, pol_once);
           } else {
-            // (DIR_B200_TUNE bit 2048: 64-byte L2 fill for one field's slice of u -- measured slower, the neighbouring
-            // field's slice is no longer left in L2 for the warp that wants it)
-            if (a.u) ub[j] = (tune & 2048) ? ldg_hint64(a.u + (int64_t)p * K + sub * 4, pol_once)
-                                           : ldg_hint(a.u + (int64_t)p * K + sub * 4, pol_once);
+            // (S before u: the other order spills 8 bytes at K = 32 and 64.  A 64-byte L2 fill for one field's slice
+            // of u measured slower: the neighbouring field's slice is no longer left in L2 for the warp that wants it)
             Sb[j] = __ldg(reinterpret_cast<const float4*>(a.S + (int64_t)bb * K) + sub);
+            if (a.u) ub[j] = ldg_hint(a.u + (int64_t)p * K + sub * 4, pol_once);
             if (BAG) {
               T[j] = __ldg(reinterpret_cast<const float4*>(a.emb + (int64_t)p * K) + sub);
             } else {
               // coherent load: this warp may rewrite the row further down
-              T[j] = (tune & 16) ? *(reinterpret_cast<const float4*>(a.table + ro) + sub)
-                                 : ld_hint(a.table + ro + sub * 4, pol_row);
+              T[j] = ld_hint(a.table + ro + sub * 4, pol_row);
             }
           }
           if (!EMIT && (ac[j] & 3) == 1) {
@@ -625,8 +554,7 @@ static int launch_bwd(const BwdArgs& a, int64_t* n_unique_out, cudaStream_t st) 
   const int64_t vchunks = a.perm_G > 1 ? a.perm_M * a.perm_G : nchunks;   // virtual chunks (>= nchunks)
   const unsigned rgrid = (unsigned)((vchunks + 7) / 8);
   if (a.mode == kModeEmit)
-    if (LPR == 4 && (a.tune & 256)) embed_bwd_reduce_kernel<LPR, kModeEmit, 4><<<rgrid, 256, 0, st>>>(a);
-    else embed_bwd_reduce_kernel<LPR, kModeEmit><<<rgrid, 256, 0, st>>>(a);
+    embed_bwd_reduce_kernel<LPR, kModeEmit><<<rgrid, 256, 0, st>>>(a);
   else if (a.mode == kModeGiven)
     embed_bwd_reduce_kernel<LPR, kModeGiven><<<rgrid, 256, 0, st>>>(a);
   else if (a.mode == kModeBag)
@@ -634,8 +562,7 @@ static int launch_bwd(const BwdArgs& a, int64_t* n_unique_out, cudaStream_t st) 
   else if (a.mode == kModeBagEmit)
     embed_bwd_reduce_kernel<LPR, kModeBagEmit><<<rgrid, 256, 0, st>>>(a);
   else
-    if (LPR == 4 && (a.tune & 256)) embed_bwd_reduce_kernel<LPR, kModeLocal, 4><<<rgrid, 256, 0, st>>>(a);
-    else embed_bwd_reduce_kernel<LPR, kModeLocal><<<rgrid, 256, 0, st>>>(a);
+    embed_bwd_reduce_kernel<LPR, kModeLocal><<<rgrid, 256, 0, st>>>(a);
   constexpr int NG = 256 / LPR;
   embed_bwd_finish_kernel<LPR><<<(unsigned)((nchunks + NG - 1) / NG), 256, 0, st>>>(a, n_unique_out);
   return launched("embed_bwd_reduce_update", 2);
@@ -656,30 +583,30 @@ constexpr int kOneRowCtas = kOneRowCtasMax;
 constexpr int kOneRowMax = 64;     // one-row fields per call
 
 struct OneRowArgs {
-  float* table;
-  float* accum;
-  int64_t row_stride;
-  float* lin;
-  float* lin_accum;
-  int64_t lin_stride;
-  const int64_t* idx;
-  const float* val;
-  const int64_t* field_offset;
-  const float* g_first;
-  const float* g_fm;
-  const float* S;
-  const float* u;
-  const int32_t* fields;
-  int64_t B;
-  int F;
-  int opt;
-  float lr;
-  double* part;  // [kOneRowCtas][kOneRowMax][K + 4]
-  int* flags;    // [kOneRowMax] some sample had a surviving lookup
-  unsigned long long* n_unique;
-  LinOpt lo;
-  float clip;    // > 0: tf.clip_by_norm of the field's gradient (its variable has this one row) before the update
-  float l1, l2;  // ProximalAdagrad strengths of the table rows
+  float* table = nullptr;
+  float* accum = nullptr;
+  int64_t row_stride = 0;
+  float* lin = nullptr;
+  float* lin_accum = nullptr;
+  int64_t lin_stride = 0;
+  const int64_t* idx = nullptr;
+  const float* val = nullptr;
+  const int64_t* field_offset = nullptr;
+  const float* g_first = nullptr;
+  const float* g_fm = nullptr;
+  const float* S = nullptr;
+  const float* u = nullptr;
+  const int32_t* fields = nullptr;
+  int64_t B = 0;
+  int F = 0;
+  int opt = DIR_OPT_SGD;
+  float lr = 0.f;
+  double* part = nullptr;  // [kOneRowCtas][kOneRowMax][K + 4]
+  int* flags = nullptr;    // [kOneRowMax] some sample had a surviving lookup
+  unsigned long long* n_unique = nullptr;
+  LinOpt lo{};
+  float clip = 0.f;        // > 0: tf.clip_by_norm of the field's gradient (its variable has this one row) before the update
+  float l1 = 0.f, l2 = 0.f;  // ProximalAdagrad strengths of the table rows
 };
 
 template <int LPR, int P>
@@ -791,21 +718,18 @@ embed_bwd_onerow_kernel(const OneRowArgs a, int f0, int nf) {
   }
 }
 
-// one CTA per one-row field: 32 component lanes x 8 "g-lanes" sum the CTA partials in a fixed order
-template <int LPR>
-__global__ void __launch_bounds__(256) embed_bwd_onerow_finish_kernel(const OneRowArgs a, int G) {
-  constexpr int K = LPR * 4;
+// One-row field j: 32 component lanes x 8 "g-lanes" of the CTA sum the `ctas` CTA partials in a fixed order;
+// tot[c] (c <= K) receives the column sum, rounded to fp32 once.  Every thread of the CTA calls it.
+template <int K>
+__device__ __forceinline__ void onerow_sum(const double* part, int j, int ctas, float* tot) {
   __shared__ double red[8][33];
-  __shared__ float tot[K + 1];
-  const int j = blockIdx.x;
-  if (a.flags[j] == 0) return;  // no surviving lookup: the row is not touched
   const int cx = threadIdx.x & 31, gy = threadIdx.x >> 5;
   for (int c0 = 0; c0 <= K; c0 += 32) {
     const int c = c0 + cx;
     double t = 0.0;
     if (c <= K)
 #pragma unroll 8
-      for (int g = gy; g < G; g += 8) t += __ldg(a.part + ((int64_t)g * kOneRowMax + j) * (K + 4) + c);
+      for (int g = gy; g < ctas; g += 8) t += __ldg(part + ((int64_t)g * kOneRowMax + j) * (K + 4) + c);
     red[gy][cx] = t;
     __syncthreads();
     if (gy == 0 && c <= K) {
@@ -816,6 +740,16 @@ __global__ void __launch_bounds__(256) embed_bwd_onerow_finish_kernel(const OneR
     }
     __syncthreads();
   }
+}
+
+// one CTA per one-row field: the column sum, then the row update
+template <int LPR>
+__global__ void __launch_bounds__(256) embed_bwd_onerow_finish_kernel(const OneRowArgs a, int G) {
+  constexpr int K = LPR * 4;
+  __shared__ float tot[K + 1];
+  const int j = blockIdx.x;
+  if (a.flags[j] == 0) return;  // no surviving lookup: the row is not touched
+  onerow_sum<K>(a.part, j, G, tot);
   if (a.clip > 0.f) {  // values * clip / max(||values||, clip), the row and the linear weight each a variable
     if (threadIdx.x == 0) {
       double sq = 0.0;
@@ -851,12 +785,14 @@ __global__ void __launch_bounds__(256) embed_bwd_onerow_finish_kernel(const OneR
 }
 
 template <int LPR>
-static int launch_onerow(const OneRowArgs& a, int n_fields, cudaStream_t st) {
+static int launch_onerow_partials(const OneRowArgs& a, int n_fields, cudaStream_t st, int* ctas) {
   constexpr int PER = kOneRowPasses * (32 / LPR);
+  constexpr int SLOTS = 32 / LPR;
   const int64_t want = (a.B + 7) / 8;
   const int G = (int)(want < kOneRowCtas ? want : kOneRowCtas);
-  constexpr int SLOTS = 32 / LPR;
   int n = 0;
+  *ctas = G;
+  if (G == 0) return 0;  // an empty batch on this rank: the emit kernel ships zeros, `touched` = 0
   for (int f0 = 0; f0 < n_fields; f0 += PER, ++n) {
     const int nf = n_fields - f0 < PER ? n_fields - f0 : PER;
     switch ((nf + SLOTS - 1) / SLOTS) {
@@ -866,8 +802,15 @@ static int launch_onerow(const OneRowArgs& a, int n_fields, cudaStream_t st) {
       default: embed_bwd_onerow_kernel<LPR, 4><<<G, 256, 0, st>>>(a, f0, nf); break;
     }
   }
-  embed_bwd_onerow_finish_kernel<LPR><<<n_fields, 256, 0, st>>>(a, G);
-  return launched("embed_bwd_onerow", n + 1);
+  return launched("embed_bwd_onerow_partials", n);
+}
+
+template <int LPR>
+static int launch_onerow(const OneRowArgs& a, int n_fields, cudaStream_t st) {
+  int ctas = 0;
+  if (int rc = launch_onerow_partials<LPR>(a, n_fields, st, &ctas)) return rc;
+  embed_bwd_onerow_finish_kernel<LPR><<<n_fields, 256, 0, st>>>(a, ctas);
+  return launched("embed_bwd_onerow");
 }
 
 __global__ void publish_count_kernel(const unsigned long long* src, int64_t* dst) { *dst = (int64_t)*src; }
@@ -881,14 +824,49 @@ static void set_div(BwdArgs& a, int F) {
   a.div_magic = (uint32_t)((((uint64_t)1 << a.div_shift) + (uint64_t)F - 1) / (uint64_t)F);
 }
 
-static int dispatch_bwd(const BwdArgs& a, int K, int64_t* n_unique_out, cudaStream_t st) {
+// The sorted list of n entries that the sort step left in w; an entry's sample is its position / per_sample.
+static void set_sorted(BwdArgs& a, const BwdWorkspace& w, int64_t n, int F, int per_sample) {
+  a.keys = w.keys;
+  a.pos = w.pos;
+  a.part = w.part;
+  a.part1 = w.part1;
+  a.long_list = w.long_list;
+  a.long_count = w.long_count;
+  a.n_unique = w.n_unique;
+  a.n = n;
+  a.F = F;
+  set_div(a, per_sample);
+}
+
+// The emit modes' sums go straight into the owners' buffers of a peer layout (after set_sorted: perm_M needs n).
+static void set_peer_emit(BwdArgs& a, const dir_peer_layout& L, const int64_t* owner_off, float* g1_local) {
+  a.emit_seg = owner_off;
+  a.emit_peers = L.peer_base;
+  a.emit_byte_off = L.off_g;
+  a.emit_dst_row = (int64_t)L.rank * L.seg_cap;
+  a.emit_seg_cap = L.seg_cap;
+  a.emit_g1 = g1_local;
+  a.emit_G = L.G;
+  a.perm_G = L.G;
+  a.perm_rank = L.rank;
+  a.perm_M = ((a.n + kChunk - 1) / kChunk + L.G - 1) / L.G;
+}
+
+// f(std::integral_constant<int, LPR>()) with LPR = K / 4 lanes per K-vector; every caller has checked that K is one
+// of 4, 8, 16, 32, 64.
+template <class Fn>
+static int with_lpr(int K, Fn&& f) {
   switch (K) {
-    case 4: return launch_bwd<1>(a, n_unique_out, st);
-    case 8: return launch_bwd<2>(a, n_unique_out, st);
-    case 16: return launch_bwd<4>(a, n_unique_out, st);
-    case 32: return launch_bwd<8>(a, n_unique_out, st);
-    default: return launch_bwd<16>(a, n_unique_out, st);
+    case 4: return f(std::integral_constant<int, 1>());
+    case 8: return f(std::integral_constant<int, 2>());
+    case 16: return f(std::integral_constant<int, 4>());
+    case 32: return f(std::integral_constant<int, 8>());
+    default: return f(std::integral_constant<int, 16>());
   }
+}
+
+static int dispatch_bwd(const BwdArgs& a, int K, int64_t* n_unique_out, cudaStream_t st) {
+  return with_lpr(K, [&](auto lpr) { return launch_bwd<lpr>(a, n_unique_out, st); });
 }
 
 }  // namespace dir
@@ -911,43 +889,22 @@ extern "C" int dir_embed_bwd_sorted(const void* workspace, int64_t n_lookups,
 
 extern "C" int dir_embed_bwd_sort(const uint32_t* sort_keys, int64_t n_lookups, int64_t n_rows,
                                   void* workspace, size_t workspace_bytes, dir_stream_t stream) {
-  const int64_t n_capacity = n_lookups;
   using namespace dir;
-  if (n_lookups < 0 || n_lookups >= 0x7fffffffLL || n_capacity < n_lookups || n_capacity >= 0x7fffffffLL)
-    return fail(DIR_EINVAL, "embed_bwd_sort: 0 <= n_lookups <= n_capacity < 2^31 required");
+  if (n_lookups < 0 || n_lookups >= 0x7fffffffLL)
+    return fail(DIR_EINVAL, "embed_bwd_sort: 0 <= n_lookups < 2^31 required");
   if (n_rows <= 0 || n_rows >= 0xffffffffLL)
     return fail(DIR_EINVAL, "embed_bwd_sort: 0 < n_rows < 2^32-1 required");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (n_lookups == 0) {
-    if (workspace && n_capacity > 0) {  // a later reduce over 0 entries must still find zeroed counters
-      BwdWorkspace w0 = carve(workspace, n_capacity, 4);
-      if (workspace_bytes < w0.total) return fail(DIR_ENOMEM, "embed_bwd_sort: workspace too small");
-      cudaMemsetAsync(w0.long_count, 0, 16, st);
-    }
-    return 0;
-  }
+  if (n_lookups == 0) return 0;
   if (!sort_keys || !workspace) return fail(DIR_EINVAL, "embed_bwd_sort: null pointer");
   // K only sizes the tail of the workspace; the sort part does not depend on it
-  BwdWorkspace w = carve(workspace, n_capacity, 4);
+  BwdWorkspace w = carve(workspace, n_lookups, 4);
   if (workspace_bytes < w.total) return fail(DIR_ENOMEM, "embed_bwd_sort: workspace too small");
   int end_bit = 1;
   while (end_bit < 32 && (((uint64_t)n_rows) >> end_bit) != 0) ++end_bit;  // n_rows itself is a key
-  if (!(tune() & 512)) {
-    // the hand-written sort (radix.cuh): three small kernels per 8-bit pass, positions implied by the input order
-    const int launches = radix_sort_pairs(sort_keys, n_lookups, end_bit, w.keys, w.pos, w.alt_keys, w.pos_in,
-                                          w.radix_hist, w.long_count, w.n_unique, st);
-    return launched("embed_bwd_sort", launches);
-  }
-  // DIR_B200_TUNE bit 512: cub::DeviceRadixSort, kept as the cross-check / timing baseline
-  const unsigned grid = (unsigned)((n_lookups + 255) / 256);
-  iota_kernel<<<grid, 256, 0, st>>>(w.pos_in, n_lookups, w.long_count, w.n_unique);
-  int rc = launched("embed_bwd_sort/iota");
-  if (rc) return rc;
-  size_t cub_bytes = w.cub_bytes;
-  cudaError_t e = sort_pairs(w.cub_temp, cub_bytes, sort_keys, w.keys, (const uint32_t*)w.pos_in, w.pos,
-                             (int)n_lookups, end_bit, st, sort_variant());
-  if (e != cudaSuccess) return fail(DIR_EIO, "embed_bwd_sort: %s", cudaGetErrorString(e));
-  return launched("embed_bwd_sort", (end_bit + 7) / 8 + 2);
+  // the hand-written sort (radix.cuh): three small kernels per 8-bit pass, positions implied by the input order
+  const int launches = radix_sort_pairs(sort_keys, n_lookups, end_bit, w.keys, w.pos, w.alt_keys, w.pos_in,
+                                        w.radix_hist, w.long_count, w.n_unique, static_cast<cudaStream_t>(stream));
+  return launched("embed_bwd_sort", launches);
 }
 
 namespace dir {
@@ -1004,7 +961,7 @@ extern "C" int dir_shard_keys_sort(const int64_t* feature_index, const float* fe
     return rc;
   const int64_t n = a.n;
   const int64_t n_keys = G > 1 ? a.cap * G : n_rows;  // the pruned key; every other key is below it
-  if (n == 0 || (tune() & 512))  {  // nothing to fuse (or the library sort was asked for): the two calls
+  if (n == 0) {  // nothing to fuse: the two calls
     if (int rc = dir_shard_keys(feature_index, feature_value, field_offset, field_rows, n_rows, B, F, G, field_sel,
                                 n_sel, keys, oob_flag, stream))
       return rc;
@@ -1066,18 +1023,14 @@ extern "C" int dir_embed_bwd_reduce_update(
   if (n == 0) cudaMemsetAsync(w.n_unique, 0, 8, st);  // no sort ran: nobody zeroed the counter
   if (n_onerow > 0) {
     cudaMemsetAsync(w.onerow_flags, 0, kOneRowMax * 4, st);
-    OneRowArgs o{table, accum, row_stride, lin, lin_accum, lin_stride, feature_index, feature_value,
-                 field_offset, g_first, g_fm, S, u, onerow_fields, B, F, optimizer, lr, w.onerow_part,
-                 w.onerow_flags, w.n_unique, lo, 0.f, tl1, tl2};
-    int rc;
-    switch (K) {
-      case 4: rc = launch_onerow<1>(o, n_onerow, st); break;
-      case 8: rc = launch_onerow<2>(o, n_onerow, st); break;
-      case 16: rc = launch_onerow<4>(o, n_onerow, st); break;
-      case 32: rc = launch_onerow<8>(o, n_onerow, st); break;
-      default: rc = launch_onerow<16>(o, n_onerow, st); break;
-    }
-    if (rc) return rc;
+    OneRowArgs o;
+    o.table = table; o.accum = accum; o.row_stride = row_stride;
+    o.lin = lin; o.lin_accum = lin_accum; o.lin_stride = lin_stride; o.lo = lo;
+    o.idx = feature_index; o.val = feature_value; o.field_offset = field_offset; o.fields = onerow_fields;
+    o.g_first = g_first; o.g_fm = g_fm; o.S = S; o.u = u; o.B = B; o.F = F;
+    o.opt = optimizer; o.lr = lr; o.l1 = tl1; o.l2 = tl2;
+    o.part = w.onerow_part; o.flags = w.onerow_flags; o.n_unique = w.n_unique;
+    if (int rc = with_lpr(K, [&](auto lpr) { return launch_onerow<lpr>(o, n_onerow, st); })) return rc;
   }
   if (n == 0) {
     if (n_unique_out) {
@@ -1086,10 +1039,14 @@ extern "C" int dir_embed_bwd_reduce_update(
     }
     return 0;
   }
-  BwdArgs a{table, accum, row_stride, lin, lin_accum, lin_stride, feature_value, g_first, g_fm, S,
-            u, w.keys, w.pos, w.part, w.part1, w.long_list, w.long_count, w.n_unique, n, F,
-            (uint32_t)n_rows, optimizer, lr, 0u, 0, tune(), field_sel, n_sel, kModeLocal, nullptr, nullptr, 0, nullptr, 0, nullptr, nullptr, 0, 0, 0, nullptr, 0, 0, 0, 0, 0, nullptr, lo, nullptr, nullptr, nullptr, tl1, tl2};
-  set_div(a, n_sel);
+  BwdArgs a;
+  set_sorted(a, w, n, F, n_sel);
+  a.mode = kModeLocal;
+  a.table = table; a.accum = accum; a.row_stride = row_stride;
+  a.lin = lin; a.lin_accum = lin_accum; a.lin_stride = lin_stride; a.lo = lo;
+  a.val = feature_value; a.g_first = g_first; a.g_fm = g_fm; a.S = S; a.u = u;
+  a.field_sel = field_sel; a.n_sel = n_sel;
+  a.pruned_key = (uint32_t)n_rows; a.opt = optimizer; a.lr = lr; a.l1 = tl1; a.l2 = tl2;
   return dispatch_bwd(a, K, n_unique_out, st);
 }
 
@@ -1120,16 +1077,15 @@ static int reduce_emit(const char* what, const float* ubuf, int64_t ubuf_stride,
   if (n_keys <= 0 || n_keys >= 0xffffffffLL) return fail(DIR_EINVAL, "%s: 0 < n_keys < 2^32-1 required", what);
   BwdWorkspace w = carve(workspace, n, K);
   if (workspace_bytes < w.total) return fail(DIR_ENOMEM, "%s: workspace too small", what);
-  BwdArgs a{const_cast<float*>(ubuf), nullptr, ubuf_stride, nullptr, nullptr, 0, feature_value, g_first,
-            g_fm, S, u, w.keys, w.pos, w.part, w.part1, w.long_list, w.long_count, w.n_unique, n, F,
-            (uint32_t)n_keys, DIR_OPT_SGD, 0.f, 0u, 0, tune(), field_sel, field_sel ? n_sel : 0, kModeEmit, uidx, gu,
-            gu_stride, nullptr, 0,
-            owner_off, layout ? layout->peer_base : nullptr, layout ? layout->off_g : 0,
-            layout ? (int64_t)layout->rank * layout->seg_cap : 0, layout ? layout->seg_cap : 0, g1_local,
-            layout ? layout->G : 0, layout ? layout->G : 0, layout ? layout->rank : 0,
-            layout ? ((n + kChunk - 1) / kChunk + layout->G - 1) / layout->G : 0, read_key, nullptr,
-            LinOpt{DIR_OPT_SGD, 0.f, 0.f, 0.f, nullptr}, nullptr, nullptr, nullptr};
-  set_div(a, n_sel);
+  BwdArgs a;
+  set_sorted(a, w, n, F, n_sel);
+  a.mode = kModeEmit;
+  a.table = const_cast<float*>(ubuf); a.row_stride = ubuf_stride; a.emit_read_key = read_key;
+  a.val = feature_value; a.g_first = g_first; a.g_fm = g_fm; a.S = S; a.u = u;
+  a.field_sel = field_sel; a.n_sel = n_sel;
+  a.pruned_key = (uint32_t)n_keys; a.rowidx = uidx;
+  a.emit = gu; a.emit_stride = gu_stride;
+  if (layout) set_peer_emit(a, *layout, owner_off, g1_local);
   return dispatch_bwd(a, K, nullptr, static_cast<cudaStream_t>(stream));
 }
 
@@ -1202,10 +1158,13 @@ extern "C" int dir_rows_reduce_update(float* table, float* accum, int64_t row_st
     return fail(DIR_EINVAL, "rows_reduce_update: 0 < n_rows < 2^32-1 required");
   BwdWorkspace w = carve(workspace, n, K);
   if (workspace_bytes < w.total) return fail(DIR_ENOMEM, "rows_reduce_update: workspace too small");
-  BwdArgs a{table, accum, row_stride, lin, lin_accum, lin_stride, nullptr, nullptr, nullptr, nullptr,
-            nullptr, w.keys, w.pos, w.part, w.part1, w.long_list, w.long_count, w.n_unique, n, 1,
-            (uint32_t)n_rows, optimizer, lr, 0u, 0, tune(), nullptr, 0, kModeGiven, nullptr, nullptr, 0, gbuf, gbuf_stride, nullptr, nullptr, 0, 0, 0, nullptr, 0, 0, 0, 0, 0, n_device, lo, nullptr, nullptr, nullptr};
-  set_div(a, 1);
+  BwdArgs a;
+  set_sorted(a, w, n, 1, 1);
+  a.mode = kModeGiven;
+  a.table = table; a.accum = accum; a.row_stride = row_stride;
+  a.lin = lin; a.lin_accum = lin_accum; a.lin_stride = lin_stride; a.lo = lo;
+  a.gbuf = gbuf; a.gbuf_stride = gbuf_stride; a.n_dev = n_device;
+  a.pruned_key = (uint32_t)n_rows; a.opt = optimizer; a.lr = lr;
   return dispatch_bwd(a, K, n_unique_out, static_cast<cudaStream_t>(stream));
 }
 
@@ -1243,11 +1202,14 @@ extern "C" int dir_embed_bag_bwd_reduce_update(
     return fail(DIR_EINVAL, "embed_bag_bwd_reduce_update: table, accum, S, u, emb must be 16-byte aligned");
   BwdWorkspace w = carve(workspace, nnz, K);
   if (workspace_bytes < w.total) return fail(DIR_ENOMEM, "embed_bag_bwd_reduce_update: workspace too small");
-  BwdArgs a{table, accum, row_stride, lin, lin_accum, lin_stride, bag_weight, g_first, g_fm, S,
-            u, w.keys, w.pos, w.part, w.part1, w.long_list, w.long_count, w.n_unique, nnz, F,
-            (uint32_t)n_rows, optimizer, lr, 0u, 0, tune(), nullptr, 0, kModeBag, nullptr, nullptr, 0, nullptr, 0,
-            nullptr, nullptr, 0, 0, 0, nullptr, 0, 0, 0, 0, 0, nullptr, lo, entry_slot, entry_x, emb};
-  set_div(a, F);
+  BwdArgs a;
+  set_sorted(a, w, nnz, F, F);
+  a.mode = kModeBag;
+  a.table = table; a.accum = accum; a.row_stride = row_stride;
+  a.lin = lin; a.lin_accum = lin_accum; a.lin_stride = lin_stride; a.lo = lo;
+  a.val = bag_weight; a.g_first = g_first; a.g_fm = g_fm; a.S = S; a.u = u;
+  a.entry_slot = entry_slot; a.entry_x = entry_x; a.emb = emb;
+  a.pruned_key = (uint32_t)n_rows; a.opt = optimizer; a.lr = lr;
   return dispatch_bwd(a, K, n_unique_out, st);
 }
 
@@ -1278,14 +1240,14 @@ extern "C" int dir_embed_bag_bwd_reduce_emit_to(const dir_peer_layout* layout, c
   if (n_keys <= 0 || n_keys >= 0xffffffffLL) return fail(DIR_EINVAL, "%s: 0 < n_keys < 2^32-1 required", what);
   BwdWorkspace w = carve(workspace, nnz, K);
   if (workspace_bytes < w.total) return fail(DIR_ENOMEM, "%s: workspace too small", what);
-  BwdArgs a{nullptr, nullptr, K, nullptr, nullptr, 0, bag_weight, g_first, g_fm, S,
-            u, w.keys, w.pos, w.part, w.part1, w.long_list, w.long_count, w.n_unique, nnz, F,
-            (uint32_t)n_keys, DIR_OPT_SGD, 0.f, 0u, 0, tune(), nullptr, 0, kModeBagEmit, uidx, nullptr, 0, nullptr, 0,
-            owner_off, layout->peer_base, layout->off_g, (int64_t)layout->rank * layout->seg_cap, layout->seg_cap,
-            g1_local, layout->G, layout->G, layout->rank,
-            ((nnz + kChunk - 1) / kChunk + layout->G - 1) / layout->G, 0, nullptr,
-            LinOpt{DIR_OPT_SGD, 0.f, 0.f, 0.f, nullptr}, entry_slot, entry_x, emb};
-  set_div(a, F);
+  BwdArgs a;
+  set_sorted(a, w, nnz, F, F);
+  a.mode = kModeBagEmit;
+  a.row_stride = K;
+  a.val = bag_weight; a.g_first = g_first; a.g_fm = g_fm; a.S = S; a.u = u;
+  a.entry_slot = entry_slot; a.entry_x = entry_x; a.emb = emb;
+  a.pruned_key = (uint32_t)n_keys; a.rowidx = uidx;
+  set_peer_emit(a, *layout, owner_off, g1_local);
   return dispatch_bwd(a, K, nullptr, static_cast<cudaStream_t>(stream));
 }
 
@@ -1312,53 +1274,15 @@ static OneRowWs onerow_carve(void* base, int K) {
   return w;
 }
 
-template <int LPR>
-static int launch_onerow_partials(const OneRowArgs& a, int n_fields, cudaStream_t st, int* ctas) {
-  constexpr int PER = kOneRowPasses * (32 / LPR);
-  constexpr int SLOTS = 32 / LPR;
-  const int64_t want = (a.B + 7) / 8;
-  const int G = (int)(want < kOneRowCtas ? want : kOneRowCtas);
-  int n = 0;
-  *ctas = G;
-  if (G == 0) return 0;  // an empty batch on this rank: the emit kernel ships zeros, `touched` = 0
-  for (int f0 = 0; f0 < n_fields; f0 += PER, ++n) {
-    const int nf = n_fields - f0 < PER ? n_fields - f0 : PER;
-    switch ((nf + SLOTS - 1) / SLOTS) {
-      case 1: embed_bwd_onerow_kernel<LPR, 1><<<G, 256, 0, st>>>(a, f0, nf); break;
-      case 2: embed_bwd_onerow_kernel<LPR, 2><<<G, 256, 0, st>>>(a, f0, nf); break;
-      case 3: embed_bwd_onerow_kernel<LPR, 3><<<G, 256, 0, st>>>(a, f0, nf); break;
-      default: embed_bwd_onerow_kernel<LPR, 4><<<G, 256, 0, st>>>(a, f0, nf); break;
-    }
-  }
-  return launched("embed_bwd_onerow_partials", n);
-}
-
-// one CTA per one-row field: the CTA partials summed exactly as embed_bwd_onerow_finish_kernel sums them, then
-// the field's (G[K], g1, touched, 0, 0) is stored into dense[rank][j] of EVERY rank's exchange buffer
+// one CTA per one-row field: the column sum of embed_bwd_onerow_finish_kernel, then the field's
+// (G[K], g1, touched, 0, 0) is stored into dense[rank][j] of EVERY rank's exchange buffer
 template <int LPR>
 __global__ void __launch_bounds__(256)
 onerow_emit_to_kernel(const OneRowArgs a, int ctas, const dir_peer_layout L) {
   constexpr int K = LPR * 4;
-  __shared__ double red[8][33];
   __shared__ __align__(16) float tot[K + 4];
   const int j = blockIdx.x;
-  const int cx = threadIdx.x & 31, gy = threadIdx.x >> 5;
-  for (int c0 = 0; c0 <= K; c0 += 32) {
-    const int c = c0 + cx;
-    double t = 0.0;
-    if (c <= K)
-#pragma unroll 8
-      for (int g = gy; g < ctas; g += 8) t += __ldg(a.part + ((int64_t)g * kOneRowMax + j) * (K + 4) + c);
-    red[gy][cx] = t;
-    __syncthreads();
-    if (gy == 0 && c <= K) {
-      double v = 0.0;
-#pragma unroll
-      for (int k = 0; k < 8; ++k) v += red[k][cx];
-      tot[c] = (float)v;
-    }
-    __syncthreads();
-  }
+  onerow_sum<K>(a.part, j, ctas, tot);
   if (threadIdx.x == 0) {
     tot[K + 1] = a.flags[j] != 0 ? 1.f : 0.f;  // some sample of this rank had a surviving lookup
     tot[K + 2] = tot[K + 3] = 0.f;
@@ -1403,23 +1327,17 @@ extern "C" int dir_shard_dense_emit(const dir_peer_layout* layout, const float* 
   if (workspace_bytes < w.total) return fail(DIR_ENOMEM, "shard_dense_emit: workspace too small");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   cudaMemsetAsync(w.flags, 0, kOneRowMax * 4, st);
-  OneRowArgs o{const_cast<float*>(dense_table), nullptr, row_stride, nullptr, nullptr, 0, feature_index,
-               feature_value, dense_field_offset, g_first, g_fm, S, u, onerow_fields, B, F, DIR_OPT_SGD, 0.f,
-               w.part, w.flags, nullptr, LinOpt{DIR_OPT_SGD, 0.f, 0.f, 0.f, nullptr}};
-  int ctas = 0, rc;
-#define DIR_ORE(LP)                                          \
-  rc = launch_onerow_partials<LP>(o, n_onerow, st, &ctas); \
-  if (rc) return rc;                                         \
-  onerow_emit_to_kernel<LP><<<n_onerow, 256, 0, st>>>(o, ctas, *layout);
-  switch (K) {
-    case 4: DIR_ORE(1) break;
-    case 8: DIR_ORE(2) break;
-    case 16: DIR_ORE(4) break;
-    case 32: DIR_ORE(8) break;
-    default: DIR_ORE(16) break;
-  }
-#undef DIR_ORE
-  return launched("shard_dense_emit");
+  OneRowArgs o;
+  o.table = const_cast<float*>(dense_table); o.row_stride = row_stride;
+  o.idx = feature_index; o.val = feature_value; o.field_offset = dense_field_offset; o.fields = onerow_fields;
+  o.g_first = g_first; o.g_fm = g_fm; o.S = S; o.u = u; o.B = B; o.F = F;
+  o.part = w.part; o.flags = w.flags;
+  return with_lpr(K, [&](auto lpr) {
+    int ctas = 0;
+    if (int rc = launch_onerow_partials<lpr>(o, n_onerow, st, &ctas)) return rc;
+    onerow_emit_to_kernel<lpr><<<n_onerow, 256, 0, st>>>(o, ctas, *layout);
+    return launched("shard_dense_emit");
+  });
 }
 
 extern "C" int dir_embed_bwd_onerow_update(float* table, float* accum, int64_t row_stride, float* lin,
@@ -1454,14 +1372,12 @@ extern "C" int dir_embed_bwd_onerow_update(float* table, float* accum, int64_t r
   OneRowWs w = onerow_carve(workspace, K);
   if (workspace_bytes < w.total) return fail(DIR_ENOMEM, "embed_bwd_onerow_update: workspace too small");
   cudaMemsetAsync(w.flags, 0, kOneRowMax * 4, st);
-  OneRowArgs o{table, accum, row_stride, lin, lin_accum, lin_stride, feature_index, feature_value, field_offset,
-               g_first, g_fm, S, u, onerow_fields, B, F, optimizer, lr, w.part, w.flags,
-               reinterpret_cast<unsigned long long*>(n_unique_out), lo, clip_norm, tl1, tl2};
-  switch (K) {
-    case 4: return launch_onerow<1>(o, n_onerow, st);
-    case 8: return launch_onerow<2>(o, n_onerow, st);
-    case 16: return launch_onerow<4>(o, n_onerow, st);
-    case 32: return launch_onerow<8>(o, n_onerow, st);
-    default: return launch_onerow<16>(o, n_onerow, st);
-  }
+  OneRowArgs o;
+  o.table = table; o.accum = accum; o.row_stride = row_stride;
+  o.lin = lin; o.lin_accum = lin_accum; o.lin_stride = lin_stride; o.lo = lo;
+  o.idx = feature_index; o.val = feature_value; o.field_offset = field_offset; o.fields = onerow_fields;
+  o.g_first = g_first; o.g_fm = g_fm; o.S = S; o.u = u; o.B = B; o.F = F;
+  o.opt = optimizer; o.lr = lr; o.l1 = tl1; o.l2 = tl2; o.clip = clip_norm;
+  o.part = w.part; o.flags = w.flags; o.n_unique = reinterpret_cast<unsigned long long*>(n_unique_out);
+  return with_lpr(K, [&](auto lpr) { return launch_onerow<lpr>(o, n_onerow, st); });
 }

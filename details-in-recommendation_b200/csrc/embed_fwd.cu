@@ -27,11 +27,12 @@ struct FwdArgs {
   float* fm;
   uint32_t* sort_keys;
   int* oob_flag;
-  int tune;  // DIR_B200_TUNE bits switch a policy OFF: 1 lin evict_last, 2 emb stores evict_first, 4 rows evict_first
 };
 
+// UNR = 8 asks for three CTAs per SM, the 80 registers it has always had (ptxas otherwise takes 99 and leaves
+// two); 0 sets no minimum for the others
 template <int LPR, int UNR>
-__global__ void __launch_bounds__(256) embed_fm_fwd_kernel(const FwdArgs a) {
+__global__ void __launch_bounds__(256, UNR >= 8 ? 3 : 0) embed_fm_fwd_kernel(const FwdArgs a) {
   constexpr int K = LPR * 4;
   constexpr int RPW = 32 / LPR;  // rows fetched by one warp-wide load
   const int lane = threadIdx.x & 31;
@@ -82,16 +83,9 @@ __global__ void __launch_bounds__(256) embed_fm_fwd_kernel(const FwdArgs a) {
       t[j] = make_float4(0.f, 0.f, 0.f, 0.f);
       w[j] = 0.f;
       if (keep[j]) {
-        const float* rp = a.table + row[j] * a.row_stride + sub * 4;
-        // DIR_B200_TUNE bit 2048: 64-byte L2 fill (the accumulator half of the line is not wanted here).  Halves the
-        // gather's DRAM bytes and changes nothing: the gather is bound by the rate of random accesses (DESIGN.md section 3)
-        t[j] = (a.tune & 4) ? __ldg(reinterpret_cast<const float4*>(rp))
-                            : ((a.tune & 2048) ? ldg_hint64(rp, pol_once)
-                                               : ldg_hint(rp, (a.tune & 4096) ? pol_keep : pol_once));
-        if (a.lin != nullptr && sub == 0) {
-          const float* lp = a.lin + row[j] * a.lin_stride;
-          w[j] = (a.tune & 1) ? __ldg(lp) : ldg_hint1(lp, pol_keep);
-        }
+        // a 64-byte L2 fill and evict_last rows were both measured and change nothing (DESIGN.md section 3)
+        t[j] = ldg_hint(a.table + row[j] * a.row_stride + sub * 4, pol_once);
+        if (a.lin != nullptr && sub == 0) w[j] = ldg_hint1(a.lin + row[j] * a.lin_stride, pol_keep);
       }
     }
 #pragma unroll
@@ -107,10 +101,7 @@ __global__ void __launch_bounds__(256) embed_fm_fwd_kernel(const FwdArgs a) {
         Qv.x = fmaf(e.x, e.x, Qv.x); Qv.y = fmaf(e.y, e.y, Qv.y);
         Qv.z = fmaf(e.z, e.z, Qv.z); Qv.w = fmaf(e.w, e.w, Qv.w);
         fo = fmaf(v[j], w[j], fo);
-        if (a.emb) {
-          float* ep = a.emb + (base + f) * K + sub * 4;
-          if (a.tune & 2) stg_stream(ep, e); else stg_hint(ep, e, pol_once);
-        }
+        if (a.emb) stg_hint(a.emb + (base + f) * K + sub * 4, e, pol_once);
         if (a.sort_keys && sub == 0)
           a.sort_keys[base + f] = keep[j] ? (uint32_t)row[j] : pruned_key;
       }
@@ -190,7 +181,7 @@ extern "C" int dir_embed_fm_fwd(const float* table, int64_t row_stride, const fl
     return fail(DIR_EINVAL, "embed_fm_fwd: 0 < n_rows (< 2^32-1 when sort_keys is given) required");
   if ((B + 7) / 8 > 0x7fffffffLL) return fail(DIR_EINVAL, "embed_fm_fwd: B too large");
   FwdArgs a{table, row_stride, lin,        lin_stride, bias, feature_index, feature_value,
-            field_offset, field_rows, n_rows, B, F, emb, S, first, fm, sort_keys, oob_flag, tune()};
+            field_offset, field_rows, n_rows, B, F, emb, S, first, fm, sort_keys, oob_flag};
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   switch (K) {
     case 4: return launch_fwd<1>(a, st);

@@ -202,14 +202,14 @@ class EmbeddingFM(torch.nn.Module):
     clip_norm: tf.clip_by_norm of every column's gradient before the update (DeepCrossNetwork.py:282-289; one
     factor per column variable, over its de-duplicated row sums): a two-pass backward, only when set.
     Storage is B200-first: with Adagrad each row and its accumulator share one 128-byte line
-    ([N, 2K] fp32), and each first-order weight sits next to its accumulator ([N, 2]).
+    ([N, 2K] fp32); the first-order weights and their accumulator are separate [N] arrays.
     """
 
     def __init__(self, field_size: int, embedding_size: int,
                  rows_per_field: Union[int, Sequence[int]], optimizer: str = "adagrad",
                  lr: float = 0.01, initial_accumulator_value: float = 0.1,
                  combiner: str = "sum", first_order: bool = True, emit_embeddings: bool = True,
-                 check_bounds: bool = False, lin_interleaved: Optional[bool] = None,
+                 check_bounds: bool = False,
                  linear_optimizer: Optional[str] = None, linear_lr: Optional[float] = None,
                  l1_regularization_strength: float = 0.0, l2_regularization_strength: float = 0.0,
                  clip_norm: Optional[float] = None, optimizer_l1: float = 0.0, optimizer_l2: float = 0.0,
@@ -221,8 +221,6 @@ class EmbeddingFM(torch.nn.Module):
         if clip_norm is not None and not clip_norm > 0:
             raise ValueError("clip_norm must be > 0 (or None)")
         self.clip_norm = None if clip_norm is None else float(clip_norm)
-        if lin_interleaved is None:
-            lin_interleaved = os.environ.get("DIR_B200_LIN_INTERLEAVED", "0") == "1"
         if field_size <= 0:
             raise ValueError("empty columns.")                      # deepFM.py:104-105
         if embedding_size not in _K_OK:
@@ -257,17 +255,15 @@ class EmbeddingFM(torch.nn.Module):
         K = embedding_size
         adagrad = optimizer != "sgd"                     # the rule keeps an accumulator next to the row
         self.row_stride = 2 * K if adagrad else K
-        if self.linear_optimizer is not None:
-            lin_interleaved = False                 # the interleaved (w, accumulator) pair is the one-optimizer layout
-        self.lin_stride = 2 if (optimizer == "adagrad" and lin_interleaved) else 1
+        self.lin_stride = 1
         dev = torch.device(device)
         self.register_buffer("field_offset", torch.tensor(offsets, dtype=torch.int64, device=dev))
         self.register_buffer("field_rows", None if rows is None else
                              torch.tensor(rows, dtype=torch.int64, device=dev))
         self.register_buffer("rows", torch.empty((n_rows, self.row_stride), dtype=torch.float32, device=dev))
-        self.register_buffer("lin_rows", torch.zeros((n_rows, self.lin_stride), dtype=torch.float32, device=dev))
+        self.register_buffer("lin_rows", torch.zeros((n_rows, 1), dtype=torch.float32, device=dev))
         self.register_buffer("lin_acc", torch.zeros((n_rows, 1), dtype=torch.float32, device=dev)
-                             if (lin_needs_acc and not (optimizer == "adagrad" and lin_interleaved)) else None)
+                             if lin_needs_acc else None)
         self.register_buffer("lin_z", torch.zeros((n_rows, 1), dtype=torch.float32, device=dev)    # Ftrl 'linear' slot
                              if lin_needs_z else None)
         self.register_buffer("oob_flag", torch.zeros(1, dtype=torch.int32, device=dev))
@@ -316,9 +312,7 @@ class EmbeddingFM(torch.nn.Module):
 
     @property
     def w1_accum(self):
-        if self.lin_acc is not None:
-            return self.lin_acc[:, 0]
-        return self.lin_rows[:, 1] if self.lin_stride == 2 else None
+        return self.lin_acc[:, 0] if self.lin_acc is not None else None
 
     @torch.no_grad()
     def load_tables(self, table=None, w1=None, accum=None, w1_accum=None):
@@ -462,8 +456,7 @@ class EmbeddingFM(torch.nn.Module):
         if self._side is None:
             # high priority: the sort's few, latency-bound CTAs must not queue behind the thousands
             # of CTAs of the forward gather it is meant to run underneath
-            prio = 0 if os.environ.get("DIR_B200_SIDE_PRIORITY", "1") == "0" else -1
-            self._side = torch.cuda.Stream(device=device, priority=prio)
+            self._side = torch.cuda.Stream(device=device, priority=-1)
         return self._side
 
     def aux_stream(self, device):

@@ -445,7 +445,7 @@ class ShardedEmbeddingFM(torch.nn.Module):
         self._in_flight = [False] * (2 * self.micro_batches)
         # gather + send CTAs per SM: NVLink-bound, so with two micro-batches a small grid leaves the SMs to the forward
         # of the other half that runs next to it
-        self.gather_ctas_per_sm = int(os.environ.get("DIR_B200_GS_CTAS", "8" if self.micro_batches == 1 else "3"))
+        self.gather_ctas_per_sm = 8 if self.micro_batches == 1 else 3
         self.trace, self.trace_pre = StageTrace(), StageTrace()
         self.capturing = False
         self.exchange_mode = os.environ.get("DIR_B200_EXCHANGE", "peer")

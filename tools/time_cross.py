@@ -1,8 +1,7 @@
 #!/usr/bin/env python
-"""Parity tests of the cross kernels, then CUDA-event timing of dir_cross_fwd / dir_cross_bwd at the cfg3 shape,
-in one process (the DIR_B200_TUNE experiment bits are read once at load):
+"""Parity tests of the cross kernels, then CUDA-event timing of dir_cross_fwd / dir_cross_bwd at the cfg3 shape
+(d = 624, L = 6: the backward takes the per-warp rings), in one process:
     python tools/time_cross.py [--no-tests]
-    DIR_B200_TUNE=1024 python tools/time_cross.py       # the tiled backward instead of the per-warp rings
 """
 import os
 import sys
@@ -39,5 +38,4 @@ for it in range(23):
     if it >= 3:
         tf += ev[0].elapsed_time(ev[1])
         tb += ev[1].elapsed_time(ev[2])
-print("tests rc=%d  DIR_B200_TUNE=%s  cross_fwd %.1f us  cross_bwd %.1f us" % (
-    rc, os.environ.get("DIR_B200_TUNE", "0"), tf / 20 * 1e3, tb / 20 * 1e3))
+print("tests rc=%d  cross_fwd %.1f us  cross_bwd %.1f us" % (rc, tf / 20 * 1e3, tb / 20 * 1e3))
