@@ -11,7 +11,7 @@ from .feeder import ColumnFeeder, HostFeeder                              # noqa
 from . import frontend                                         # noqa: F401
 from .frontend import FeatureFrontEnd                          # noqa: F401
 from .layers import CrossNetwork, EmbeddingFM, InputLayer, SortedLookups # noqa: F401
-from .models import DCN, DeepFM                               # noqa: F401
+from .models import DCN, DeepFM, TFAdam                       # noqa: F401
 from .sharded import ShardedEmbeddingBagFM, ShardedEmbeddingFM, ShardedLookups, ShardPlan  # noqa: F401
 
-__all__ = ["DeepFM", "DCN", "EmbeddingFM", "EmbeddingBagFM", "InputLayer", "CrossNetwork", "ShardedEmbeddingFM", "ShardedEmbeddingBagFM", "ShardPlan", "HostFeeder", "ColumnFeeder", "FeatureFrontEnd", "frontend", "synth", "roofline", "build", "launch_count", "LIB_PATH"]
+__all__ = ["DeepFM", "DCN", "TFAdam", "EmbeddingFM", "EmbeddingBagFM", "InputLayer", "CrossNetwork", "ShardedEmbeddingFM", "ShardedEmbeddingBagFM", "ShardPlan", "HostFeeder", "ColumnFeeder", "FeatureFrontEnd", "frontend", "synth", "roofline", "build", "launch_count", "LIB_PATH"]

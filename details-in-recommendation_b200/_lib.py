@@ -24,6 +24,11 @@ class TableOpt(ctypes.Structure):
     _fields_ = [("l1", c_float), ("l2", c_float)]
 
 
+class AdamOpt(ctypes.Structure):
+    """struct dir_adam_opt (include/dir_b200.h): Adam's hyper-parameters and its device-resident beta powers."""
+    _fields_ = [("lr", c_float), ("beta1", c_float), ("beta2", c_float), ("epsilon", c_float), ("beta_power", c_void_p)]
+
+
 class PeerLayout(ctypes.Structure):
     """struct dir_peer_layout (include/dir_b200.h): the exchange buffer every rank owns, per parity."""
     _fields_ = [("G", c_int), ("rank", c_int), ("K", c_int), ("n_dense", c_int),
@@ -62,6 +67,9 @@ SIGNATURES = {
     "dir_rows_apply_clipped": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_int64,
                                        c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_float, c_int,
                                        c_float, c_void_p, c_void_p, c_void_p]),
+    "dir_rows_apply_adam": (c_int, [c_void_p, c_int64, c_int64, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
+                                    c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_void_p, c_float, c_void_p,
+                                    c_void_p, c_void_p]),
     "dir_embed_bwd_sorted": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     "dir_shard_keys": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int,
                                c_void_p, c_int, c_void_p, c_void_p, c_void_p]),

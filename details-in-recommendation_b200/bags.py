@@ -98,8 +98,9 @@ class EmbeddingBagFM(EmbeddingFM):
     `forward`; `forward_bags` takes the CSR form."""
 
     def __init__(self, field_size, embedding_size, rows_per_field, combiner="mean", **kw):
-        if str(kw.get("optimizer", "adagrad")).lower() == "proximal_adagrad":
-            raise ValueError("EmbeddingBagFM trains with 'adagrad' or 'sgd'; proximal_adagrad is an EmbeddingFM option")
+        if str(kw.get("optimizer", "adagrad")).lower() in ("proximal_adagrad", "adam"):
+            raise ValueError("EmbeddingBagFM trains with 'adagrad' or 'sgd'; proximal_adagrad and adam are EmbeddingFM "
+                             "options")
         if kw.get("clip_norm") is not None:
             raise ValueError("EmbeddingBagFM applies its gradients unclipped: clip_norm is an EmbeddingFM option")
         super().__init__(field_size, embedding_size, rows_per_field, combiner=combiner, **kw)

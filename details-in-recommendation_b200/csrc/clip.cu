@@ -15,9 +15,6 @@
 
 namespace dir {
 
-constexpr int kClipSlices = 16;    // CTAs per column in the norm pass
-constexpr int kClipMaxFields = 1024;
-
 // first distinct row u with urows[u] >= row (urows ascending, as unsigned)
 __device__ __forceinline__ int64_t lower_bound_u32(const uint32_t* __restrict__ a, int64_t n, uint64_t row) {
   int64_t lo = 0, hi = n;
@@ -74,8 +71,6 @@ field_sqnorm_kernel(const float* __restrict__ gu, int64_t stride, const uint32_t
   }
 }
 
-// [TF] clip_by_norm: values * clip_norm / max(l2norm, clip_norm)
-__device__ __forceinline__ float clip1(float g, float clip, float denom) { return __fdiv_rn(__fmul_rn(g, clip), denom); }
 
 template <int LPR>
 __global__ void __launch_bounds__(256)
@@ -87,16 +82,7 @@ rows_apply_clipped_kernel(float* table, float* accum, int64_t row_stride, float*
   constexpr int K = LPR * 4;
   __shared__ int64_t s_off[kClipMaxFields];
   __shared__ float s_den[kClipMaxFields], s_den1[kClipMaxFields];
-  for (int f = threadIdx.x; f < F; f += blockDim.x) {
-    s_off[f] = field_offset[f];
-    double a = 0.0, b = 0.0;
-    for (int s = 0; s < kClipSlices; ++s) {  // fixed order: the same factor in every CTA
-      a += part[((int64_t)f * kClipSlices + s) * 2];
-      b += part[((int64_t)f * kClipSlices + s) * 2 + 1];
-    }
-    s_den[f] = fmaxf((float)sqrt(a), clip);
-    s_den1[f] = fmaxf((float)sqrt(b), clip);
-  }
+  clip_denominators(part, field_offset, F, clip, s_off, s_den, s_den1);
   __syncthreads();
   const int64_t U = *count;
   if (n_unique_out && blockIdx.x == 0 && threadIdx.x == 0) *n_unique_out = U;

@@ -81,6 +81,30 @@ __device__ __forceinline__ void lin_load(const LinOpt& o, const float* lin_accum
   z = o.opt == DIR_OPT_FTRL ? o.z[off] : 0.f;
 }
 
+// dir_field_sqnorms' partials: [F][kClipSlices][2] doubles (sum of squares of G, of g1), one slice per CTA of the
+// norm pass (clip.cu).  Read by every apply that scales a column's gradient by its clip_by_norm factor.
+constexpr int kClipSlices = 16;
+constexpr int kClipMaxFields = 1024;
+
+// Per column f < F: its first row and the clip_by_norm denominators max(||G_f||, clip), max(||g1_f||, clip), from the
+// partials summed in a fixed order (the same factor in every CTA).  Block-strided; the caller synchronises.
+__device__ __forceinline__ void clip_denominators(const double* __restrict__ part, const int64_t* __restrict__ field_offset,
+                                                  int F, float clip, int64_t* s_off, float* s_den, float* s_den1) {
+  for (int f = threadIdx.x; f < F; f += blockDim.x) {
+    s_off[f] = field_offset[f];
+    double a = 0.0, b = 0.0;
+    for (int s = 0; s < kClipSlices; ++s) {
+      a += part[((int64_t)f * kClipSlices + s) * 2];
+      b += part[((int64_t)f * kClipSlices + s) * 2 + 1];
+    }
+    s_den[f] = fmaxf((float)sqrt(a), clip);
+    s_den1[f] = fmaxf((float)sqrt(b), clip);
+  }
+}
+
+// [TF] clip_by_norm: values * clip_norm / max(l2norm, clip_norm)
+__device__ __forceinline__ float clip1(float g, float clip, float denom) { return __fdiv_rn(__fmul_rn(g, clip), denom); }
+
 // The linear scope's optimizer: the caller's dir_linear_opt, or the tables' optimizer and rate.
 inline int resolve_lin(const char* what, const dir_linear_opt* in, int optimizer, float lr, const float* lin,
                        const float* lin_accum, LinOpt& out) {

@@ -173,7 +173,11 @@ class _EmbeddingFMFunction(torch.autograd.Function):
                 g_bias.record_stream(main)
             if ctx.handle is not None:
                 layer.apply_onerow_gradients(idx, val, g_first, g_fm, S, u, B)
-        if ctx.handle is not None:
+        if layer.optimizer == "adam":          # TF's Adam steps every row, also after an empty batch
+            if ctx.handle is not None and ctx.handle.event is not None:
+                main.wait_event(ctx.handle.event)
+            layer.apply_sorted_gradients_adam(ctx.handle, idx, val, g_first, g_fm, S, u, B)
+        elif ctx.handle is not None:
             if ctx.handle.event is not None:
                 main.wait_event(ctx.handle.event)
             if layer.clip_norm is None:
@@ -203,6 +207,11 @@ class EmbeddingFM(torch.nn.Module):
     factor per column variable, over its de-duplicated row sums): a two-pass backward, only when set.
     Storage is B200-first: with Adagrad each row and its accumulator share one 128-byte line
     ([N, 2K] fp32); the first-order weights and their accumulator are separate [N] arrays.
+    optimizer='adam': [TF] tf.train.AdamOptimizer(lr, optimizer_beta1, optimizer_beta2, optimizer_epsilon) on the
+    tables, the reference's DCN optimizer (models/DeepCrossNetwork/train.py:104-124).  TF's sparse apply decays the
+    moments of EVERY row, so each backward sweeps the whole [N, 3K] storage ([T | m | v] per row); the beta powers
+    live on the device (`beta_power`).  Every field goes through the sort (no one-row split).  Adam does not train
+    the first-order weights: with first_order=True a linear_optimizer must be named.
     """
 
     def __init__(self, field_size: int, embedding_size: int,
@@ -213,7 +222,8 @@ class EmbeddingFM(torch.nn.Module):
                  linear_optimizer: Optional[str] = None, linear_lr: Optional[float] = None,
                  l1_regularization_strength: float = 0.0, l2_regularization_strength: float = 0.0,
                  clip_norm: Optional[float] = None, optimizer_l1: float = 0.0, optimizer_l2: float = 0.0,
-                 device="cuda"):
+                 device="cuda", optimizer_beta1: float = 0.9, optimizer_beta2: float = 0.999,
+                 optimizer_epsilon: float = 1e-8):
         super().__init__()
         if optimizer_l1 < 0 or optimizer_l2 < 0:
             raise ValueError("optimizer_l1 / optimizer_l2 must be >= 0")
@@ -226,10 +236,25 @@ class EmbeddingFM(torch.nn.Module):
         if embedding_size not in _K_OK:
             raise ValueError("embedding_size must be one of %r" % (_K_OK,))
         optimizer = optimizer.lower()
-        if optimizer not in _TABLE_OPTIMIZERS:
-            raise ValueError("optimizer must be 'adagrad', 'sgd' or 'proximal_adagrad'")
+        adam = optimizer == "adam"              # kept out of _TABLE_OPTIMIZERS: no other entry point learns Adam
+        if optimizer not in _TABLE_OPTIMIZERS and not adam:
+            raise ValueError("optimizer must be 'adagrad', 'sgd', 'proximal_adagrad' or 'adam'")
         if optimizer == "proximal_adagrad" and self.clip_norm is not None:
             raise ValueError("clip_norm is not available with proximal_adagrad")
+        if adam:
+            if not lr > 0:
+                raise ValueError("adam needs lr > 0")
+            if not (0 <= optimizer_beta1 < 1 and 0 <= optimizer_beta2 < 1):
+                raise ValueError("optimizer_beta1 / optimizer_beta2 must be in [0, 1)")
+            if not optimizer_epsilon > 0:
+                raise ValueError("optimizer_epsilon must be > 0")
+            if first_order and linear_optimizer is None:
+                raise ValueError("Adam does not train first-order weights: name a linear_optimizer "
+                                 "(%s) or pass first_order=False" % ", ".join(sorted(_LINEAR_OPTIMIZERS)))
+            if linear_optimizer is None:
+                linear_lr = None
+        self.optimizer_beta1, self.optimizer_beta2 = float(optimizer_beta1), float(optimizer_beta2)
+        self.optimizer_epsilon = float(optimizer_epsilon)
         self.l1, self.l2 = float(l1_regularization_strength), float(l2_regularization_strength)
         self.linear_optimizer, self.linear_lr, lin_needs_acc, lin_needs_z = resolve_linear_optimizer(
             optimizer, lr, linear_optimizer, linear_lr, self.l1, self.l2)
@@ -253,8 +278,8 @@ class EmbeddingFM(torch.nn.Module):
         self.combiner, self.first_order = combiner, first_order
         self.emit_embeddings, self.check_bounds = emit_embeddings, check_bounds
         K = embedding_size
-        adagrad = optimizer != "sgd"                     # the rule keeps an accumulator next to the row
-        self.row_stride = 2 * K if adagrad else K
+        adagrad = optimizer not in ("sgd", "adam")       # the rule keeps an accumulator next to the row
+        self.row_stride = 3 * K if adam else (2 * K if adagrad else K)
         self.lin_stride = 1
         dev = torch.device(device)
         self.register_buffer("field_offset", torch.tensor(offsets, dtype=torch.int64, device=dev))
@@ -267,11 +292,14 @@ class EmbeddingFM(torch.nn.Module):
         self.register_buffer("lin_z", torch.zeros((n_rows, 1), dtype=torch.float32, device=dev)    # Ftrl 'linear' slot
                              if lin_needs_z else None)
         self.register_buffer("oob_flag", torch.zeros(1, dtype=torch.int32, device=dev))
+        # Adam's (beta1_power, beta2_power), advanced on the device by every apply
+        self.register_buffer("beta_power", torch.tensor([optimizer_beta1, optimizer_beta2], dtype=torch.float32,
+                                                        device=dev) if adam else None)
         # Field plan: a field whose table has ONE row (a numeric feature scaled by feature_value) needs no
         # sort -- every sample hits the same row -- so only the other fields' lookups are sorted.
         onerow = [f for f in range(field_size) if rows is not None and rows[f] == 1][:64]
-        if os.environ.get("DIR_B200_SORT_ALL_FIELDS", "0") == "1":
-            onerow = []
+        if os.environ.get("DIR_B200_SORT_ALL_FIELDS", "0") == "1" or adam:
+            onerow = []             # Adam: the one apply kernel must see every gradient of the step
         srt = [f for f in range(field_size) if f not in set(onerow)]
         self.n_sorted_fields, self.n_onerow_fields = len(srt), len(onerow)
         self.register_buffer("sorted_fields", torch.tensor(srt or [0], dtype=torch.int32, device=dev))
@@ -289,6 +317,8 @@ class EmbeddingFM(torch.nn.Module):
             torch.nn.init.trunc_normal_(self.table, 0.0, 1.0 / math.sqrt(K), -2.0 / math.sqrt(K), 2.0 / math.sqrt(K))
             if adagrad:
                 self.accum.fill_(initial_accumulator_value)
+            if adam:
+                self.rows[:, K:].zero_()
             if self.w1_accum is not None:
                 self.w1_accum.fill_(initial_accumulator_value)     # Adagrad and Ftrl both start at 0.1 in TF
 
@@ -304,7 +334,17 @@ class EmbeddingFM(torch.nn.Module):
 
     @property
     def accum(self):
-        return self.rows[:, self.embedding_size:] if self.optimizer != "sgd" else None
+        return self.rows[:, self.embedding_size:] if self.optimizer not in ("sgd", "adam") else None
+
+    @property
+    def adam_m(self):
+        K = self.embedding_size
+        return self.rows[:, K:2 * K] if self.optimizer == "adam" else None
+
+    @property
+    def adam_v(self):
+        K = self.embedding_size
+        return self.rows[:, 2 * K:3 * K] if self.optimizer == "adam" else None
 
     @property
     def w1(self):
@@ -328,7 +368,8 @@ class EmbeddingFM(torch.nn.Module):
     def export_columns(self, column_names=None, with_slots=False):
         """-> {name + '/embedding_weights': [N_f, K], name + '/weights': [N_f, 1]} on the CPU, one pair per field
         (plus '/embedding_weights/Adagrad', '/weights/Adagrad' / '/weights/Ftrl', '/weights/Ftrl_1' with
-        `with_slots`).  column_names defaults to field_0 .. field_{F-1}."""
+        `with_slots`; under Adam '/embedding_weights/Adam' (m), '/embedding_weights/Adam_1' (v) and the non-slot
+        'beta1_power', 'beta2_power', TF's names).  column_names defaults to field_0 .. field_{F-1}."""
         if self.shared_table:
             raise ValueError("export_columns needs per-field tables (rows_per_field given as a list)")
         names = list(column_names) if column_names is not None else ["field_%d" % f for f in range(self.field_size)]
@@ -342,6 +383,11 @@ class EmbeddingFM(torch.nn.Module):
         acc1 = None if acc1 is None else acc1.cpu()
         z = None if self.lin_z is None else self.lin_z[:, 0].cpu()
         lin_slot = "Ftrl" if (self.linear_optimizer or self.optimizer) == "ftrl" else "Adagrad"
+        adam_m = None if self.adam_m is None else self.adam_m.cpu()
+        adam_v = None if self.adam_v is None else self.adam_v.cpu()
+        if with_slots and adam_m is not None:
+            bp = self.beta_power.cpu()
+            out["beta1_power"], out["beta2_power"] = bp[0].clone(), bp[1].clone()
         for f, name in enumerate(names):
             sl = slice(off[f], off[f] + rows[f])
             out[name + "/embedding_weights"] = table[sl].clone()
@@ -349,6 +395,9 @@ class EmbeddingFM(torch.nn.Module):
             if with_slots:
                 if acc is not None:
                     out[name + "/embedding_weights/Adagrad"] = acc[sl].clone()
+                if adam_m is not None:
+                    out[name + "/embedding_weights/Adam"] = adam_m[sl].clone()
+                    out[name + "/embedding_weights/Adam_1"] = adam_v[sl].clone()
                 if acc1 is not None:
                     out[name + "/weights/" + lin_slot] = acc1[sl].clone().reshape(-1, 1)
                 if z is not None:
@@ -368,7 +417,8 @@ class EmbeddingFM(torch.nn.Module):
         lin_slot = "Ftrl" if (self.linear_optimizer or self.optimizer) == "ftrl" else "Adagrad"
         targets = [("/embedding_weights", self.table, K), ("/weights", self.w1, None),
                    ("/embedding_weights/Adagrad", self.accum, K), ("/weights/" + lin_slot, self.w1_accum, None),
-                   ("/weights/Ftrl_1", None if self.lin_z is None else self.lin_z[:, 0], None)]
+                   ("/weights/Ftrl_1", None if self.lin_z is None else self.lin_z[:, 0], None),
+                   ("/embedding_weights/Adam", self.adam_m, K), ("/embedding_weights/Adam_1", self.adam_v, K)]
         for f, name in enumerate(names):
             sl = slice(off[f], off[f] + rows[f])
             for suffix, dst, width in targets:
@@ -385,6 +435,11 @@ class EmbeddingFM(torch.nn.Module):
                 if tuple(src.shape) != want:
                     raise ValueError("%s: expected shape %r, got %r" % (name + suffix, want, tuple(src.shape)))
                 dst[sl].copy_(src.to(dst.device))
+        for i, key in enumerate(("beta1_power", "beta2_power")):
+            if key in columns:
+                if self.beta_power is None:
+                    raise ValueError("%s given but this layer keeps no such slot" % key)
+                self.beta_power[i] = float(columns[key])
 
     def _prepare(self, feature_index, feature_value):
         if feature_index.dim() != 2 or feature_index.shape[1] != self.field_size:
@@ -504,20 +559,18 @@ class EmbeddingFM(torch.nn.Module):
             table_opt_struct(self), linear_opt_struct(self), self.clip_norm or 0.0, ptr(ows), ows.numel(), ptr(self._nu_onerow), _stream()),
             "dir_embed_bwd_onerow_update")
 
-    @torch.no_grad()
-    def apply_sorted_gradients_clipped(self, handle, feature_index, feature_value, g_first, g_fm, S, u, B):
-        """The backward with tf.clip_by_norm on every column's gradient (DeepCrossNetwork.py:282-289): a column's
-        factor is known only once all of its row sums are, so the sums go to a buffer first (dir_embed_bwd_reduce_emit_local),
-        the per-column norms are reduced in a fixed order (dir_field_sqnorms) and a second pass scales and applies
-        (dir_rows_apply_clipped)."""
-        if self.shared_table:
+    def _emit_unique_sums(self, handle, feature_value, g_first, g_fm, S, u, B):
+        """First pass of the two-pass backward: number the distinct rows of the sorted list (dir_shard_unique), write
+        their gradient sums gu[u] = (G[K], g1) (dir_embed_bwd_reduce_emit_local) and, with a clip norm, the
+        per-column sums of squares (dir_field_sqnorms, fixed order).  -> (the buffers, device pointer of the
+        distinct-row count, n lookups); n = 0: nothing was launched."""
+        if self.clip_norm is not None and self.shared_table:
             raise ValueError("clip_norm needs per-field tables (one variable per column, as in the reference)")
         F, K = self.field_size, self.embedding_size
         n_sel = self.n_sorted_fields
-        n = B * n_sel
+        n = B * n_sel if handle is not None else 0
         if n == 0:
-            self._nu_sorted.zero_()
-            return
+            return None, None, 0
         L = _lib.lib()
         dev = S.device
         ws = handle.ws.get(L.dir_embed_bwd_workspace_bytes(max(B * F, 1), K), dev)
@@ -538,15 +591,47 @@ class EmbeddingFM(torch.nn.Module):
             ptr(S), ptr(u), ptr(c["uidx"]), B, F, K, self.n_rows, ptr(self.sorted_fields), n_sel, ptr(c["gu"]), K + 4,
             ptr(ws), ws.numel(), st), "dir_embed_bwd_reduce_emit_local")
         n_dev = c["count"].data_ptr() + 8                      # count[1] = distinct rows (dir_shard_unique, G = 1)
-        check(L.dir_field_sqnorms(ptr(c["gu"]), K + 4, ptr(c["urows"]), n_dev, ptr(self.field_offset), F, K,
-                                  self.n_rows, ptr(c["part"]), st), "dir_field_sqnorms")
+        if self.clip_norm is not None:
+            check(L.dir_field_sqnorms(ptr(c["gu"]), K + 4, ptr(c["urows"]), n_dev, ptr(self.field_offset), F, K,
+                                      self.n_rows, ptr(c["part"]), st), "dir_field_sqnorms")
+        return c, n_dev, n
+
+    @torch.no_grad()
+    def apply_sorted_gradients_clipped(self, handle, feature_index, feature_value, g_first, g_fm, S, u, B):
+        """The backward with tf.clip_by_norm on every column's gradient (DeepCrossNetwork.py:282-289): a column's
+        factor is known only once all of its row sums are, so the sums go to a buffer first (dir_embed_bwd_reduce_emit_local),
+        the per-column norms are reduced in a fixed order (dir_field_sqnorms) and a second pass scales and applies
+        (dir_rows_apply_clipped)."""
+        c, n_dev, n = self._emit_unique_sums(handle, feature_value, g_first, g_fm, S, u, B)
+        if n == 0:
+            self._nu_sorted.zero_()
+            return
+        F, K = self.field_size, self.embedding_size
         adagrad = self.optimizer == "adagrad"
-        check(L.dir_rows_apply_clipped(
+        check(_lib.lib().dir_rows_apply_clipped(
             ptr(self.table), ptr(self.accum) if adagrad else None, self.row_stride,
             ptr(self.w1) if self.first_order else None, ptr(self.w1_accum) if self.first_order else None,
             self.lin_stride, ptr(c["gu"]), K + 4, ptr(c["urows"]), n_dev, n, ptr(self.field_offset), F, K,
             ptr(c["part"]), self.clip_norm, _OPTIMIZERS[self.optimizer], self.lr, linear_opt_struct(self),
-            ptr(self._nu_sorted), st), "dir_rows_apply_clipped")
+            ptr(self._nu_sorted), _stream()), "dir_rows_apply_clipped")
+
+    @torch.no_grad()
+    def apply_sorted_gradients_adam(self, handle, feature_index, feature_value, g_first, g_fm, S, u, B):
+        """Adam (optimizer='adam'): the first pass of the clipped backward (`_emit_unique_sums`), then one sweep of
+        the whole table (dir_rows_apply_adam) that decays every row's moments, adds the batch's de-duplicated
+        (and, with clip_norm, clipped) gradients, moves every row and steps the first-order weights of the touched
+        rows with the linear optimizer.  The beta powers advance on the device after the sweep."""
+        c, n_dev, n = self._emit_unique_sums(handle, feature_value, g_first, g_fm, S, u, B)
+        F, K = self.field_size, self.embedding_size
+        opt = _lib.AdamOpt(self.lr, self.optimizer_beta1, self.optimizer_beta2, self.optimizer_epsilon,
+                           self.beta_power.data_ptr())
+        first = self.first_order and n > 0
+        check(_lib.lib().dir_rows_apply_adam(
+            ptr(self.rows), self.row_stride, self.n_rows, K, ptr(self.w1) if first else None,
+            ptr(self.w1_accum) if first else None, self.lin_stride, linear_opt_struct(self) if first else None,
+            ptr(c["gu"]) if n else None, K + 4, ptr(c["urows"]) if n else None, n_dev, n, ptr(self.field_offset), F,
+            ptr(c["part"]) if (n and self.clip_norm is not None) else None, self.clip_norm or 0.0,
+            _lib.ctypes.byref(opt), ptr(self._nu_sorted), _stream()), "dir_rows_apply_adam")
 
 
 class _CrossFunction(torch.autograd.Function):

@@ -11,7 +11,8 @@ Estimator orchestration, input_fn, metrics and checkpoints stay out of scope (DE
 
 Embedding tables and first-order weights are optimizer-owned state of the layer (updated in place during
 `.backward()`); everything else is an ordinary Parameter stepped by `dense_optimizer()`, the dense
-counterpart of the same rule ([TF] ApplyAdagrad: accumulator 0.1, no epsilon).
+counterpart of the same rule ([TF] ApplyAdagrad: accumulator 0.1, no epsilon; `DCN(optimizer='adam')`: [TF] ApplyAdam,
+`TFAdam`).
 """
 from typing import Optional, Sequence
 
@@ -61,6 +62,62 @@ def _embedding_layer(sharded, *args, **kw):
     return (ShardedEmbeddingFM if sharded else EmbeddingFM)(*args, **kw)
 
 
+class TFAdam(torch.optim.Optimizer):
+    """[TF] ApplyAdam, tf.train.AdamOptimizer's rule for dense variables (the reference's DCN optimizer,
+    models/DeepCrossNetwork/train.py:104-124), in fp32:
+        lr_t = lr * sqrt(1 - beta2_power) / (1 - beta1_power)
+        m += (g - m) * (1 - beta1);  v += (g * g - v) * (1 - beta2);  var -= (m * lr_t) / (sqrt(v) + epsilon)
+        then beta1_power *= beta1, beta2_power *= beta2 (once per step, shared by every parameter)
+    Not torch.optim.Adam, which adds epsilon after the bias correction of v.  The beta powers are one device tensor
+    (`beta_power`, kept in the optimizer's state so state_dict() / load_state_dict() carry it), so a captured step
+    replays with the right bias correction."""
+
+    def __init__(self, params, lr, beta1=0.9, beta2=0.999, epsilon=1e-8):
+        if not lr > 0 or not (0 <= beta1 < 1 and 0 <= beta2 < 1) or not epsilon > 0:
+            raise ValueError("TFAdam needs lr > 0, 0 <= beta1, beta2 < 1 and epsilon > 0")
+        super().__init__(params, dict(lr=float(lr)))
+        self.beta1, self.beta2, self.epsilon = float(beta1), float(beta2), float(epsilon)
+        # 1 - beta as TF evaluates it, in fp32 (1 - 0.9 in fp64 rounds to a different fp32 value)
+        self._omb1 = float(torch.tensor(1.0) - torch.tensor(self.beta1))
+        self._omb2 = float(torch.tensor(1.0) - torch.tensor(self.beta2))
+        self._betas = None
+
+    @property
+    def beta_power(self):
+        """(beta1_power, beta2_power), float32[2] on the parameters' device (None before the first step)."""
+        return self.state.get("beta_power")
+
+    @torch.no_grad()
+    def step(self, closure=None):
+        loss = closure() if closure is not None else None
+        params = [p for g in self.param_groups for p in g["params"]]
+        if not params:
+            return loss
+        dev = params[0].device
+        bp = self.state.get("beta_power")
+        if bp is None:
+            bp = torch.tensor([self.beta1, self.beta2], dtype=torch.float32, device=dev)
+        elif bp.device != dev:                   # loaded from a checkpoint on another device
+            bp = bp.to(dev)
+        self.state["beta_power"] = bp            # not a parameter's state: load_state_dict copies it as it is
+        if self._betas is None or self._betas.device != dev:
+            self._betas = torch.tensor([self.beta1, self.beta2], dtype=torch.float32, device=dev)
+        for group in self.param_groups:
+            lr_t = (group["lr"] * torch.sqrt(1 - bp[1])) / (1 - bp[0])
+            for p in group["params"]:
+                if p.grad is None:
+                    continue
+                st = self.state[p]
+                if not st:
+                    st["m"], st["v"] = torch.zeros_like(p), torch.zeros_like(p)
+                g, m, v = p.grad, st["m"], st["v"]
+                m.add_((g - m) * self._omb1)
+                v.add_((g * g - v) * self._omb2)
+                p.sub_((m * lr_t) / (v.sqrt() + self.epsilon))
+        bp.mul_(self._betas)
+        return loss
+
+
 def clip_by_norm_(parameters, clip_norm):
     """tf.clip_by_norm applied to EACH gradient tensor (DeepCrossNetwork.py:284), not a global norm."""
     for p in parameters:
@@ -87,6 +144,8 @@ class DeepFM(torch.nn.Module):
                  linear_learning_rate: Optional[float] = None, loss_reduction: str = "sum", sharded: bool = False,
                  device="cuda", **layer_kw):
         super().__init__()
+        if str(dnn_optimizer).lower() == "adam":
+            raise ValueError("DeepFM trains with Adagrad (the reference's dnn_optimizer) or SGD; adam is a DCN option")
         if not dnn_hidden_units:
             raise ValueError("dnn_hidden_units must name at least one layer")
         if loss_reduction not in ("sum", "mean"):
@@ -133,18 +192,26 @@ class DCN(torch.nn.Module):
     The per-tensor clip_by_norm(100) is applied to every gradient, as the reference does: the dense ones here, each
     column's table gradient inside the layer (`EmbeddingFM(clip_norm=...)`, a two-pass backward).  The sharded
     layer applies its table gradients unclipped (a column's norm would need a cross-rank reduction per step).
+    optimizer='adam' is the reference's own (train.py:104-124, epsilon = adam_epsilon = 1e-4): TF's Adam on the
+    tables (`EmbeddingFM(optimizer='adam')`, every row's moments decay at every step) and `TFAdam` on the dense
+    parameters.  Single-GPU layer only.
     """
 
     def __init__(self, field_size: int, embedding_size: int, rows_per_field: Sequence[int],
                  cross_layer_num: int = 2, hidden_units: Sequence[int] = (256, 128), dnn_activation_fn=torch.relu,
                  dnn_dropout: Optional[float] = None, batch_norm: bool = False, optimizer: str = "adagrad",
                  learning_rate: float = _ADAGRAD_LR, clip_norm: Optional[float] = 100.0, sharded: bool = False,
-                 device="cuda", **layer_kw):
+                 device="cuda", adam_epsilon: float = 1e-4, **layer_kw):
         super().__init__()
         d = field_size * embedding_size
         self.learning_rate, self.clip_norm = float(learning_rate), clip_norm
+        self.optimizer, self.adam_epsilon = optimizer.lower(), float(adam_epsilon)
         if clip_norm and not sharded:
             layer_kw = dict(layer_kw, clip_norm=clip_norm)      # every column's gradient is clipped too (:284)
+        if self.optimizer == "adam":
+            if sharded:
+                raise ValueError("DCN(optimizer='adam') needs the single-GPU layer (sharded=False)")
+            layer_kw = dict(layer_kw, optimizer_epsilon=self.adam_epsilon)
         self.embedding = _embedding_layer(sharded, field_size, embedding_size, list(rows_per_field), optimizer=optimizer,
                                           lr=learning_rate, first_order=False, device=device, **layer_kw)
         self.cross = CrossNetwork(d, cross_layer_num, device=device)
@@ -167,6 +234,8 @@ class DCN(torch.nn.Module):
         return [p for n, p in self.named_parameters() if not n.endswith(skip)]
 
     def dense_optimizer(self):
+        if self.optimizer == "adam":
+            return TFAdam(self.dense_parameters(), self.learning_rate, epsilon=self.adam_epsilon)
         return torch.optim.Adagrad(self.dense_parameters(), lr=self.learning_rate,
                                    initial_accumulator_value=0.1, eps=0.0)
 

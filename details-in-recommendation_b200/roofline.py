@@ -28,6 +28,18 @@ def embed_bwd_bytes(B, F, K, U, weighted=True, upstream=True, optimizer="adagrad
     return 4 * B + (B * F * R if upstream else 0) + B * F * (I_BYTES + V + R) + U * (R + 4) * c
 
 
+def adam_apply_bytes(n_rows, K, U, first_order=False, linear_optimizer=None):
+    """dir_rows_apply_adam: TF's Adam decays every row's moments, so the sweep reads and writes all n_rows rows
+    [T | m | v] (3R each way) plus, per distinct row, its index (4 B) and its gradient G and, with first-order
+    weights, g1 and the weight's state (as embed_bwd_bytes counts it: c = 4 for Adagrad / Ftrl-like, 2 for SGD)."""
+    R = 4 * K
+    lin = 0
+    if first_order:
+        c = 2 if linear_optimizer == "sgd" else 4
+        lin = U * (4 + 4 * c + (8 if linear_optimizer == "ftrl" else 0))
+    return n_rows * 3 * R * 2 + U * (4 + R) + lin
+
+
 def cross_fwd_bytes(B, d, L):
     return 2 * B * d * 4 + 2 * L * d * 4
 

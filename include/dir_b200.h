@@ -182,6 +182,34 @@ int dir_rows_apply_clipped(float* table, float* accum, int64_t row_stride, float
                            int K, const double* partials, float clip_norm, int optimizer, float lr,
                            const dir_linear_opt* linear_opt, int64_t* n_unique_out, dir_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * [TF] tf.train.AdamOptimizer on a table (the reference's DCN optimizer, models/DeepCrossNetwork/train.py:104-124).
+ * On an IndexedSlices gradient TF decays the moments of EVERY row of the variable, not only the batch's:
+ *   lr_t = lr * sqrt(1 - beta2_power) / (1 - beta1_power)        (fp32, the powers before this step)
+ *   m = m * beta1;  m[r] += g_r * (1 - beta1);  v = v * beta2;  v[r] += (g_r * g_r) * (1 - beta2)
+ *   T = T - (lr_t * m) / (sqrt(v) + epsilon)                      every row
+ *   then beta1_power *= beta1, beta2_power *= beta2                (they start at beta1, beta2)
+ * dir_rows_apply_adam is that step as one sweep over all n_rows rows, laid out [T(K) | m(K) | v(K)] with
+ * row_stride >= 3K, after dir_shard_unique + dir_embed_bwd_reduce_emit_local (gu, unique_rows, n_unique_dev as for
+ * dir_rows_apply_clipped; n_capacity = 0: no gradient, gu / unique_rows / n_unique_dev may be NULL).
+ *   partials (NULL = no clip): dir_field_sqnorms' output, every column's gradient scaled by clip_by_norm(clip_norm)
+ *   lin (may be NULL): first-order weights of the rows with a gradient, stepped by linear_opt (required with lin:
+ *   Adam on the first-order weights is not supported); lin_accum as for dir_embed_bwd_reduce_update
+ *   adam->beta_power: DEVICE float[2] = (beta1_power, beta2_power), read by the sweep and advanced after it on the
+ *   same stream, so a captured CUDA graph applies the right bias correction at every replay.
+ * Deterministic (no atomics).  Rows whose m and v are zero and that have no gradient are left unwritten (they do
+ * not change).
+ */
+typedef struct dir_adam_opt {
+  float lr, beta1, beta2, epsilon;  /* lr > 0, 0 <= beta < 1, epsilon > 0 */
+  float* beta_power;                /* DEVICE float[2] */
+} dir_adam_opt;
+int dir_rows_apply_adam(float* table, int64_t row_stride, int64_t n_rows, int K, float* lin, float* lin_accum,
+                        int64_t lin_stride, const dir_linear_opt* linear_opt, const float* gu, int64_t gu_stride,
+                        const uint32_t* unique_rows, const int64_t* n_unique_dev, int64_t n_capacity,
+                        const int64_t* field_offset, int F, const double* partials, float clip_norm,
+                        const dir_adam_opt* adam, int64_t* n_unique_out, dir_stream_t stream);
+
 /* Where step 1 left the sorted (row, position) pairs inside its workspace (read-only views). */
 int dir_embed_bwd_sorted(const void* workspace, int64_t n_lookups, const uint32_t** sorted_keys,
                          const uint32_t** sorted_pos);
