@@ -26,6 +26,7 @@ _OPTIMIZERS = {"sgd": _lib.OPT_SGD, "adagrad": _lib.OPT_ADAGRAD}
 _TABLE_OPTIMIZERS = dict(_OPTIMIZERS, proximal_adagrad=_lib.OPT_PROXIMAL_ADAGRAD)       # single-GPU layer
 _LINEAR_OPTIMIZERS = dict(_TABLE_OPTIMIZERS, ftrl=_lib.OPT_FTRL)
 _K_OK = (4, 8, 16, 32, 64)
+_CLIP_MAX_FIELDS = 1024       # columns the clip's norm and apply kernels hold factors for (kClipMaxFields, update.cuh)
 
 
 def table_opt_struct(layer):
@@ -233,6 +234,9 @@ class EmbeddingFM(torch.nn.Module):
         self.clip_norm = None if clip_norm is None else float(clip_norm)
         if field_size <= 0:
             raise ValueError("empty columns.")                      # deepFM.py:104-105
+        if self.clip_norm is not None and field_size > _CLIP_MAX_FIELDS:
+            raise ValueError("clip_norm supports at most %d fields (one clip factor per column), got field_size=%d"
+                             % (_CLIP_MAX_FIELDS, field_size))
         if embedding_size not in _K_OK:
             raise ValueError("embedding_size must be one of %r" % (_K_OK,))
         optimizer = optimizer.lower()
