@@ -105,14 +105,6 @@ SIGNATURES = {
                                       c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dir_table_init_counter": (c_int, [c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_int64, c_uint64, c_float,
                                        c_void_p]),
-    "dir_rows_gather": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p,
-                                c_int64, c_void_p]),
-    "dir_embed_bwd_reduce_emit": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                                          c_void_p, c_int64, c_int, c_int, c_int64, c_void_p, c_int64,
-                                          c_void_p, c_size_t, c_void_p]),
-    "dir_rows_reduce_update": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
-                                       c_int64, c_int64, c_int, c_int64, c_int, c_float, c_void_p, c_void_p,
-                                       c_void_p, c_size_t, c_void_p, c_void_p]),
     "dir_embed_bag_fm_fwd": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p,
                                      c_int64, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_void_p,
                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -108,8 +108,6 @@ struct BwdArgs {
   const uint32_t* rowidx = nullptr;  // kModeEmit: row of `table` (the exchanged unique-row buffer) per sorted entry
   float* emit = nullptr;             // kModeEmit: [n_unique, emit_stride] receives (G[K], g1) per run
   int64_t emit_stride = 0;
-  const float* gbuf = nullptr;       // kModeGiven: [n, gbuf_stride] per-lookup (G[K], g1), indexed by position
-  int64_t gbuf_stride = 0;
   // kModeEmit straight into the owners' buffers over NVLink (emit_peers != NULL; csrc/shard_peer.cu): distinct
   // row u of segment q (emit_seg[q] <= u < emit_seg[q+1]) is row emit_dst_row + u - emit_seg[q] of the gradient
   // region (emit_byte_off) of the buffer at the peer-mapped address emit_peers[q]; its g1 goes to emit_g1[u]
@@ -123,9 +121,6 @@ struct BwdArgs {
   int perm_G = 0, perm_rank = 0;  // > 1: warps take the chunks in an owner-interleaved, rank-rotated order (see chunk_of)
   int64_t perm_M = 0;
   int emit_read_key = 0;  // kModeEmit over the table itself: rows are read at the key, sums still go to row uidx of `emit`
-  // entries actually in the sorted list, read on the device (NULL: n).  `n` then only bounds the launch
-  // and lays out the workspace, so a step whose sizes are known on the device alone needs no host read.
-  const int64_t* n_dev = nullptr;
   LinOpt lo{};
   // kModeBag (multi-hot bags, embed_bag.cu): sorted payload = entry index j
   const uint32_t* entry_slot = nullptr;  // [nnz] slot b*F+f of entry j
@@ -133,12 +128,6 @@ struct BwdArgs {
   const float* emb = nullptr;            // [B*F, K] combined embeddings e_s saved by the forward
   float l1 = 0.f, l2 = 0.f;              // ProximalAdagrad strengths of the table rows
 };
-
-__device__ __forceinline__ int64_t entries(const BwdArgs& a) {
-  if (a.n_dev == nullptr) return a.n;
-  const int64_t m = __ldg(a.n_dev);
-  return m < a.n ? m : a.n;
-}
 
 // one distinct row's sums: LPR lanes store the K-vector; g1 follows it in a local emit row, or goes to emit_g1[u]
 // when the rows cross NVLink (64-byte rows there: whole 16-byte stores only, g1 is shipped in bulk afterwards)
@@ -162,7 +151,6 @@ __device__ __forceinline__ void emit_store(const BwdArgs& a, uint32_t u, int sub
 
 constexpr int kModeLocal = 0;  // gradients formed from g, S, u, row; the row is updated in place
 constexpr int kModeEmit = 1;   // requester side of a sharded table: per-row sums go to `emit`
-constexpr int kModeGiven = 2;  // owner side: per-lookup gradients arrive in `gbuf`; update in place
 constexpr int kModeBag = 3;    // multi-hot bags: entry j of slot s contributes x_j (g_fm (S - e_s) + u_s)
 constexpr int kModeBagEmit = 4;  // requester side of a sharded table fed with bags: kModeBag's gradients, kModeEmit's sums
 __host__ __device__ constexpr bool mode_emits(int m) { return m == kModeEmit || m == kModeBagEmit; }
@@ -244,7 +232,7 @@ __global__ void __launch_bounds__(256, 3) embed_bwd_reduce_kernel(const BwdArgs 
   int64_t chunk = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (a.perm_G > 1) chunk = (int64_t)((chunk + a.perm_rank) % a.perm_G) * a.perm_M + chunk / a.perm_G;
   const int64_t i0 = chunk * kChunk;
-  const int64_t n = entries(a);
+  const int64_t n = a.n;
   if (i0 >= n) return;  // whole warp
   const int64_t chunk_end = min(n, i0 + (int64_t)kChunk);
   const uint32_t prev_key = i0 > 0 ? __ldg(a.keys + i0 - 1) : kNoKey;
@@ -304,9 +292,7 @@ __global__ void __launch_bounds__(256, 3) embed_bwd_reduce_kernel(const BwdArgs 
     if (a.field_sel != nullptr)  // compact list of selected fields -> position in the [B, F] inputs
       pos = b * (uint32_t)a.F + (uint32_t)__ldg(a.field_sel + (pos - b * (uint32_t)a.n_sel));
     if (valid) {
-      if (MODE == kModeGiven) {
-        d1l = __ldg(a.gbuf + (int64_t)pos * a.gbuf_stride + K);
-      } else if (BAG) {
+      if (BAG) {
         if (a.g_first) d1l = __fmul_rn(__ldg(a.g_first + b), wraw);   // first order combines with 'sum'
         g2 = __ldg(a.g_fm + b);
       } else {
@@ -345,28 +331,23 @@ __global__ void __launch_bounds__(256, 3) embed_bwd_reduce_kernel(const BwdArgs 
         k[j] = __shfl_sync(FULL, key, l);
         rw[j] = EMIT ? __shfl_sync(FULL, row, l) : k[j];
         const uint32_t p = __shfl_sync(FULL, pos, l);
-        const uint32_t bb = MODE == kModeGiven ? 0u : __shfl_sync(FULL, b, l);
+        const uint32_t bb = __shfl_sync(FULL, b, l);
         ac[j] = __shfl_sync(FULL, act, l);
         Sb[j] = ub[j] = T[j] = A[j] = make_float4(0.f, 0.f, 0.f, 0.f);
         lw[j] = a1[j] = lz[j] = 0.f;
         if (k[j] != a.pruned_key) {
           const int64_t ro = (int64_t)((EMIT && a.emit_read_key) ? k[j] : rw[j]) * a.row_stride;
-          if (MODE == kModeGiven) {  // the per-lookup gradient was formed by the requester
-            ub[j] = ldg_hint(a.gbuf + (int64_t)p * a.gbuf_stride + sub * 4, pol_once);
+          // (S before u: the other order spills 8 bytes at K = 32 and 64.  A 64-byte L2 fill for one field's slice
+          // of u measured slower: the neighbouring field's slice is no longer left in L2 for the warp that wants it)
+          Sb[j] = __ldg(reinterpret_cast<const float4*>(a.S + (int64_t)bb * K) + sub);
+          if (a.u) ub[j] = ldg_hint(a.u + (int64_t)p * K + sub * 4, pol_once);
+          if (BAG) {
+            T[j] = __ldg(reinterpret_cast<const float4*>(a.emb + (int64_t)p * K) + sub);
           } else {
-            // (S before u: the other order spills 8 bytes at K = 32 and 64.  A 64-byte L2 fill for one field's slice
-            // of u measured slower: the neighbouring field's slice is no longer left in L2 for the warp that wants it)
-            Sb[j] = __ldg(reinterpret_cast<const float4*>(a.S + (int64_t)bb * K) + sub);
-            if (a.u) ub[j] = ldg_hint(a.u + (int64_t)p * K + sub * 4, pol_once);
-            if (BAG) {
-              T[j] = __ldg(reinterpret_cast<const float4*>(a.emb + (int64_t)p * K) + sub);
-            } else {
-              // coherent load: this warp may rewrite the row further down
-              T[j] = ld_hint(a.table + ro + sub * 4, pol_row);
-            }
+            // coherent load: this warp may rewrite the row further down
+            T[j] = ld_hint(a.table + ro + sub * 4, pol_row);
           }
           if (!EMIT && (ac[j] & 3) == 1) {
-            if (MODE == kModeGiven) T[j] = ld_hint(a.table + ro + sub * 4, pol_row);
             if (MODE == kModeBag) Rw[j] = ld_hint(a.table + ro + sub * 4, pol_row);
             if (adagrad) A[j] = ld_hint(a.accum + ro + sub * 4, pol_row);
             if (a.lin != nullptr && sub == 0) {
@@ -379,18 +360,16 @@ __global__ void __launch_bounds__(256, 3) embed_bwd_reduce_kernel(const BwdArgs 
 #pragma unroll
       for (int j = 0; j < PB; ++j) {
         const int l = (j0 + j) * SLOTS + slot;
-        float4 d = ub[j];
+        float4 d;
         float d1 = __shfl_sync(FULL, d1l, l);
-        if (MODE != kModeGiven) {
-          // value * (g_fm * (S - value*T) + u), evaluation order of the oracle
-          const float x = __shfl_sync(FULL, v, l), gg = __shfl_sync(FULL, g2, l);
-          // e of this lookup: value * row, or (bags) the combined embedding of its slot
-          const float xe = BAG ? 1.f : x;
-          d.x = __fmul_rn(x, __fadd_rn(__fmul_rn(gg, __fsub_rn(Sb[j].x, __fmul_rn(xe, T[j].x))), ub[j].x));
-          d.y = __fmul_rn(x, __fadd_rn(__fmul_rn(gg, __fsub_rn(Sb[j].y, __fmul_rn(xe, T[j].y))), ub[j].y));
-          d.z = __fmul_rn(x, __fadd_rn(__fmul_rn(gg, __fsub_rn(Sb[j].z, __fmul_rn(xe, T[j].z))), ub[j].z));
-          d.w = __fmul_rn(x, __fadd_rn(__fmul_rn(gg, __fsub_rn(Sb[j].w, __fmul_rn(xe, T[j].w))), ub[j].w));
-        }
+        // value * (g_fm * (S - value*T) + u), evaluation order of the oracle
+        const float x = __shfl_sync(FULL, v, l), gg = __shfl_sync(FULL, g2, l);
+        // e of this lookup: value * row, or (bags) the combined embedding of its slot
+        const float xe = BAG ? 1.f : x;
+        d.x = __fmul_rn(x, __fadd_rn(__fmul_rn(gg, __fsub_rn(Sb[j].x, __fmul_rn(xe, T[j].x))), ub[j].x));
+        d.y = __fmul_rn(x, __fadd_rn(__fmul_rn(gg, __fsub_rn(Sb[j].y, __fmul_rn(xe, T[j].y))), ub[j].y));
+        d.z = __fmul_rn(x, __fadd_rn(__fmul_rn(gg, __fsub_rn(Sb[j].z, __fmul_rn(xe, T[j].z))), ub[j].z));
+        d.w = __fmul_rn(x, __fadd_rn(__fmul_rn(gg, __fsub_rn(Sb[j].w, __fmul_rn(xe, T[j].w))), ub[j].w));
         if (k[j] == a.pruned_key) {
           d = make_float4(0.f, 0.f, 0.f, 0.f);
           d1 = 0.f;
@@ -455,8 +434,9 @@ __global__ void __launch_bounds__(256, 3) embed_bwd_reduce_kernel(const BwdArgs 
 // spans more than kLongRun chunks is left to phase 3: the whole CTA finds its end by probing chunk
 // heads in parallel, sums the partials strided over lane groups (sequential per group) and combines
 // the groups with a fixed-shape tree.
+// (six CTAs per SM keeps 40 registers; without the bound ptxas took 48)
 template <int LPR>
-__global__ void __launch_bounds__(256) embed_bwd_finish_kernel(const BwdArgs a, int64_t* n_unique_out) {
+__global__ void __launch_bounds__(256, 6) embed_bwd_finish_kernel(const BwdArgs a, int64_t* n_unique_out) {
   constexpr int K = LPR * 4;
   constexpr int NG = 256 / LPR;  // lane groups per CTA
   __shared__ float4 sm[256];
@@ -467,7 +447,7 @@ __global__ void __launch_bounds__(256) embed_bwd_finish_kernel(const BwdArgs a, 
   __syncthreads();
   const int q = threadIdx.x / LPR;
   const int sub = threadIdx.x % LPR;
-  const int64_t n = entries(a);
+  const int64_t n = a.n;
   {
     const int64_t gid = (int64_t)blockIdx.x * NG + q;
     const int64_t i0 = gid * kChunk;
@@ -555,8 +535,6 @@ static int launch_bwd(const BwdArgs& a, int64_t* n_unique_out, cudaStream_t st) 
   const unsigned rgrid = (unsigned)((vchunks + 7) / 8);
   if (a.mode == kModeEmit)
     embed_bwd_reduce_kernel<LPR, kModeEmit><<<rgrid, 256, 0, st>>>(a);
-  else if (a.mode == kModeGiven)
-    embed_bwd_reduce_kernel<LPR, kModeGiven><<<rgrid, 256, 0, st>>>(a);
   else if (a.mode == kModeBag)
     embed_bwd_reduce_kernel<LPR, kModeBag><<<rgrid, 256, 0, st>>>(a);
   else if (a.mode == kModeBagEmit)
@@ -1089,19 +1067,6 @@ static int reduce_emit(const char* what, const float* ubuf, int64_t ubuf_stride,
   return dispatch_bwd(a, K, nullptr, static_cast<cudaStream_t>(stream));
 }
 
-extern "C" int dir_embed_bwd_reduce_emit(const float* ubuf, int64_t ubuf_stride,
-                                         const float* feature_value, const float* g_first,
-                                         const float* g_fm, const float* S, const float* u,
-                                         const uint32_t* uidx, int64_t B, int F, int K,
-                                         int64_t n_keys, float* gu, int64_t gu_stride,
-                                         void* workspace, size_t workspace_bytes,
-                                         dir_stream_t stream) {
-  if (!gu) return dir::fail(DIR_EINVAL, "embed_bwd_reduce_emit: gu is required");
-  return reduce_emit("embed_bwd_reduce_emit", ubuf, ubuf_stride, feature_value, g_first, g_fm, S, u, uidx, B, F,
-                     K, n_keys, gu, gu_stride, nullptr, nullptr, nullptr, workspace, workspace_bytes, stream,
-                     nullptr, 0);
-}
-
 /* the same per-distinct-row sums for a table that lives HERE (rows read at their global row, sums written to
  * gu[uidx]): the first pass of the clipped backward (csrc/clip.cu) */
 extern "C" int dir_embed_bwd_reduce_emit_local(const float* table, int64_t row_stride, const float* feature_value,
@@ -1129,43 +1094,6 @@ extern "C" int dir_embed_bwd_reduce_emit_to(const dir_peer_layout* layout, const
   return reduce_emit("embed_bwd_reduce_emit_to", rows, layout->K, feature_value, g_first, g_fm, S, u, uidx, B, F,
                      layout->K, n_keys, nullptr, 0, layout, owner_off, g1_local, workspace, workspace_bytes, stream,
                      field_sel, n_sel);
-}
-
-/* owner side: per-lookup gradients arrive from the requesters; segmented sum + fused row update */
-extern "C" int dir_rows_reduce_update(float* table, float* accum, int64_t row_stride, float* lin,
-                                      float* lin_accum, int64_t lin_stride, const float* gbuf,
-                                      int64_t gbuf_stride, int64_t n, int K, int64_t n_rows,
-                                      int optimizer, float lr, const dir_linear_opt* linear_opt,
-                                      const int64_t* n_device, void* workspace, size_t workspace_bytes,
-                                      int64_t* n_unique_out, dir_stream_t stream) {
-  using namespace dir;
-  if (n < 0 || n >= 0x7fffffffLL) return fail(DIR_EINVAL, "rows_reduce_update: 0 <= n < 2^31 required");
-  if (optimizer != DIR_OPT_SGD && optimizer != DIR_OPT_ADAGRAD)
-    return fail(DIR_EINVAL, "rows_reduce_update: unknown optimizer");
-  if (n == 0) return 0;
-  if (!table || !gbuf || !workspace)
-    return fail(DIR_EINVAL, "rows_reduce_update: table, gbuf, workspace are required");
-  if (optimizer == DIR_OPT_ADAGRAD && !accum) return fail(DIR_EINVAL, "rows_reduce_update: Adagrad needs accum");
-  LinOpt lo;
-  if (int rc = resolve_lin("rows_reduce_update", linear_opt, optimizer, lr, lin, lin_accum, lo)) return rc;
-  if (K != 4 && K != 8 && K != 16 && K != 32 && K != 64)
-    return fail(DIR_EINVAL, "rows_reduce_update: K must be one of 4, 8, 16, 32, 64");
-  if (row_stride < K || (row_stride & 3) || gbuf_stride < K + 1 || (gbuf_stride & 3))
-    return fail(DIR_EINVAL, "rows_reduce_update: strides must be multiples of 4, >= K (rows), >= K+1 (gbuf)");
-  if (!aligned16(table) || !aligned16(accum) || !aligned16(gbuf))
-    return fail(DIR_EINVAL, "rows_reduce_update: table, accum, gbuf must be 16-byte aligned");
-  if (n_rows <= 0 || n_rows >= 0xffffffffLL)
-    return fail(DIR_EINVAL, "rows_reduce_update: 0 < n_rows < 2^32-1 required");
-  BwdWorkspace w = carve(workspace, n, K);
-  if (workspace_bytes < w.total) return fail(DIR_ENOMEM, "rows_reduce_update: workspace too small");
-  BwdArgs a;
-  set_sorted(a, w, n, 1, 1);
-  a.mode = kModeGiven;
-  a.table = table; a.accum = accum; a.row_stride = row_stride;
-  a.lin = lin; a.lin_accum = lin_accum; a.lin_stride = lin_stride; a.lo = lo;
-  a.gbuf = gbuf; a.gbuf_stride = gbuf_stride; a.n_dev = n_device;
-  a.pruned_key = (uint32_t)n_rows; a.opt = optimizer; a.lr = lr;
-  return dispatch_bwd(a, K, n_unique_out, static_cast<cudaStream_t>(stream));
 }
 
 /* multi-hot bags: backward + fused update on the sorted (row, entry) list (include/dir_b200.h) */

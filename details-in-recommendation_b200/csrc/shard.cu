@@ -1,4 +1,4 @@
-// Row-sharded tables: the id-only kernels (keys, distinct-row numbering) and the NCCL flavour's row gather.
+// Row-sharded tables: the id-only kernels (keys, distinct-row numbering).
 //
 // Tables are sharded by row over G ranks (owner = global row mod G, local row = global row div G:
 // modulo, so hot low-numbered rows spread evenly).  The batch stays data-parallel.  Per step a rank
@@ -6,8 +6,7 @@
 //                             (key, lookup position)                                  [keys.cuh, embed_bwd.cu, radix.cuh]
 //   2. dir_shard_unique       numbers the distinct keys: only those cross NVLink
 //   3. the exchange: ids to the owners, rows back, per-distinct-row gradient sums to the owners -- stored
-//      straight into the peers' buffers by the kernels of shard_peer.cu (default), or through NCCL
-//      all-to-all with dir_rows_gather / dir_embed_bwd_reduce_emit / dir_rows_reduce_update (DIR_B200_EXCHANGE=nccl)
+//      straight into the peers' buffers by the kernels of shard_peer.cu
 //   4. dir_embed_fm_fwd       runs on the received unique-row buffer, indexed by `inv`  [embed_fwd.cu]
 // Bags (CSR) take dir_shard_bag_keys instead of step 1's key kernel; everything after it is shared.
 // The reference has no counterpart: its only hook is the partitioner wrapped around the embedding
@@ -212,22 +211,6 @@ shard_bag_keys_kernel(const int64_t* __restrict__ bag_offsets, const int64_t* __
   }
 }
 
-template <int LPR>
-__global__ void __launch_bounds__(256)
-rows_gather_kernel(const float* __restrict__ table, int64_t row_stride, const float* __restrict__ lin,
-                   int64_t lin_stride, const int32_t* __restrict__ ids, int64_t n,
-                   float* __restrict__ out, int64_t out_stride) {
-  constexpr int K = LPR * 4;
-  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t i = t / LPR;
-  const int sub = (int)(t % LPR);
-  if (i >= n) return;
-  const int64_t r = __ldg(ids + i);
-  const float4 v = __ldg(reinterpret_cast<const float4*>(table + r * row_stride) + sub);
-  stg_stream(out + i * out_stride + sub * 4, v);
-  if (sub == 0) out[i * out_stride + K] = lin ? __ldg(lin + r * lin_stride) : 0.f;
-}
-
 struct UniqueWs {
   uint32_t* tilecnt;  // [tiles] head flags per tile, then their exclusive prefix
   int64_t tiles;
@@ -310,31 +293,6 @@ extern "C" int dir_shard_unique(const uint32_t* sorted_keys, const uint32_t* sor
       sorted_keys, sorted_pos, w.tilecnt, n_lookups, pruned, (uint32_t)cap, G, field_sel, n_sel, F, uidx,
       unique_local_rows, inv, owner_off);
   return launched("shard_unique", 3);
-}
-
-extern "C" int dir_rows_gather(const float* table, int64_t row_stride, const float* lin,
-                               int64_t lin_stride, const int32_t* local_rows, int64_t n, int K,
-                               float* out, int64_t out_stride, dir_stream_t stream) {
-  using namespace dir;
-  if (n < 0) return fail(DIR_EINVAL, "rows_gather: n >= 0 required");
-  if (K != 4 && K != 8 && K != 16 && K != 32 && K != 64)
-    return fail(DIR_EINVAL, "rows_gather: K must be one of 4, 8, 16, 32, 64");
-  if (n == 0) return 0;
-  if (!table || !local_rows || !out) return fail(DIR_EINVAL, "rows_gather: null pointer");
-  if (row_stride < K || (row_stride & 3) || out_stride < K + 1 || (out_stride & 3))
-    return fail(DIR_EINVAL, "rows_gather: strides must be multiples of 4, >= K (rows), >= K+1 (out)");
-  if (!aligned16(table) || !aligned16(out)) return fail(DIR_EINVAL, "rows_gather: 16-byte alignment required");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int lpr = K / 4;
-  const unsigned grid = (unsigned)((n * lpr + 255) / 256);
-  switch (lpr) {
-    case 1: rows_gather_kernel<1><<<grid, 256, 0, st>>>(table, row_stride, lin, lin_stride, local_rows, n, out, out_stride); break;
-    case 2: rows_gather_kernel<2><<<grid, 256, 0, st>>>(table, row_stride, lin, lin_stride, local_rows, n, out, out_stride); break;
-    case 4: rows_gather_kernel<4><<<grid, 256, 0, st>>>(table, row_stride, lin, lin_stride, local_rows, n, out, out_stride); break;
-    case 8: rows_gather_kernel<8><<<grid, 256, 0, st>>>(table, row_stride, lin, lin_stride, local_rows, n, out, out_stride); break;
-    default: rows_gather_kernel<16><<<grid, 256, 0, st>>>(table, row_stride, lin, lin_stride, local_rows, n, out, out_stride); break;
-  }
-  return launched("rows_gather");
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -10,15 +10,12 @@ the owner answered runs the ordinary forward kernel on the received rows; in the
 the gradients of each distinct row before shipping them, so a Zipf-hot row costs one row of traffic
 per rank and step instead of one per lookup.  One-row (numeric) fields are replicated parameters.
 
-Two exchange flavours (DIR_B200_EXCHANGE):
-  peer  (default) NVLink peer memory, driven from the device: kernels store straight into the peers'
-        exchange buffers (symmetric memory), counts travel as headers read on the device, a
-        device-side barrier separates the phases.  No NCCL, no host read: the whole step replays
-        from a CUDA graph (csrc/shard_peer.cu).  With one process the buffers are plain local memory.
-  nccl  the baseline: counts and payload through `all_to_all_single`, one host read per step.
+The exchange runs over NVLink peer memory and is driven from the device: kernels store straight into the
+peers' exchange buffers (symmetric memory), counts travel as headers read on the device, a device-side barrier
+separates the phases.  No NCCL, no host read: the whole step replays from a CUDA graph (csrc/shard_peer.cu).
+With one process the buffers are plain local memory.
 
-`ShardPlan` (pure index arithmetic) and `exchange` / `exchange_counts` (the collectives) carry no
-CUDA-only code: tests run them under gloo with world_size 2 on CPU.
+`ShardPlan` (pure index arithmetic) carries no CUDA-only code: tests run it on CPU.
 """
 import math
 import os
@@ -30,7 +27,7 @@ import torch.distributed as dist
 
 from . import _lib
 from ._lib import check, ptr
-from .layers import (_K_OK, _OPTIMIZERS, _TABLE_OPTIMIZERS, _Workspace, _need_cuda, _stream, linear_opt_struct,
+from .layers import (_K_OK, _TABLE_OPTIMIZERS, _Workspace, _need_cuda, _stream, linear_opt_struct,
                      table_opt_struct,
                      resolve_linear_optimizer)
 
@@ -65,26 +62,6 @@ class ShardPlan:
     def shard_of(self, full):
         """This rank's rows of a full [n_rows, ...] array (numpy or torch)."""
         return full[self.rank::self.world_size]
-
-
-def exchange_counts(send_counts: torch.Tensor, group=None) -> torch.Tensor:
-    """all-to-all of one int64 per peer: recv[g] = what rank g will send to this rank."""
-    if not dist.is_initialized():                 # a single process owns every row
-        return send_counts.clone()
-    recv = torch.empty_like(send_counts)
-    dist.all_to_all_single(recv, send_counts.contiguous(), group=group)
-    return recv
-
-
-def exchange(payload: torch.Tensor, send_splits, recv_splits, group=None) -> torch.Tensor:
-    """Variable-size all-to-all along dim 0: rows [sum(send_splits), ...] grouped by destination ->
-    rows [sum(recv_splits), ...] grouped by source."""
-    if not dist.is_initialized():
-        return payload.contiguous()
-    out = payload.new_empty((int(sum(recv_splits)),) + tuple(payload.shape[1:]))
-    dist.all_to_all_single(out, payload.contiguous(), output_split_sizes=list(recv_splits),
-                           input_split_sizes=list(send_splits), group=group)
-    return out
 
 
 class StageTrace:
@@ -175,17 +152,15 @@ class PeerExchange:
 class ShardedLookups:
     """What `ShardedEmbeddingFM.presort` leaves behind for one batch -- everything that depends on the
     ids only: this rank's lookups sorted by (owner, local row), the distinct rows numbered, the ids
-    already at their owners (and, NCCL flavour, the owner's list sorted for the gradient merge)."""
+    already at their owners."""
 
     def __init__(self):
-        self.ws, self.ws2, self.ws3 = _Workspace(), _Workspace(), _Workspace()
+        self.ws, self.ws2 = _Workspace(), _Workspace()
         self.keys = self.uidx = self.ulocal = self.inv = self.owner_off = self.g1_local = None
-        self.send_splits = self.recv_splits = self.recv_ids = None      # NCCL flavour
-        self.U = self.R = 0
         self.event = None
         self.src = None
         self.n_entries = 0          # lookups in the sorted list (B * sparse fields; bags: nnz)
-        self.parity = None          # which exchange buffers this batch uses (peer flavour; set by presort)
+        self.parity = None          # which exchange buffers this batch uses (set by presort)
         self.half = 0               # micro-batch of its batch (0, or 1 when the batch is exchanged as two halves)
         self.buf = None             # = parity * micro_batches + half: index of the exchange buffer / slot map
         self.gs_done = None         # event: this half's rows have been sent (the other half's exchange may start)
@@ -213,64 +188,42 @@ class _ShardedFunction(torch.autograd.Function):
         fm = torch.empty((B, 1), dtype=torch.float32, device=dev)
         first = torch.empty((B, 1), dtype=torch.float32, device=dev)
         S = torch.empty((B, K), dtype=torch.float32, device=dev) if train else None
-        ubuf = None
-        if layer.px is not None:
-            # the owner answers the ids it received: one kernel gathers the rows and stores them straight
-            # into the requesters' buffers over NVLink
-            px, p = layer.px, h.buf
-            if train:
-                # the owner marks who asked for which row (cells carry this use's epoch: nothing is cleared
-                # afterwards).  Only the owner's update needs the marks: a second stream, underneath the row exchange
-                # and the forward; the backward joins it.
-                main, aux = torch.cuda.current_stream(), layer.aux_stream(dev, h.half)
-                aux.wait_stream(main)
-                check(L.dir_shard_slots(px.ref(p), ptr(layer.slot[p]), layer.n_rows, ptr(layer.slot_epoch[p]),
-                                        ptr(layer.err_flag),
-                                        layer._n_unique2.data_ptr() + 8 * h.parity if h.half == 0 else None,
-                                        aux.cuda_stream), "dir_shard_slots")
-            check(L.dir_shard_gather_send(px.ref(p), ptr(layer.table), layer.row_stride,
-                                          ptr(layer.w1) if layer.first_order else None, layer.lin_stride,
-                                          ptr(layer.dense_table) if layer.n_dense else None, layer.row_stride,
-                                          ptr(layer.dense_lin) if (layer.n_dense and layer.first_order) else None,
-                                          layer.gather_ctas_per_sm, st), "dir_shard_gather_send")
-            h.gs_done = torch.cuda.Event()
-            h.gs_done.record()
-            tr.mark("fwd.gather+send")
-            px.barrier(p, 0)
-            layer._note_forward(h.half)
-            tr.mark("fwd.barrier")
-            rows, lin = px.rows(p), px.w(p) if layer.first_order else None
-            check(L.dir_embed_fm_fwd(ptr(rows), K, ptr(lin), 1, ptr(bias) if layer.first_order else None,
-                                     ptr(h.inv), ptr(val), ptr(layer.zero_offset), None, rows.shape[0], B, F, K,
-                                     ptr(emb), ptr(S), ptr(first), ptr(fm), None, None, st), "dir_embed_fm_fwd")
-            tr.mark("fwd.fm")
-        else:
-            U, R = h.U, h.R
-            pad = layer.pad_stride
-            answer = torch.empty((R, pad), dtype=torch.float32, device=dev)
-            check(L.dir_rows_gather(ptr(layer.table), layer.row_stride,
-                                    ptr(layer.w1) if layer.first_order else None, layer.lin_stride,
-                                    ptr(h.recv_ids), R, K, ptr(answer), pad, st), "dir_rows_gather")
-            tr.mark("fwd.gather")
-            ubuf = exchange(answer, h.recv_splits, h.send_splits, layer.group)          # [U, K+4]
-            tr.mark("fwd.a2a_rows")
-            if U == 0:
-                ubuf = torch.zeros((1, pad), dtype=torch.float32, device=dev)
-            lin = ubuf[:, K] if layer.first_order else None
-            check(L.dir_embed_fm_fwd(ptr(ubuf), pad, ptr(lin), pad, ptr(bias) if layer.first_order else None,
-                                     ptr(h.inv), ptr(val), ptr(layer.zero_offset), None, max(U, 1), B, F, K,
-                                     ptr(emb), ptr(S), ptr(first), ptr(fm), None, None, st), "dir_embed_fm_fwd")
-            tr.mark("fwd.fm")
+        # the owner answers the ids it received: one kernel gathers the rows and stores them straight
+        # into the requesters' buffers over NVLink
+        px, p = layer.px, h.buf
+        if train:
+            # the owner marks who asked for which row (cells carry this use's epoch: nothing is cleared
+            # afterwards).  Only the owner's update needs the marks: a second stream, underneath the row exchange
+            # and the forward; the backward joins it.
+            main, aux = torch.cuda.current_stream(), layer.aux_stream(dev, h.half)
+            aux.wait_stream(main)
+            check(L.dir_shard_slots(px.ref(p), ptr(layer.slot[p]), layer.n_rows, ptr(layer.slot_epoch[p]),
+                                    ptr(layer.err_flag),
+                                    layer._n_unique2.data_ptr() + 8 * h.parity if h.half == 0 else None,
+                                    aux.cuda_stream), "dir_shard_slots")
+        check(L.dir_shard_gather_send(px.ref(p), ptr(layer.table), layer.row_stride,
+                                      ptr(layer.w1) if layer.first_order else None, layer.lin_stride,
+                                      ptr(layer.dense_table) if layer.n_dense else None, layer.row_stride,
+                                      ptr(layer.dense_lin) if (layer.n_dense and layer.first_order) else None,
+                                      layer.gather_ctas_per_sm, st), "dir_shard_gather_send")
+        h.gs_done = torch.cuda.Event()
+        h.gs_done.record()
+        tr.mark("fwd.gather+send")
+        px.barrier(p, 0)
+        layer._note_forward(h.half)
+        tr.mark("fwd.barrier")
+        rows, lin = px.rows(p), px.w(p) if layer.first_order else None
+        check(L.dir_embed_fm_fwd(ptr(rows), K, ptr(lin), 1, ptr(bias) if layer.first_order else None,
+                                 ptr(h.inv), ptr(val), ptr(layer.zero_offset), None, rows.shape[0], B, F, K,
+                                 ptr(emb), ptr(S), ptr(first), ptr(fm), None, None, st), "dir_embed_fm_fwd")
+        tr.mark("fwd.fm")
         if not layer.first_order:
             first.zero_()
         ctx.layer, ctx.train, ctx.shape, ctx.h = layer, train, (B, F, K), h
         ctx.idx, ctx.defer = idx, defer
         ctx.set_materialize_grads(False)
         if train:
-            if ubuf is None:
-                ctx.save_for_backward(val, S)
-            else:
-                ctx.save_for_backward(val, S, ubuf)
+            ctx.save_for_backward(val, S)
         if emb is None:
             emb = torch.empty((B, 0), dtype=torch.float32, device=dev)
             ctx.mark_non_differentiable(emb)
@@ -284,11 +237,7 @@ class _ShardedFunction(torch.autograd.Function):
         B, F, K = ctx.shape
         L = _lib.lib()
         st = _stream()
-        if layer.px is not None:
-            val, S = ctx.saved_tensors
-            ubuf = None
-        else:
-            val, S, ubuf = ctx.saved_tensors
+        val, S = ctx.saved_tensors
         dev = S.device
         g_first = (torch.zeros(B, dtype=torch.float32, device=dev) if g_first is None
                    else g_first.reshape(B).contiguous().float())
@@ -299,71 +248,42 @@ class _ShardedFunction(torch.autograd.Function):
         tr = layer.trace
         tr.mark("between")
         g_bias = None
-        adagrad = layer.optimizer == "adagrad"
         gfp = ptr(g_first) if layer.first_order else None
         n_keys = layer.plan.cap * layer.plan.world_size
         with torch.no_grad():
-            if layer.px is not None:
-                px, p = layer.px, h.buf
-                n = B * layer.n_sel
-                # Next to the segmented reduce, on a second stream: the replicated one-row fields' column sums over
-                # this rank's samples -> every rank's buffer, and the bias gradient.
-                main, aux = torch.cuda.current_stream(), layer.aux_stream(dev, h.half)
-                aux.wait_stream(main)
-                with torch.cuda.stream(aux):
-                    if layer.first_order:
-                        g_bias = g_first.sum().reshape(1)
-                        g_bias.record_stream(main)
-                    if layer.n_dense:
-                        ows = layer._dense_ws[h.half].get(L.dir_shard_dense_workspace_bytes(K), dev)
-                        check(L.dir_shard_dense_emit(
-                            px.ref(p), ptr(layer.dense_table), layer.row_stride, ptr(ctx.idx), ptr(val),
-                            ptr(layer.dense_field_offset), gfp, ptr(g_fm), ptr(S), ptr(u), ptr(layer.onerow_fields), B, F,
-                            ptr(ows), ows.numel(), aux.cuda_stream), "dir_shard_dense_emit")
-                # per-distinct-row sums on the requester (the sorted list is in the handle's workspace), each
-                # stored straight into its owner's buffer over NVLink as soon as its run is summed
-                ws = h.ws.get(L.dir_embed_bwd_workspace_bytes(max(n, 1), K), dev)
-                check(L.dir_embed_bwd_reduce_emit_to(
-                    px.ref(p), ptr(val), gfp, ptr(g_fm), ptr(S), ptr(u), ptr(h.uidx), ptr(h.owner_off), B, F, n_keys,
-                    ptr(layer.sparse_fields) if layer.n_sel < F else None, layer.n_sel, ptr(h.g1_local),
-                    ptr(ws), ws.numel(), st), "dir_embed_bwd_reduce_emit_to")
-                check(L.dir_shard_g1_push(px.ref(p), ptr(h.g1_local), ptr(h.owner_off), n, st), "dir_shard_g1_push")
-                main.wait_stream(aux)
-                tr.mark("bwd.emit+push")
-                if not ctx.defer:
-                    layer._owner_step([h])
-            else:
-                U, R = h.U, h.R
-                pad = layer.pad_stride
-                n = B * F
-                ws = h.ws.get(L.dir_embed_bwd_workspace_bytes(n, K), dev)
-                gu = torch.empty((max(U, 1), pad), dtype=torch.float32, device=dev)
-                check(L.dir_embed_bwd_reduce_emit(ptr(ubuf), pad, ptr(val), gfp, ptr(g_fm), ptr(S), ptr(u),
-                                                  ptr(h.uidx), B, F, K, n_keys, ptr(gu), pad,
-                                                  ptr(ws), ws.numel(), st), "dir_embed_bwd_reduce_emit")
-                tr.mark("bwd.emit")
-                grecv = exchange(gu[:U], h.send_splits, h.recv_splits, layer.group)      # [R, K+4]
-                tr.mark("bwd.a2a_grads")
-                if R > 0:
-                    ws3 = h.ws3.get(L.dir_embed_bwd_workspace_bytes(R, K), dev)     # sorted by presort
-                    check(L.dir_rows_reduce_update(
-                        ptr(layer.table), ptr(layer.accum) if adagrad else None, layer.row_stride,
-                        ptr(layer.w1) if layer.first_order else None,
-                        ptr(layer.w1_accum) if layer.first_order else None, layer.lin_stride,
-                        ptr(grecv), pad, R, K, layer.plan.cap, _OPTIMIZERS[layer.optimizer], layer.lr,
-                        linear_opt_struct(layer), None,
-                        ptr(ws3), ws3.numel(), layer._n_unique2.data_ptr(), st), "dir_rows_reduce_update")
-                    tr.mark("bwd.owner_update")
-                else:
-                    layer._n_unique2.zero_()
-                layer._last_parity = 0
+            px, p = layer.px, h.buf
+            n = B * layer.n_sel
+            # Next to the segmented reduce, on a second stream: the replicated one-row fields' column sums over
+            # this rank's samples -> every rank's buffer, and the bias gradient.
+            main, aux = torch.cuda.current_stream(), layer.aux_stream(dev, h.half)
+            aux.wait_stream(main)
+            with torch.cuda.stream(aux):
+                if layer.first_order:
+                    g_bias = g_first.sum().reshape(1)
+                    g_bias.record_stream(main)
+                if layer.n_dense:
+                    ows = layer._dense_ws[h.half].get(L.dir_shard_dense_workspace_bytes(K), dev)
+                    check(L.dir_shard_dense_emit(
+                        px.ref(p), ptr(layer.dense_table), layer.row_stride, ptr(ctx.idx), ptr(val),
+                        ptr(layer.dense_field_offset), gfp, ptr(g_fm), ptr(S), ptr(u), ptr(layer.onerow_fields), B, F,
+                        ptr(ows), ows.numel(), aux.cuda_stream), "dir_shard_dense_emit")
+            # per-distinct-row sums on the requester (the sorted list is in the handle's workspace), each
+            # stored straight into its owner's buffer over NVLink as soon as its run is summed
+            ws = h.ws.get(L.dir_embed_bwd_workspace_bytes(max(n, 1), K), dev)
+            check(L.dir_embed_bwd_reduce_emit_to(
+                px.ref(p), ptr(val), gfp, ptr(g_fm), ptr(S), ptr(u), ptr(h.uidx), ptr(h.owner_off), B, F, n_keys,
+                ptr(layer.sparse_fields) if layer.n_sel < F else None, layer.n_sel, ptr(h.g1_local),
+                ptr(ws), ws.numel(), st), "dir_embed_bwd_reduce_emit_to")
+            check(L.dir_shard_g1_push(px.ref(p), ptr(h.g1_local), ptr(h.owner_off), n, st), "dir_shard_g1_push")
+            main.wait_stream(aux)
+            tr.mark("bwd.emit+push")
+            if not ctx.defer:
+                layer._owner_step([h])
             tr.close_step()
         if h is layer._inline:
             layer._inline_busy = False
-        if layer.px is not None and not ctx.defer:
+        if not ctx.defer:
             layer._in_flight[h.buf] = False
-        if g_bias is None and layer.first_order:
-            g_bias = g_first.sum().reshape(1)
         return None, g_bias, None, None, None, None, None, None
 
 
@@ -375,8 +295,7 @@ class ShardedEmbeddingFM(torch.nn.Module):
     rows this rank owns with the gradients of every rank's samples.  `bias` is an ordinary
     replicated parameter: all-reduce its gradient like any dense parameter.
 
-    `max_batch` sizes the exchange buffers (peer flavour).  `presort` may run at most one batch ahead
-    of `forward`.
+    `max_batch` sizes the exchange buffers.  `presort` may run at most one batch ahead of `forward`.
     """
 
     def __init__(self, field_size: int, embedding_size: int, rows_per_field: Sequence[int],
@@ -401,8 +320,6 @@ class ShardedEmbeddingFM(torch.nn.Module):
         self.optimizer_l1, self.optimizer_l2 = float(optimizer_l1), float(optimizer_l2)
         if self.optimizer_l1 < 0 or self.optimizer_l2 < 0:
             raise ValueError("optimizer_l1 / optimizer_l2 must be >= 0")
-        if optimizer == "proximal_adagrad" and os.environ.get("DIR_B200_EXCHANGE", "peer") != "peer":
-            raise ValueError("proximal_adagrad needs the peer-memory exchange (DIR_B200_EXCHANGE=peer)")
         if init not in ("trunc_normal", "counter", "none"):
             raise ValueError("init must be 'trunc_normal', 'counter' or 'none'")
         self.l1, self.l2 = float(l1_regularization_strength), float(l2_regularization_strength)
@@ -422,7 +339,6 @@ class ShardedEmbeddingFM(torch.nn.Module):
         adagrad = optimizer != "sgd"                                # the rule keeps an accumulator next to the row
         self.row_stride = 2 * K if adagrad else K
         self.lin_stride = 1
-        self.pad_stride = K + 4                                     # NCCL flavour: (row[K], first-order weight, 3 pad)
         self.n_rows = max(self.plan.cap, 1)                         # local rows allocated
         self.max_batch = int(max_batch)
         dev = torch.device(device)
@@ -448,43 +364,32 @@ class ShardedEmbeddingFM(torch.nn.Module):
         self.gather_ctas_per_sm = 8 if self.micro_batches == 1 else 3
         self.trace, self.trace_pre = StageTrace(), StageTrace()
         self.capturing = False
-        self.exchange_mode = os.environ.get("DIR_B200_EXCHANGE", "peer")
-        if self.exchange_mode not in ("peer", "nccl"):
-            raise ValueError("DIR_B200_EXCHANGE must be 'peer' or 'nccl'")
         if dev.type != "cuda":
             raise ValueError("ShardedEmbeddingFM needs a CUDA device: this layer has no CPU path")
-        if self.exchange_mode == "peer" and world > 1 and dist.get_backend(process_group) != "nccl":
+        if world > 1 and dist.get_backend(process_group) != "nccl":
             raise ValueError("the peer-memory exchange needs the nccl backend (one process per GPU)")
-        # One-row (numeric) fields are replicated parameters in the peer flavour: every sample of every rank hits
-        # the same row, so they stay out of the sort and the exchange; their gradients are column sums.
-        onerow = ([f for f, r in enumerate(rows) if r == 1][:64]
-                  if (self.exchange_mode == "peer" and replicate_onerow) else [])
+        # One-row (numeric) fields are replicated parameters: every sample of every rank hits the same row, so they
+        # stay out of the sort and the exchange; their gradients are column sums.
+        onerow = [f for f, r in enumerate(rows) if r == 1][:64] if replicate_onerow else []
         sparse = [f for f in range(field_size) if f not in set(onerow)]
         self.n_dense, self.n_sel = len(onerow), len(sparse)
         self.register_buffer("onerow_fields", torch.tensor(onerow or [0], dtype=torch.int32, device=dev))
         self.register_buffer("sparse_fields", torch.tensor(sparse or [0], dtype=torch.int32, device=dev))
-        self.px, self.slot, self.slot_epoch = None, None, None
         self._ids_issued = self._fwd_issued = 0       # batches (their half 0) whose id exchange / forward was issued
         self._fwd_event = None
-        # the id exchange of the NEXT batch runs concurrently with this batch's row / gradient exchange: the NCCL
-        # flavour gives it a communicator of its own so the two never queue behind each other
-        self.side_group = process_group
-        if self.exchange_mode == "peer":
-            # lookups of one batch that go through the exchange (bags: entries, `max_entries`)
-            self.max_entries = int(max_entries) if max_entries else self.max_batch * max(self.n_sel, 1)
-            seg_cap = max(1, min(self.max_entries, cap))   # rows one requester can ask of one owner
-            u_cap = max(1, self.max_entries)               # distinct rows a requester can ask for
-            if seg_cap >= 1 << 24:
-                raise ValueError("max_batch * sparse fields must stay below 2^24 rows per requester and owner")
-            if self.micro_batches == 2 and world > 32:
-                raise ValueError("two micro-batches need world_size <= 32")
-            n_buf = 2 * self.micro_batches          # two parities (consecutive steps alternate) x micro-batches
-            self.px = PeerExchange(process_group, world, rank, K, self.n_dense, seg_cap, u_cap, dev, n_buf)
-            # who asked for which of my rows: one cell per (local row, requester), tagged with the buffer's epoch
-            self.slot = [torch.zeros(cap * world, dtype=torch.int32, device=dev) for _ in range(n_buf)]
-            self.slot_epoch = [torch.zeros(2, dtype=torch.int32, device=dev) for _ in range(n_buf)]
-        elif dist.is_initialized() and dist.get_backend(process_group) == "nccl":
-            self.side_group = dist.new_group(ranks=dist.get_process_group_ranks(process_group or dist.group.WORLD))
+        # lookups of one batch that go through the exchange (bags: entries, `max_entries`)
+        self.max_entries = int(max_entries) if max_entries else self.max_batch * max(self.n_sel, 1)
+        seg_cap = max(1, min(self.max_entries, cap))   # rows one requester can ask of one owner
+        u_cap = max(1, self.max_entries)               # distinct rows a requester can ask for
+        if seg_cap >= 1 << 24:
+            raise ValueError("max_batch * sparse fields must stay below 2^24 rows per requester and owner")
+        if self.micro_batches == 2 and world > 32:
+            raise ValueError("two micro-batches need world_size <= 32")
+        n_buf = 2 * self.micro_batches          # two parities (consecutive steps alternate) x micro-batches
+        self.px = PeerExchange(process_group, world, rank, K, self.n_dense, seg_cap, u_cap, dev, n_buf)
+        # who asked for which of my rows: one cell per (local row, requester), tagged with the buffer's epoch
+        self.slot = [torch.zeros(cap * world, dtype=torch.int32, device=dev) for _ in range(n_buf)]
+        self.slot_epoch = [torch.zeros(2, dtype=torch.int32, device=dev) for _ in range(n_buf)]
         with torch.no_grad():
             sd = 1.0 / math.sqrt(K)
             if init == "trunc_normal":
@@ -698,8 +603,8 @@ class ShardedEmbeddingFM(torch.nn.Module):
     def finish_step(self, handle_a, handle_b):
         """After the backward of both micro-batches of a batch (run with `defer_update=True`): the one owner update
         of the batch.  Call it on the stream both backwards have been joined into."""
-        if self.px is None or self.micro_batches != 2:
-            raise RuntimeError("finish_step needs the peer exchange with micro_batches=2")
+        if self.micro_batches != 2:
+            raise RuntimeError("finish_step needs micro_batches=2")
         if handle_a.parity != handle_b.parity or (handle_a.half, handle_b.half) != (0, 1):
             raise ValueError("finish_step takes the two halves (0, 1) of one batch")
         self._owner_step([handle_a, handle_b])
@@ -724,8 +629,7 @@ class ShardedEmbeddingFM(torch.nn.Module):
         dev = idx.device
         L = _lib.lib()
         st = _stream()
-        peer = self.px is not None
-        n_sel = self.n_sel if peer else F
+        n_sel = self.n_sel
         n = B * n_sel
         tr = self.trace_pre
         tr.mark("pre.start")
@@ -738,8 +642,8 @@ class ShardedEmbeddingFM(torch.nn.Module):
             h.owner_off = torch.zeros(G + 1, dtype=torch.int64, device=dev)
             h.shape = (B, F)
         h.n_entries = n
-        sel = ptr(self.sparse_fields) if (peer and n_sel < F) else None
-        if peer and self.n_dense:
+        sel = ptr(self.sparse_fields) if n_sel < F else None
+        if self.n_dense:
             # the replicated one-row fields' part of `inv` needs the inputs only: first, off the chain that ends in
             # the id exchange (keys -> sort -> numbering -> push)
             check(L.dir_shard_dense_inv(ptr(idx), ptr(val), ptr(self.onerow_fields), self.n_dense, B, F,
@@ -764,47 +668,28 @@ class ShardedEmbeddingFM(torch.nn.Module):
 
     @torch.no_grad()
     def id_exchange(self, h):
-        """Ships the distinct ids to their owners (current stream).  Peer flavour: header + ids stored into the
-        owners' buffers, a device-side barrier, then the owner marks who asked for which row.  NCCL flavour: counts
-        and ids through all-to-all, one host read, then the owner's sort for the gradient merge."""
+        """Ships the distinct ids to their owners (current stream): header + ids stored into the owners' buffers,
+        a device-side barrier, then the owner marks who asked for which row."""
         L = _lib.lib()
         st = _stream()
         tr = self.trace_pre
-        B, F = h.shape
-        K = self.embedding_size
-        dev = h.keys.device
-        if self.px is not None:
-            if h.half == 0:
-                if self._ids_issued - self._fwd_issued >= 2 and not self.capturing:
-                    raise RuntimeError("ShardedEmbeddingFM.presort may run at most one batch ahead of forward")
-                if h.parity is None or not self.capturing:
-                    h.parity = self._ids_issued % 2
-                self._ids_issued += 1
-            elif h.parity is None or not self.capturing:
-                h.parity = (self._ids_issued - 1) % 2          # the second half follows its batch's first half
-            h.buf = h.parity * self.micro_batches + h.half
-            p, px = h.buf, self.px
-            if self._fwd_event is not None and not self.capturing:
-                torch.cuda.current_stream().wait_event(self._fwd_event)     # every rank is done with parity p
-            check(L.dir_shard_ids_push(px.ref(p), ptr(h.ulocal), ptr(h.owner_off), h.n_entries,
-                                       ptr(self.err_flag), ptr(self.slot_epoch[p]), st), "dir_shard_ids_push")
-            tr.mark("pre.ids_push")
-            px.barrier(p, 1)
-            tr.mark("pre.barrier")
-            return
-        send_counts = h.owner_off[1:] - h.owner_off[:-1]
-        recv_counts = exchange_counts(send_counts, self.side_group)
-        both = torch.stack([send_counts, recv_counts]).cpu()        # the one host read of a step
-        h.send_splits, h.recv_splits = both[0].tolist(), both[1].tolist()
-        h.U, h.R = int(sum(h.send_splits)), int(sum(h.recv_splits))
-        tr.mark("pre.counts+sync")
-        h.recv_ids = exchange(h.ulocal[:h.U], h.send_splits, h.recv_splits, self.side_group)
-        tr.mark("pre.a2a_ids")
-        if h.R > 0:                     # the owner's half: arrival order -> local-row order
-            ws3 = h.ws3.get(L.dir_embed_bwd_workspace_bytes(h.R, K), dev)
-            check(L.dir_embed_bwd_sort(ptr(h.recv_ids), h.R, self.plan.cap, ptr(ws3), ws3.numel(), st),
-                  "dir_embed_bwd_sort")
-        tr.mark("pre.owner_sort")
+        if h.half == 0:
+            if self._ids_issued - self._fwd_issued >= 2 and not self.capturing:
+                raise RuntimeError("ShardedEmbeddingFM.presort may run at most one batch ahead of forward")
+            if h.parity is None or not self.capturing:
+                h.parity = self._ids_issued % 2
+            self._ids_issued += 1
+        elif h.parity is None or not self.capturing:
+            h.parity = (self._ids_issued - 1) % 2          # the second half follows its batch's first half
+        h.buf = h.parity * self.micro_batches + h.half
+        p, px = h.buf, self.px
+        if self._fwd_event is not None and not self.capturing:
+            torch.cuda.current_stream().wait_event(self._fwd_event)     # every rank is done with parity p
+        check(L.dir_shard_ids_push(px.ref(p), ptr(h.ulocal), ptr(h.owner_off), h.n_entries,
+                                   ptr(self.err_flag), ptr(self.slot_epoch[p]), st), "dir_shard_ids_push")
+        tr.mark("pre.ids_push")
+        px.barrier(p, 1)
+        tr.mark("pre.barrier")
 
     @torch.no_grad()
     def presort(self, feature_index, feature_value=None, handle=None, after=None, fork=True, inline=False,
@@ -816,7 +701,7 @@ class ShardedEmbeddingFM(torch.nn.Module):
         ids are already on the device, or `after` marks their arrival).  `inline=True`: on the current stream (a
         caller that captures CUDA graphs places the two phases itself).  At most one batch ahead of `forward`."""
         idx, val = self._prepare(feature_index, feature_value)
-        if self.px is not None and idx.shape[0] > self.max_batch:
+        if idx.shape[0] > self.max_batch:
             raise ValueError("batch %d exceeds max_batch=%d the exchange buffers were sized for" % (
                 idx.shape[0], self.max_batch))
         if phase not in ("both", "local", "exchange"):
@@ -854,8 +739,8 @@ class ShardedEmbeddingFM(torch.nn.Module):
         `finish_step(half0, half1)` after both halves' backward."""
         idx, val = self._prepare(feature_index, feature_value)
         train = self.training and torch.is_grad_enabled()
-        if defer_update and (self.px is None or self.micro_batches != 2 or presorted is None):
-            raise ValueError("defer_update needs micro_batches=2, the peer exchange and a presorted handle")
+        if defer_update and (self.micro_batches != 2 or presorted is None):
+            raise ValueError("defer_update needs micro_batches=2 and a presorted handle")
         if presorted is None:
             # the layer's own handle serves one forward at a time (a second forward before the first one's backward
             # gets a handle of its own)
@@ -865,7 +750,7 @@ class ShardedEmbeddingFM(torch.nn.Module):
                 self._inline_busy = True
         elif presorted.src != ShardedLookups.key_of(feature_index, feature_value):
             raise ValueError("presorted handle was made for other feature_index / feature_value tensors")
-        if self.px is not None and train:
+        if train:
             if self._in_flight[presorted.buf] and not self.capturing:
                 raise RuntimeError("ShardedEmbeddingFM: two exchange buffers = at most two batches between forward and "
                                    "backward; run the backward of an earlier batch first")
@@ -973,7 +858,7 @@ class ShardedEmbeddingBagFM(ShardedEmbeddingFM):
     bag_index[nnz], bag_weight[nnz] | None)` for THIS rank's samples; `.backward()` updates the rows this rank
     owns with every rank's gradients.  Every field goes through the exchange (a bag of a one-row field still has
     a length and weights).  `max_entries` bounds nnz of one call (it sizes the exchange buffers; default
-    max_batch * field_size).  Peer-memory exchange only; one batch at a time (no `presort`, no micro-batches)."""
+    max_batch * field_size).  One batch at a time (no `presort`, no micro-batches)."""
 
     def __init__(self, field_size, embedding_size, rows_per_field, combiner="mean", max_entries=None, **kw):
         if combiner not in _COMBINER_CODE:
@@ -982,8 +867,6 @@ class ShardedEmbeddingBagFM(ShardedEmbeddingFM):
             raise ValueError("ShardedEmbeddingBagFM exchanges a batch in one piece: micro_batches must be 1")
         super().__init__(field_size, embedding_size, rows_per_field, replicate_onerow=False,
                          max_entries=max_entries, **kw)
-        if self.px is None:
-            raise ValueError("ShardedEmbeddingBagFM needs the peer-memory exchange (DIR_B200_EXCHANGE=peer)")
         self.combiner = combiner
         self._bag_handle = ShardedLookups()
 

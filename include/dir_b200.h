@@ -222,7 +222,7 @@ int dir_embed_bwd_sorted(const void* workspace, int64_t n_lookups, const uint32_
  * sharded by row and ids / IndexedSlices travel over gRPC).  Here only DISTINCT rows travel,
  * once per step in each direction.
  *
- * Id-only part (both exchange flavours):
+ * Id-only part:
  * dir_shard_keys: keys[b*n_sel + j] = owner * cap + local row of field field_sel[j], cap = ceil(n_rows / G);
  *   pruned lookups (id < 0, value <= 0, id beyond its field) get G * cap, the `n_rows` to pass to
  *   dir_embed_bwd_sort.  With G = 1 the key is the global row: this is also how the single-GPU layer forms
@@ -263,37 +263,7 @@ int dir_shard_dense_inv(const int64_t* feature_index, const float* feature_value
                         const int32_t* onerow_fields, int n_onerow, int64_t B, int F, int64_t tail_row,
                         int64_t* inv, int* oob_flag, dir_stream_t stream);
 
-/* Exchange over NCCL all-to-all, issued by the host layer (DIR_B200_EXCHANGE=nccl; the baseline):
- *   requester                                          owner
- *   dir_shard_keys / dir_embed_bwd_sort / dir_shard_unique  --ids-->  dir_rows_gather  (row | first-order weight)
- *   dir_embed_fm_fwd    on the returned buffer <-rows--
- *   dir_embed_bwd_reduce_emit  per-row sums   --grads-> dir_embed_bwd_sort + dir_rows_reduce_update
- * dir_rows_gather: out[i, 0:K] = table[local_rows[i]], out[i, K] = lin[local_rows[i]] (0 if lin is
- *   NULL); out rows are out_stride floats apart (multiple of 4, >= K + 1).
- * dir_embed_bwd_reduce_emit: as dir_embed_bwd_reduce_update, but rows are read from the exchanged
- *   buffer `ubuf` at uidx[i] and each distinct row's (G[K], g1) is written to gu[u] instead of
- *   being applied.  Deterministic, same chunking.
- * dir_rows_reduce_update: the owner's half.  gbuf[j] = (G[K], g1) received for the j-th id it
- *   answered; dir_embed_bwd_sort(ids, n, n_local_rows) must have run on `workspace`.  Sums the
- *   contributions of each local row in arrival order (source rank major) and applies the update.
- *   n_device (device int64, may be NULL): the number of entries really in the list when `n` is only a bound.
- */
-int dir_rows_gather(const float* table, int64_t row_stride, const float* lin, int64_t lin_stride,
-                    const int32_t* local_rows, int64_t n, int K, float* out, int64_t out_stride,
-                    dir_stream_t stream);
-int dir_embed_bwd_reduce_emit(const float* ubuf, int64_t ubuf_stride, const float* feature_value,
-                              const float* g_first, const float* g_fm, const float* S, const float* u,
-                              const uint32_t* uidx, int64_t B, int F, int K, int64_t n_keys, float* gu,
-                              int64_t gu_stride, void* workspace, size_t workspace_bytes,
-                              dir_stream_t stream);
-int dir_rows_reduce_update(float* table, float* accum, int64_t row_stride, float* lin,
-                           float* lin_accum, int64_t lin_stride, const float* gbuf,
-                           int64_t gbuf_stride, int64_t n, int K, int64_t n_rows, int optimizer,
-                           float lr, const dir_linear_opt* linear_opt, const int64_t* n_device,
-                           void* workspace, size_t workspace_bytes, int64_t* n_unique_out,
-                           dir_stream_t stream);
-
-/* Exchange over NVLink peer memory, driven from the device (the default; csrc/shard_peer.cu).  No NCCL and
+/* Exchange over NVLink peer memory, driven from the device (csrc/shard_peer.cu).  No NCCL and
  * no host read on the step: data-dependent counts travel as headers and are read by the kernels, every
  * launch is sized by capacities, so the whole step -- id phase included -- replays from a CUDA graph.
  * Every rank allocates one exchange buffer per parity (consecutive steps alternate) with the layout below
@@ -357,8 +327,9 @@ int dir_shard_gather_send(const dir_peer_layout* layout, const float* table, int
                           const float* lin, int64_t lin_stride, const float* dense_table,
                           int64_t dense_row_stride, const float* dense_lin, int ctas_per_sm,
                           dir_stream_t stream);
-/* dir_embed_bwd_reduce_emit with the transfer fused in: each distinct row's G[K] is stored straight into its
- * owner's buffer over NVLink as soon as its run is summed (no round trip through HBM, the NVLink stores overlap
+/* The requester's per-distinct-row gradient sums (the chunking of dir_embed_bwd_reduce_update, rows read from
+ * the exchanged rows at uidx[i]): each distinct row's G[K] is stored straight into its owner's buffer over NVLink
+ * as soon as its run is summed (no round trip through HBM, the NVLink stores overlap
  * the kernel's gathers); g1 goes to g1_local[u] and is shipped by dir_shard_g1_push.  The sorted list covers
  * the fields field_sel[n_sel] (NULL: all); owner_off[G+1] as written by dir_shard_unique. */
 int dir_embed_bwd_reduce_emit_to(const dir_peer_layout* layout, const float* feature_value,

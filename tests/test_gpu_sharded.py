@@ -177,10 +177,10 @@ CASES = {"small": ([50, 1, 9, 1000, 3, 17, 1], 16, 96),          # at world 8: c
          "wide": ([300, 1, 400, 350, 1, 500], 8, 600)}           # at world 2: ceil(n_rows / G) = 776 < ~1 200 distinct rows
 
 
-def _rank_main(rank, world, port, out, exchange_mode, case_name="small"):
+def _rank_main(rank, world, port, out, case_name="small"):
     import torch.distributed as dist
     import dir_b200
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), DIR_B200_EXCHANGE=exchange_mode)
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     torch.cuda.set_device(rank)
     dist.init_process_group("nccl", rank=rank, world_size=world, device_id=torch.device("cuda", rank))
     try:
@@ -194,7 +194,6 @@ def _rank_main(rank, world, port, out, exchange_mode, case_name="small"):
         sl = slice(rank * Bl, (rank + 1) * Bl)
         layer = dir_b200.ShardedEmbeddingFM(F, K, rows, optimizer="adagrad", lr=0.05, max_batch=Bl,
                                             device="cuda").train()
-        assert (layer.px is not None) == (exchange_mode == "peer"), "exchange mode not honoured"
         layer.load_tables(case["table"], case["w1"])
         d = "cuda"
         first, fm, emb = layer(to_dev(case["idx"][sl], d), to_dev(case["val"][sl], d))
@@ -206,8 +205,7 @@ def _rank_main(rank, world, port, out, exchange_mode, case_name="small"):
                 + (emb * to_dev(u[sl].reshape(Bl, -1), d)).sum())
         loss.backward()
         torch.cuda.synchronize()
-        if exchange_mode == "peer":
-            layer.check_errors()
+        layer.check_errors()
         shards = [torch.empty_like(layer.rows) for _ in range(world)]
         lins = [torch.empty_like(layer.lin_rows) for _ in range(world)]
         dist.all_gather(shards, layer.rows)
@@ -232,7 +230,7 @@ def _rank_main(rank, world, port, out, exchange_mode, case_name="small"):
             assert np.array_equal(full[:N, :K][untouched], case["table"][untouched])
             floor = 0.1 + 2 * np.abs(G) * np.abs(G)
             assert rel_err(full[:N, K:][urows], acc[urows], floor + 1e-3) <= 10 * REL
-        if exchange_mode == "peer" and layer.n_dense:
+        if layer.n_dense:
             # every rank's replica of a one-row field equals the owner's row of the sharded table
             for j, g in enumerate(layer.dense_global_rows):
                 own = [torch.zeros_like(layer.dense_rows[j]) for _ in range(world)]
@@ -246,8 +244,7 @@ def _rank_main(rank, world, port, out, exchange_mode, case_name="small"):
         f2, m2, e2 = layer(idx2, val2, presorted=h)
         (f2.sum() + m2.sum() + e2.sum()).backward()
         torch.cuda.synchronize()
-        if exchange_mode == "peer":
-            layer.check_errors()
+        layer.check_errors()
         if rank == 0:
             e_want, _ = O.embedding_lookup(full[:N, :K], case["off"], case["idx"][sl], case["val"][sl], "sum", np.float32)
             assert np.array_equal(e2.detach().cpu().numpy().reshape(Bl, F, K), e_want), "step 2 must see step 1's rows"
@@ -260,15 +257,15 @@ def _rank_main(rank, world, port, out, exchange_mode, case_name="small"):
 
 
 @pytest.mark.parametrize("world", [2, 4, 8])
-@pytest.mark.parametrize("exchange_mode,case_name", [("peer", "small"), ("peer", "wide"), ("nccl", "small")])
-def test_multi_rank_matches_oracle(pkg, cuda, exchange_mode, case_name, world):
+@pytest.mark.parametrize("case_name", [pytest.param("small", id="peer-small"), pytest.param("wide", id="peer-wide")])
+def test_multi_rank_matches_oracle(pkg, cuda, case_name, world):
     if torch.cuda.device_count() < world:
         pytest.skip("needs %d GPUs (gpurun --gpus %d)" % (world, world))
     import torch.multiprocessing as mp
     ctx = mp.get_context("spawn")
     out = ctx.Queue()
     port = _free_port()
-    procs = [ctx.Process(target=_rank_main, args=(r, world, port, out, exchange_mode, case_name)) for r in range(world)]
+    procs = [ctx.Process(target=_rank_main, args=(r, world, port, out, case_name)) for r in range(world)]
     for p in procs:
         p.start()
     res = [out.get(timeout=300) for _ in procs]
@@ -358,7 +355,7 @@ def test_world1_two_micro_batches(pkg, cuda, B, rows, K):
 def _rank_main_micro(rank, world, port, out):
     import torch.distributed as dist
     import dir_b200
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), DIR_B200_EXCHANGE="peer")
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     torch.cuda.set_device(rank)
     dist.init_process_group("nccl", rank=rank, world_size=world, device_id=torch.device("cuda", rank))
     try:
