@@ -254,9 +254,8 @@ static CrossBwdWs cross_carve(void* base, int64_t B, int d, int L) {
 template <int VEC, int NPL>
 __global__ void __launch_bounds__(kCrossWarps * 32)
 cross_bwd_sample_kernel(const float* __restrict__ x0g, const float* __restrict__ wg,
-                        const float* __restrict__ bg, const float* __restrict__ dyg,
-                        const float* __restrict__ sg, int64_t B, int d, int L,
-                        float* __restrict__ dx0g, float* __restrict__ alpha,
+                        const float* __restrict__ bg, const float* __restrict__ dyg, int64_t B, int d,
+                        int L, float* __restrict__ dx0g, float* __restrict__ alpha,
                         float* __restrict__ Dpart, float* __restrict__ dypart) {
   constexpr int E = VEC * NPL;
   extern __shared__ float smem[];  // [kCrossWarps][d] then [kCrossWarps][32]
@@ -287,37 +286,34 @@ cross_bwd_sample_kernel(const float* __restrict__ x0g, const float* __restrict__
         accDy[i * VEC + e] += dx[i * VEC + e];
       }
     }
-    // s_l = x_l . w_l : lane l keeps s_l.  Saved by the forward, or recomputed here.
+    // s_l = x_l . w_l : lane l keeps s_l.  Always recomputed layer by layer: the forward saves
+    // p_l = x0 . w_l, not s_l, and this pass needs s_l.
     float s_mine = 0.f;
-    if (sg) {
-      if (lane < L) s_mine = __ldg(sg + b * L + lane);
-    } else {
-      float xl[E];
+    float xl[E];
 #pragma unroll
-      for (int e = 0; e < E; ++e) xl[e] = x0[e];
-      for (int l = 0; l < L; ++l) {
-        float dot = 0.f;
-        float bv[E];
+    for (int e = 0; e < E; ++e) xl[e] = x0[e];
+    for (int l = 0; l < L; ++l) {
+      float dot = 0.f;
+      float bv[E];
 #pragma unroll
-        for (int i = 0; i < NPL; ++i) {
-          const int c = (i * 32 + lane) * VEC;
-          Pack<VEC> pw{}, pb{};
-          if (c < d) {
-            pw = ld_pack<VEC>(wg + l * d + c, false);
-            pb = ld_pack<VEC>(bg + l * d + c, false);
-          }
-#pragma unroll
-          for (int e = 0; e < VEC; ++e) {
-            dot = fmaf(xl[i * VEC + e], (c < d) ? pw.v[e] : 0.f, dot);
-            bv[i * VEC + e] = (c < d) ? pb.v[e] : 0.f;
-          }
+      for (int i = 0; i < NPL; ++i) {
+        const int c = (i * 32 + lane) * VEC;
+        Pack<VEC> pw{}, pb{};
+        if (c < d) {
+          pw = ld_pack<VEC>(wg + l * d + c, false);
+          pb = ld_pack<VEC>(bg + l * d + c, false);
         }
-        dot = warp_sum(dot);
 #pragma unroll
-        for (int e = 0; e < E; ++e)
-          xl[e] = __fadd_rn(__fadd_rn(__fmul_rn(x0[e], dot), bv[e]), xl[e]);
-        if (lane == l) s_mine = dot;
+        for (int e = 0; e < VEC; ++e) {
+          dot = fmaf(xl[i * VEC + e], (c < d) ? pw.v[e] : 0.f, dot);
+          bv[i * VEC + e] = (c < d) ? pb.v[e] : 0.f;
+        }
       }
+      dot = warp_sum(dot);
+#pragma unroll
+      for (int e = 0; e < E; ++e)
+        xl[e] = __fadd_rn(__fadd_rn(__fmul_rn(x0[e], dot), bv[e]), xl[e]);
+      if (lane == l) s_mine = dot;
     }
     // c_l = 1 + sum_{j<l} s_j  (lane l keeps c_l)
     float c_mine = 1.f;
@@ -1081,7 +1077,7 @@ extern "C" int dir_cross_bwd(const float* x0, const float* cross_w, const float*
   const size_t smem1 = (size_t)kCrossWarps * (d + 32) * 4;
 #define DIR_BWD(V, N)                                                                        \
   cross_bwd_sample_kernel<V, N><<<w.G1, kCrossWarps * 32, smem1, st>>>(                      \
-      x0, cross_w, cross_b, dy, nullptr, B, d, L, dx0, w.alpha, w.Dpart, w.dypart)
+      x0, cross_w, cross_b, dy, B, d, L, dx0, w.alpha, w.Dpart, w.dypart)
   DIR_CROSS_DISPATCH(DIR_BWD)
 #undef DIR_BWD
   cross_bwd_dw_kernel<<<w.G2, 256, kDwUnroll * 8 * 4, st>>>(x0, w.alpha, B, d, L, w.dwpart);
