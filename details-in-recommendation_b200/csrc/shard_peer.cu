@@ -23,6 +23,14 @@
 //                                                       dir_shard_slots(clear)
 //   dir_shard_dense_apply   replicated one-row fields: ranks' sums added in rank order, same update everywhere
 //
+// With clip_norm (tf.clip_by_norm per column), the owner half after the grads barrier is instead
+//                                                       dir_shard_owner_sqnorms  per column: squares of the merged
+//                                                         sums -> norm[me] of every rank's norm buffer
+//   ---- barrier (norms) ----
+//                                                       dir_shard_owner_update_clipped  partials combined in rank
+//                                                         order, the same update with each sum scaled
+//   dir_shard_dense_apply_clipped   replicated one-row fields, each clipped by its own sum
+//
 // The owner never sorts: a requester sends each row at most once, so slot[row][q] (one cell per local row and
 // requester, written without atomics) tells an arrival whether an earlier rank asked for the same row; the first
 // one merges.  Deterministic: no floating-point atomics, sums in rank order.  A cell is (epoch << 24) | (i + 1) and
@@ -240,15 +248,44 @@ struct OwnerSrc {
   const uint32_t* epoch[2];
 };
 
-template <int LPR, int NBUF>
+// CLIP: tf.clip_by_norm per column of the merged sums (dir_shard_owner_update_clipped).  The column's denominators come
+// from the combined partials (clip.part, [F][kClipSlices][2]) into shared memory; a row's column is looked up from its
+// local row (clip.field_offset: the columns' first local rows, ascending).
+struct OwnerClip {
+  const int64_t* field_offset;
+  const double* part;
+  int F;
+  float clip;
+};
+// 16 KB, allocated only by the kernels that call it (an extern __shared__ array would add to every kernel's static
+// shared memory in this file)
+struct ClipSmem {
+  int64_t off[kClipMaxFields];
+  float den[kClipMaxFields], den1[kClipMaxFields];
+};
+__device__ __forceinline__ ClipSmem& clip_smem() {
+  __shared__ ClipSmem cs;
+  return cs;
+}
+
+template <int LPR, int NBUF, bool CLIP = false>
 __global__ void __launch_bounds__(256, LPR <= 4 ? 3 : 1)
 peer_owner_update_kernel(const dir_peer_layout L, const OwnerSrc src, float* table, float* accum,
                          int64_t row_stride, float* lin, float* lin_accum, int64_t lin_stride, const LinOpt lo,
-                         const RowRule rule, int64_t n_local, unsigned long long* n_unique) {
+                         const RowRule rule, int64_t n_local, unsigned long long* n_unique, const OwnerClip clip) {
   constexpr int SLOTS = 32 / LPR;
   constexpr int PB = LPR <= 4 ? 2 : 1;
   constexpr unsigned FULL = 0xffffffffu;
   __shared__ Arrivals s[NBUF];
+  const int64_t* c_off = nullptr;
+  const float *c_den = nullptr, *c_den1 = nullptr;
+  if constexpr (CLIP) {
+    ClipSmem& cs = clip_smem();
+    clip_denominators(clip.part, clip.field_offset, clip.F, clip.clip, cs.off, cs.den, cs.den1);
+    c_off = cs.off;
+    c_den = cs.den;
+    c_den1 = cs.den1;
+  }
   uint32_t tag[NBUF];
   int64_t tot[NBUF];
 #pragma unroll
@@ -359,6 +396,18 @@ peer_owner_update_kernel(const dir_peer_layout L, const OwnerSrc src, float* tab
           if (sub == 0 && lin != nullptr)
             g1[j] = __fadd_rn(g1[j], __ldg(reinterpret_cast<const float*>(src.local[bb] + L.off_g1) + e2));
         }
+        if constexpr (CLIP) {
+          int f = 0, hi = clip.F;  // last column whose first local row <= the row
+          while (hi - f > 1) {
+            const int mid = (f + hi) >> 1;
+            if (c_off[mid] <= rr[j]) f = mid; else hi = mid;
+          }
+          g[j].x = clip1(g[j].x, clip.clip, c_den[f]);
+          g[j].y = clip1(g[j].y, clip.clip, c_den[f]);
+          g[j].z = clip1(g[j].z, clip.clip, c_den[f]);
+          g[j].w = clip1(g[j].w, clip.clip, c_den[f]);
+          g1[j] = clip1(g1[j], clip.clip, c_den1[f]);
+        }
         const int64_t ro = rr[j] * row_stride;
         T[j].x = upd_rule(T[j].x, g[j].x, A[j].x, rule);
         T[j].y = upd_rule(T[j].y, g[j].y, A[j].y, rule);
@@ -374,6 +423,155 @@ peer_owner_update_kernel(const dir_peer_layout L, const OwnerSrc src, float* tab
     }
   }
   if (lane == 0 && leaders && n_unique) atomicAdd(n_unique, leaders);
+}
+
+// ---- tf.clip_by_norm per column on the owner (dir_shard_owner_sqnorms, dir_shard_owner_update_clipped)
+// A column's norm is over its MERGED per-row sums, and only the owner of a row sees that sum, so every owner reduces
+// its own rows per column and the ranks exchange [F][kClipSlices][2] partials:
+//   1. per arrival: the leading arrival builds the merged vector exactly as peer_owner_update_kernel does (same
+//      leader rule, same __fadd_rn order) and writes its (sum g^2, g1^2) in fp64 to sq[a]; others write zeros.
+//      The cost grows with the arrivals, not with the table (no sweep of the slot map).
+//   2. CTA (f, s): the column's arrivals of requester q are one contiguous range of q's id segment, found with two
+//      lower_bounds: a requester numbers its distinct keys (owner, local row) in sorted order (dir_shard_unique
+//      after dir_shard_keys_sort or dir_shard_bag_keys), so each segment is strictly ascending in local row, and a
+//      column is a contiguous range of local rows (local row l of rank r is global row l * G + r).  Fixed-order fp64
+//      sums, independent of the grid; the partials go to norm[rank] of EVERY rank's norm buffer.
+//   3. (after a barrier) peer_clip_combine_kernel: part[f][s] = sum over q of norm[q][f][s] in rank order, so every
+//      rank divides by bit-identical denominators.
+template <int LPR>
+__global__ void __launch_bounds__(256)
+peer_owner_sqnorm_kernel(const dir_peer_layout L, const uint32_t* __restrict__ slot,
+                         const uint32_t* __restrict__ epoch, int64_t n_local, bool with_g1, double2* __restrict__ sq) {
+  constexpr int SLOTS = 32 / LPR;
+  constexpr unsigned FULL = 0xffffffffu;
+  __shared__ Arrivals s;
+  load_arrivals(L, s);
+  const uint32_t tag = epoch[0];
+  const int64_t total = s.pre[L.G];
+  const int G = L.G;
+  const int lane = threadIdx.x & 31;
+  const int sub = lane % LPR, grp = lane / LPR;
+  const int32_t* ids = reinterpret_cast<const int32_t*>(L.local + L.off_ids);
+  const float4* gb = reinterpret_cast<const float4*>(L.local + L.off_g);
+  const float* g1b = reinterpret_cast<const float*>(L.local + L.off_g1);
+  const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t a0 = warp * 32; a0 < total; a0 += nwarps * 32) {  // warp-uniform trip count
+    const int64_t a = a0 + lane;
+    bool lead = false;
+    int64_t e = 0, r = 0;
+    unsigned long long more = 0;
+    if (a < total) {
+      const int q = seg_of(s.pre, G, a);
+      e = (int64_t)q * L.seg_cap + (a - s.pre[q]);
+      r = __ldg(ids + e);
+      if (r >= 0 && r < n_local) {
+        bool earlier = false;
+        for (int p = 0; p < G; ++p) {
+          const bool on = (__ldg(slot + r * G + p) >> 24) == tag;
+          earlier |= on && p < q;
+          if (on && p > q) more |= 1ull << p;
+        }
+        lead = !earlier;
+      }
+      if (!lead) sq[a] = make_double2(0.0, 0.0);
+    }
+    const unsigned lm = __ballot_sync(FULL, lead);
+    const int nl = __popc(lm);
+    for (int k0 = 0; k0 < nl; k0 += SLOTS) {
+      const int n = k0 + grp;
+      const bool on = n < nl;
+      const int from = on ? (int)__fns(lm, 0, n + 1) : 0;
+      const int64_t rr = __shfl_sync(FULL, r, from);
+      const int64_t ee = __shfl_sync(FULL, e, from);
+      unsigned long long m = __shfl_sync(FULL, more, from);
+      double v = 0.0, v1 = 0.0;
+      if (on) {
+        float4 g = __ldg(gb + ee * LPR + sub);
+        float g1 = with_g1 && sub == 0 ? __ldg(g1b + ee) : 0.f;
+        while (m) {  // the order of peer_owner_update_kernel: rank
+          const int p = __ffsll((long long)m) - 1;
+          m &= m - 1;
+          const uint32_t sp = __ldg(slot + rr * G + p) & 0xffffffu;
+          const int64_t e2 = (int64_t)p * L.seg_cap + (sp - 1u);
+          const float4 o = __ldg(gb + e2 * LPR + sub);
+          g.x = __fadd_rn(g.x, o.x);
+          g.y = __fadd_rn(g.y, o.y);
+          g.z = __fadd_rn(g.z, o.z);
+          g.w = __fadd_rn(g.w, o.w);
+          if (with_g1 && sub == 0) g1 = __fadd_rn(g1, __ldg(g1b + e2));
+        }
+        v = (double)g.x * g.x + (double)g.y * g.y + (double)g.z * g.z + (double)g.w * g.w;
+        v1 = (double)g1 * g1;
+      }
+#pragma unroll
+      for (int o = LPR / 2; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);  // the row's LPR lanes, fixed tree
+      if (on && sub == 0) sq[a0 + from] = make_double2(v, v1);
+    }
+  }
+}
+
+// first i < n with a[i] >= x (a ascending)
+__device__ __forceinline__ int64_t lower_bound_i32(const int32_t* __restrict__ a, int64_t n, int64_t x) {
+  int64_t lo = 0, hi = n;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if ((int64_t)__ldg(a + mid) < x) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+// grid (F, kClipSlices): slice sl of column f -> norm_peers[every q][rank][f][sl][2]
+__global__ void __launch_bounds__(256, 1)
+peer_owner_sqnorm_reduce_kernel(const dir_peer_layout L, const double2* __restrict__ sq,
+                                const int64_t* __restrict__ local_field_offset, int F,
+                                const unsigned long long* __restrict__ norm_peers) {
+  __shared__ Arrivals s;
+  __shared__ int64_t s_lo[kMaxG], s_hi[kMaxG];
+  __shared__ double red[2][256];
+  const int f = blockIdx.x, sl = blockIdx.y;
+  load_arrivals(L, s);
+  const int G = L.G;
+  if (threadIdx.x < G) {
+    const int q = threadIdx.x;
+    const int32_t* seg = reinterpret_cast<const int32_t*>(L.local + L.off_ids) + (int64_t)q * L.seg_cap;
+    const int64_t cnt = s.pre[q + 1] - s.pre[q];
+    s_lo[q] = lower_bound_i32(seg, cnt, local_field_offset[f]);
+    s_hi[q] = lower_bound_i32(seg, cnt, local_field_offset[f + 1]);
+  }
+  __syncthreads();
+  double v = 0.0, v1 = 0.0;
+  for (int q = 0; q < G; ++q)
+    for (int64_t i = s_lo[q] + (int64_t)sl * 256 + threadIdx.x; i < s_hi[q]; i += (int64_t)kClipSlices * 256) {
+      const double2 t = sq[s.pre[q] + i];
+      v += t.x;
+      v1 += t.y;
+    }
+  red[0][threadIdx.x] = v;
+  red[1][threadIdx.x] = v1;
+  __syncthreads();
+  for (int st = 128; st > 0; st >>= 1) {
+    if (threadIdx.x < st) {
+      red[0][threadIdx.x] += red[0][threadIdx.x + st];
+      red[1][threadIdx.x] += red[1][threadIdx.x + st];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x < G) {
+    double* dst = reinterpret_cast<double*>(__ldg(norm_peers + threadIdx.x)) +
+                  (((int64_t)L.rank * F + f) * kClipSlices + sl) * 2;
+    *reinterpret_cast<double2*>(dst) = make_double2(red[0][0], red[1][0]);
+  }
+}
+
+// part[x] = sum over q of norm[q][x] in rank order, x < F * kClipSlices * 2
+__global__ void __launch_bounds__(256)
+peer_clip_combine_kernel(const double* __restrict__ norm, int G, int64_t n, double* __restrict__ part) {
+  const int64_t x = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (x >= n) return;
+  double v = norm[x];
+  for (int q = 1; q < G; ++q) v += norm[(int64_t)q * n + x];
+  part[x] = v;
 }
 
 // replicated one-row fields: the G ranks' sums added in rank order, the same update applied to every replica;
@@ -397,22 +595,40 @@ struct DenseApplyArgs {
   unsigned long long* n_unique;
 };
 
-template <int LPR>
+// CLIP: a one-row field is a column with one row, so tf.clip_by_norm divides by max(||g||, clip) of the rank-ordered
+// sum itself (and the linear weight by max(|g1|, clip)), the arithmetic of dir_embed_bwd_onerow_update(..., clip_norm).
+// Every rank forms the same sum: no exchange.
+template <int LPR, bool CLIP = false>
 __global__ void __launch_bounds__(128)
-peer_dense_apply_kernel(const dir_peer_layout L, const char* local_b, const DenseApplyArgs a) {
+peer_dense_apply_kernel(const dir_peer_layout L, const char* local_b, const DenseApplyArgs a, float clip = 0.f) {
   constexpr int K = LPR * 4;
   const int j = blockIdx.x, c = threadIdx.x;
-  if (c > K) return;
+  if (!CLIP && c > K) return;
+  const int cc = c <= K ? c : K;  // (CLIP keeps every thread until the norm is known)
   float g = 0.f, touched = 0.f;
   for (int b = 0; b < (local_b ? 2 : 1); ++b) {  // buffer (micro-batch), then rank: the same sum on every rank
     const float* gbuf = reinterpret_cast<const float*>((b ? local_b : L.local) + L.off_dense);
     for (int q = 0; q < L.G; ++q) {
       const float* src = gbuf + ((int64_t)q * L.n_dense + j) * (K + 4);
-      g = (b == 0 && q == 0) ? src[c] : __fadd_rn(g, src[c]);
+      g = (b == 0 && q == 0) ? src[cc] : __fadd_rn(g, src[cc]);
       touched += src[K + 1];
     }
   }
-  if (touched == 0.f) return;  // no rank had a surviving lookup: the row is not touched
+  if (touched == 0.f) return;  // no rank had a surviving lookup: the row is not touched (the same for every thread)
+  if constexpr (CLIP) {
+    __shared__ float s_g[K + 1], s_den[2];
+    if (c <= K) s_g[c] = g;
+    __syncthreads();
+    if (c == 0) {
+      double sq = 0.0;
+      for (int k = 0; k < K; ++k) sq += (double)s_g[k] * s_g[k];
+      s_den[0] = fmaxf((float)sqrt(sq), clip);
+      s_den[1] = fmaxf(fabsf(s_g[K]), clip);
+    }
+    __syncthreads();
+    if (c > K) return;
+    g = clip1(g, clip, s_den[c < K ? 0 : 1]);
+  }
   const int64_t sr = __ldg(a.shard_row + j);
   const bool adagrad = a.rr.opt != DIR_OPT_SGD;
   if (c < K) {
@@ -587,43 +803,48 @@ extern "C" int dir_shard_g1_push(const dir_peer_layout* layout, const float* g1_
   return launched("shard_g1_push");
 }
 
-extern "C" int dir_shard_owner_update(const dir_peer_layout* layout, const uint32_t* slot, float* table, float* accum,
-                                      int64_t row_stride, float* lin, float* lin_accum, int64_t lin_stride,
-                                      int64_t n_local_rows, const uint32_t* slot_epoch, int optimizer, float lr,
-                                      const dir_table_opt* table_opt, const dir_linear_opt* linear_opt,
-                                      const dir_peer_layout* layout_b,
-                                      const uint32_t* slot_b, const uint32_t* slot_epoch_b, int64_t* n_unique_out,
-                                      dir_stream_t stream) {
-  using namespace dir;
-  if (int rc = check_layout("shard_owner_update", layout)) return rc;
+namespace dir {
+
+// dir_shard_owner_update[_clipped]: clip == nullptr -> the unclipped kernels
+static int owner_update(const char* what, const dir_peer_layout* layout, const uint32_t* slot, float* table,
+                        float* accum, int64_t row_stride, float* lin, float* lin_accum, int64_t lin_stride,
+                        int64_t n_local_rows, const uint32_t* slot_epoch, int optimizer, float lr,
+                        const dir_table_opt* table_opt, const dir_linear_opt* linear_opt,
+                        const dir_peer_layout* layout_b, const uint32_t* slot_b, const uint32_t* slot_epoch_b,
+                        int64_t* n_unique_out, const OwnerClip* clip, cudaStream_t st) {
+  if (int rc = check_layout(what, layout)) return rc;
   if (layout_b != nullptr) {
-    if (int rc = check_layout("shard_owner_update", layout_b)) return rc;
+    if (int rc = check_layout(what, layout_b)) return rc;
     if (!slot_b || !slot_epoch_b || layout_b->G != layout->G || layout_b->seg_cap != layout->seg_cap ||
         layout_b->off_g != layout->off_g || layout->G > 32)
-      return fail(DIR_EINVAL, "shard_owner_update: the second buffer needs its slot map and epoch, the same layout, G <= 32");
+      return fail(DIR_EINVAL, "%s: the second buffer needs its slot map and epoch, the same layout, G <= 32", what);
   }
   const int K = layout->K;
   if (optimizer != DIR_OPT_SGD && optimizer != DIR_OPT_ADAGRAD && optimizer != DIR_OPT_PROXIMAL_ADAGRAD)
-    return fail(DIR_EINVAL, "shard_owner_update: unknown optimizer");
+    return fail(DIR_EINVAL, "%s: unknown optimizer", what);
   const RowRule rr{optimizer, lr, table_opt ? table_opt->l1 : 0.f, table_opt ? table_opt->l2 : 0.f};
-  if (rr.l1 < 0.f || rr.l2 < 0.f) return fail(DIR_EINVAL, "shard_owner_update: l1, l2 must be >= 0");
+  if (rr.l1 < 0.f || rr.l2 < 0.f) return fail(DIR_EINVAL, "%s: l1, l2 must be >= 0", what);
   if (!slot || !slot_epoch || !table || n_local_rows <= 0)
-    return fail(DIR_EINVAL, "shard_owner_update: slot, slot_epoch, table, n_local_rows > 0 required");
-  if (optimizer != DIR_OPT_SGD && !accum) return fail(DIR_EINVAL, "shard_owner_update: Adagrad needs accum");
+    return fail(DIR_EINVAL, "%s: slot, slot_epoch, table, n_local_rows > 0 required", what);
+  if (optimizer != DIR_OPT_SGD && !accum) return fail(DIR_EINVAL, "%s: Adagrad needs accum", what);
   if (row_stride < K || (row_stride & 3) || !aligned16(table) || !aligned16(accum))
-    return fail(DIR_EINVAL, "shard_owner_update: rows must be 16-byte aligned, row_stride >= K and a multiple of 4");
+    return fail(DIR_EINVAL, "%s: rows must be 16-byte aligned, row_stride >= K and a multiple of 4", what);
   LinOpt lo;
-  if (int rc = resolve_lin("shard_owner_update", linear_opt, optimizer, lr, lin, lin_accum, lo)) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (int rc = resolve_lin(what, linear_opt, optimizer, lr, lin, lin_accum, lo)) return rc;
   unsigned long long* nu = reinterpret_cast<unsigned long long*>(n_unique_out);  // += (zeroed by dir_shard_slots)
   OwnerSrc src{{layout->local, layout_b ? layout_b->local : nullptr}, {slot, slot_b}, {slot_epoch, slot_epoch_b}};
+  const OwnerClip oc = clip ? *clip : OwnerClip{nullptr, nullptr, 0, 0.f};
 #define DIR_OU(LP)                                                                                                  \
-  if (layout_b)                                                                                                     \
+  if (clip)                                                                                                         \
+    peer_owner_update_kernel<LP, 1, true><<<kPeerCtas, 256, 0, st>>>(*layout, src, table, accum, row_stride, lin, \
+                                                                        lin_accum, lin_stride, lo, rr, n_local_rows, \
+                                                                        nu, oc);                                    \
+  else if (layout_b)                                                                                                \
     peer_owner_update_kernel<LP, 2><<<kPeerCtas, 256, 0, st>>>(*layout, src, table, accum, row_stride, lin, lin_accum, \
-                                                               lin_stride, lo, rr, n_local_rows, nu);                \
+                                                               lin_stride, lo, rr, n_local_rows, nu, oc);            \
   else                                                                                                              \
     peer_owner_update_kernel<LP, 1><<<kPeerCtas, 256, 0, st>>>(*layout, src, table, accum, row_stride, lin, lin_accum, \
-                                                               lin_stride, lo, rr, n_local_rows, nu)
+                                                               lin_stride, lo, rr, n_local_rows, nu, oc)
   switch (K / 4) {
     case 1: DIR_OU(1); break;
     case 2: DIR_OU(2); break;
@@ -632,7 +853,66 @@ extern "C" int dir_shard_owner_update(const dir_peer_layout* layout, const uint3
     default: DIR_OU(16); break;
   }
 #undef DIR_OU
-  return launched("shard_owner_update");
+  return launched(what);
+}
+
+// dir_shard_dense_apply[_clipped]: clip_norm == 0 -> unclipped
+static int dense_apply(const char* what, const dir_peer_layout* layout, float* dense_table, float* dense_accum,
+                       int64_t row_stride, float* dense_lin, float* dense_lin_accum, int optimizer, float lr,
+                       const dir_table_opt* table_opt, const dir_linear_opt* linear_opt, float* shard_table,
+                       float* shard_accum, int64_t shard_row_stride, float* shard_lin, float* shard_lin_accum,
+                       float* shard_lin_z, int64_t shard_lin_stride, const int64_t* shard_row,
+                       const dir_peer_layout* layout_b, int64_t* n_unique_inout, float clip_norm, cudaStream_t st) {
+  if (int rc = check_layout(what, layout)) return rc;
+  if (layout_b != nullptr) {
+    if (int rc = check_layout(what, layout_b)) return rc;
+    if (layout_b->off_dense != layout->off_dense || layout_b->G != layout->G)
+      return fail(DIR_EINVAL, "%s: the second buffer must have the same layout", what);
+  }
+  const char* local_b = layout_b ? layout_b->local : nullptr;
+  if (layout->n_dense == 0) return 0;
+  if (optimizer != DIR_OPT_SGD && optimizer != DIR_OPT_ADAGRAD && optimizer != DIR_OPT_PROXIMAL_ADAGRAD)
+    return fail(DIR_EINVAL, "%s: unknown optimizer", what);
+  const RowRule rr{optimizer, lr, table_opt ? table_opt->l1 : 0.f, table_opt ? table_opt->l2 : 0.f};
+  if (!dense_table || !shard_row || !shard_table) return fail(DIR_EINVAL, "%s: null pointer", what);
+  if (optimizer != DIR_OPT_SGD && (!dense_accum || !shard_accum))
+    return fail(DIR_EINVAL, "%s: Adagrad needs the accumulators", what);
+  LinOpt lo;
+  if (int rc = resolve_lin(what, linear_opt, optimizer, lr, dense_lin, dense_lin_accum, lo)) return rc;
+  if (dense_lin && (!shard_lin || (lo.opt != DIR_OPT_SGD && !shard_lin_accum) || (lo.opt == DIR_OPT_FTRL && !shard_lin_z)))
+    return fail(DIR_EINVAL, "%s: the sharded copies of the linear state are required", what);
+  DenseApplyArgs a{dense_table, dense_accum, row_stride, dense_lin, dense_lin_accum, lo, rr,
+                   shard_table, shard_accum, shard_row_stride, shard_lin, shard_lin_accum, shard_lin_z,
+                   shard_lin_stride, shard_row, reinterpret_cast<unsigned long long*>(n_unique_inout)};
+  const int n = layout->n_dense;
+#define DIR_DA(LP)                                                                                       \
+  if (clip_norm > 0.f)                                                                                   \
+    peer_dense_apply_kernel<LP, true><<<n, 128, 0, st>>>(*layout, local_b, a, clip_norm);               \
+  else                                                                                                   \
+    peer_dense_apply_kernel<LP><<<n, 128, 0, st>>>(*layout, local_b, a)
+  switch (layout->K / 4) {
+    case 1: DIR_DA(1); break;
+    case 2: DIR_DA(2); break;
+    case 4: DIR_DA(4); break;
+    case 8: DIR_DA(8); break;
+    default: DIR_DA(16); break;
+  }
+#undef DIR_DA
+  return launched(what);
+}
+
+}  // namespace dir
+
+extern "C" int dir_shard_owner_update(const dir_peer_layout* layout, const uint32_t* slot, float* table, float* accum,
+                                      int64_t row_stride, float* lin, float* lin_accum, int64_t lin_stride,
+                                      int64_t n_local_rows, const uint32_t* slot_epoch, int optimizer, float lr,
+                                      const dir_table_opt* table_opt, const dir_linear_opt* linear_opt,
+                                      const dir_peer_layout* layout_b,
+                                      const uint32_t* slot_b, const uint32_t* slot_epoch_b, int64_t* n_unique_out,
+                                      dir_stream_t stream) {
+  return dir::owner_update("shard_owner_update", layout, slot, table, accum, row_stride, lin, lin_accum, lin_stride,
+                           n_local_rows, slot_epoch, optimizer, lr, table_opt, linear_opt, layout_b, slot_b,
+                           slot_epoch_b, n_unique_out, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int dir_shard_dense_apply(const dir_peer_layout* layout, float* dense_table, float* dense_accum,
@@ -643,36 +923,75 @@ extern "C" int dir_shard_dense_apply(const dir_peer_layout* layout, float* dense
                                      float* shard_lin_accum, float* shard_lin_z, int64_t shard_lin_stride,
                                      const int64_t* shard_row, const dir_peer_layout* layout_b,
                                      int64_t* n_unique_inout, dir_stream_t stream) {
+  return dir::dense_apply("shard_dense_apply", layout, dense_table, dense_accum, row_stride, dense_lin,
+                          dense_lin_accum, optimizer, lr, table_opt, linear_opt, shard_table, shard_accum,
+                          shard_row_stride, shard_lin, shard_lin_accum, shard_lin_z, shard_lin_stride, shard_row,
+                          layout_b, n_unique_inout, 0.f, static_cast<cudaStream_t>(stream));
+}
+
+// ---- tf.clip_by_norm per column (see the kernels above)
+extern "C" int dir_shard_owner_sqnorms(const dir_peer_layout* layout, const uint32_t* slot, const uint32_t* slot_epoch,
+                                       int64_t n_local_rows, const int64_t* local_field_offset, int F, int with_g1,
+                                       double* sq_scratch, const uint64_t* norm_peers, dir_stream_t stream) {
   using namespace dir;
-  if (int rc = check_layout("shard_dense_apply", layout)) return rc;
-  if (layout_b != nullptr) {
-    if (int rc = check_layout("shard_dense_apply", layout_b)) return rc;
-    if (layout_b->off_dense != layout->off_dense || layout_b->G != layout->G)
-      return fail(DIR_EINVAL, "shard_dense_apply: the second buffer must have the same layout");
-  }
-  const char* local_b = layout_b ? layout_b->local : nullptr;
-  if (layout->n_dense == 0) return 0;
-  if (optimizer != DIR_OPT_SGD && optimizer != DIR_OPT_ADAGRAD && optimizer != DIR_OPT_PROXIMAL_ADAGRAD)
-    return fail(DIR_EINVAL, "shard_dense_apply: unknown optimizer");
-  const RowRule rr{optimizer, lr, table_opt ? table_opt->l1 : 0.f, table_opt ? table_opt->l2 : 0.f};
-  if (!dense_table || !shard_row || !shard_table) return fail(DIR_EINVAL, "shard_dense_apply: null pointer");
-  if (optimizer != DIR_OPT_SGD && (!dense_accum || !shard_accum))
-    return fail(DIR_EINVAL, "shard_dense_apply: Adagrad needs the accumulators");
-  LinOpt lo;
-  if (int rc = resolve_lin("shard_dense_apply", linear_opt, optimizer, lr, dense_lin, dense_lin_accum, lo)) return rc;
-  if (dense_lin && (!shard_lin || (lo.opt != DIR_OPT_SGD && !shard_lin_accum) || (lo.opt == DIR_OPT_FTRL && !shard_lin_z)))
-    return fail(DIR_EINVAL, "shard_dense_apply: the sharded copies of the linear state are required");
-  DenseApplyArgs a{dense_table, dense_accum, row_stride, dense_lin, dense_lin_accum, lo, rr,
-                   shard_table, shard_accum, shard_row_stride, shard_lin, shard_lin_accum, shard_lin_z,
-                   shard_lin_stride, shard_row, reinterpret_cast<unsigned long long*>(n_unique_inout)};
+  if (int rc = check_layout("shard_owner_sqnorms", layout)) return rc;
+  if (F <= 0 || F > kClipMaxFields) return fail(DIR_EINVAL, "shard_owner_sqnorms: 0 < F <= 1024 required");
+  if (!slot || !slot_epoch || !local_field_offset || !sq_scratch || !norm_peers || n_local_rows <= 0)
+    return fail(DIR_EINVAL, "shard_owner_sqnorms: slot, slot_epoch, local_field_offset, sq_scratch, norm_peers, "
+                            "n_local_rows > 0 required");
+  if ((reinterpret_cast<uintptr_t>(sq_scratch) & 15u) != 0)
+    return fail(DIR_EINVAL, "shard_owner_sqnorms: sq_scratch must be 16-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int n = layout->n_dense;
+  double2* sq = reinterpret_cast<double2*>(sq_scratch);
   switch (layout->K / 4) {
-    case 1: peer_dense_apply_kernel<1><<<n, 128, 0, st>>>(*layout, local_b, a); break;
-    case 2: peer_dense_apply_kernel<2><<<n, 128, 0, st>>>(*layout, local_b, a); break;
-    case 4: peer_dense_apply_kernel<4><<<n, 128, 0, st>>>(*layout, local_b, a); break;
-    case 8: peer_dense_apply_kernel<8><<<n, 128, 0, st>>>(*layout, local_b, a); break;
-    default: peer_dense_apply_kernel<16><<<n, 128, 0, st>>>(*layout, local_b, a); break;
+    case 1: peer_owner_sqnorm_kernel<1><<<kPeerCtas, 256, 0, st>>>(*layout, slot, slot_epoch, n_local_rows, with_g1 != 0, sq); break;
+    case 2: peer_owner_sqnorm_kernel<2><<<kPeerCtas, 256, 0, st>>>(*layout, slot, slot_epoch, n_local_rows, with_g1 != 0, sq); break;
+    case 4: peer_owner_sqnorm_kernel<4><<<kPeerCtas, 256, 0, st>>>(*layout, slot, slot_epoch, n_local_rows, with_g1 != 0, sq); break;
+    case 8: peer_owner_sqnorm_kernel<8><<<kPeerCtas, 256, 0, st>>>(*layout, slot, slot_epoch, n_local_rows, with_g1 != 0, sq); break;
+    default: peer_owner_sqnorm_kernel<16><<<kPeerCtas, 256, 0, st>>>(*layout, slot, slot_epoch, n_local_rows, with_g1 != 0, sq); break;
   }
-  return launched("shard_dense_apply");
+  peer_owner_sqnorm_reduce_kernel<<<dim3((unsigned)F, kClipSlices), 256, 0, st>>>(
+      *layout, sq, local_field_offset, F, reinterpret_cast<const unsigned long long*>(norm_peers));
+  return launched("shard_owner_sqnorms", 2);
+}
+
+extern "C" int dir_shard_owner_update_clipped(const dir_peer_layout* layout, const uint32_t* slot, float* table,
+                                              float* accum, int64_t row_stride, float* lin, float* lin_accum,
+                                              int64_t lin_stride, int64_t n_local_rows, const uint32_t* slot_epoch,
+                                              int optimizer, float lr, const dir_linear_opt* linear_opt,
+                                              const int64_t* local_field_offset, int F, const double* norm,
+                                              double* partials, float clip_norm, int64_t* n_unique_inout,
+                                              dir_stream_t stream) {
+  using namespace dir;
+  if (int rc = check_layout("shard_owner_update_clipped", layout)) return rc;
+  if (F <= 0 || F > kClipMaxFields) return fail(DIR_EINVAL, "shard_owner_update_clipped: 0 < F <= 1024 required");
+  if (optimizer != DIR_OPT_SGD && optimizer != DIR_OPT_ADAGRAD)
+    return fail(DIR_EINVAL, "shard_owner_update_clipped: optimizer must be SGD or Adagrad");
+  if (!(clip_norm > 0.f)) return fail(DIR_EINVAL, "shard_owner_update_clipped: clip_norm must be > 0");
+  if (!local_field_offset || !norm || !partials) return fail(DIR_EINVAL, "shard_owner_update_clipped: null pointer");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int64_t n = (int64_t)F * kClipSlices * 2;
+  peer_clip_combine_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(norm, layout->G, n, partials);
+  if (int rc = launched("shard_owner_update_clipped")) return rc;
+  const OwnerClip oc{local_field_offset, partials, F, clip_norm};
+  return owner_update("shard_owner_update_clipped", layout, slot, table, accum, row_stride, lin, lin_accum, lin_stride,
+                      n_local_rows, slot_epoch, optimizer, lr, nullptr, linear_opt, nullptr, nullptr, nullptr,
+                      n_unique_inout, &oc, st);
+}
+
+extern "C" int dir_shard_dense_apply_clipped(const dir_peer_layout* layout, float* dense_table, float* dense_accum,
+                                             int64_t row_stride, float* dense_lin, float* dense_lin_accum,
+                                             int optimizer, float lr, const dir_linear_opt* linear_opt,
+                                             float* shard_table, float* shard_accum, int64_t shard_row_stride,
+                                             float* shard_lin, float* shard_lin_accum, float* shard_lin_z,
+                                             int64_t shard_lin_stride, const int64_t* shard_row, float clip_norm,
+                                             int64_t* n_unique_inout, dir_stream_t stream) {
+  using namespace dir;
+  if (optimizer != DIR_OPT_SGD && optimizer != DIR_OPT_ADAGRAD)
+    return fail(DIR_EINVAL, "shard_dense_apply_clipped: optimizer must be SGD or Adagrad");
+  if (!(clip_norm > 0.f)) return fail(DIR_EINVAL, "shard_dense_apply_clipped: clip_norm must be > 0");
+  return dense_apply("shard_dense_apply_clipped", layout, dense_table, dense_accum, row_stride, dense_lin,
+                     dense_lin_accum, optimizer, lr, nullptr, linear_opt, shard_table, shard_accum, shard_row_stride,
+                     shard_lin, shard_lin_accum, shard_lin_z, shard_lin_stride, shard_row, nullptr, n_unique_inout,
+                     clip_norm, static_cast<cudaStream_t>(stream));
 }

@@ -191,7 +191,9 @@ class DCN(torch.nn.Module):
     to K: BASELINE.json's d = 624 convention).
     The per-tensor clip_by_norm(100) is applied to every gradient, as the reference does: the dense ones here, each
     column's table gradient inside the layer (`EmbeddingFM(clip_norm=...)`, a two-pass backward).  The sharded
-    layer applies its table gradients unclipped (a column's norm would need a cross-rank reduction per step).
+    layer clips its table gradients only with clip_sharded_tables=True (`ShardedEmbeddingFM(clip_norm=...)`: each
+    column's norm over the merged sums of the global batch, reduced across ranks on the device); by default it
+    applies them unclipped, as it always has.
     optimizer='adam' is the reference's own (train.py:104-124, epsilon = adam_epsilon = 1e-4): TF's Adam on the
     tables (`EmbeddingFM(optimizer='adam')`, every row's moments decay at every step) and `TFAdam` on the dense
     parameters.  Single-GPU layer only.
@@ -201,12 +203,12 @@ class DCN(torch.nn.Module):
                  cross_layer_num: int = 2, hidden_units: Sequence[int] = (256, 128), dnn_activation_fn=torch.relu,
                  dnn_dropout: Optional[float] = None, batch_norm: bool = False, optimizer: str = "adagrad",
                  learning_rate: float = _ADAGRAD_LR, clip_norm: Optional[float] = 100.0, sharded: bool = False,
-                 device="cuda", adam_epsilon: float = 1e-4, **layer_kw):
+                 device="cuda", adam_epsilon: float = 1e-4, clip_sharded_tables: bool = False, **layer_kw):
         super().__init__()
         d = field_size * embedding_size
         self.learning_rate, self.clip_norm = float(learning_rate), clip_norm
         self.optimizer, self.adam_epsilon = optimizer.lower(), float(adam_epsilon)
-        if clip_norm and not sharded:
+        if clip_norm and (clip_sharded_tables or not sharded):
             layer_kw = dict(layer_kw, clip_norm=clip_norm)      # every column's gradient is clipped too (:284)
         if self.optimizer == "adam":
             if sharded:

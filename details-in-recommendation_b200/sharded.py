@@ -27,9 +27,8 @@ import torch.distributed as dist
 
 from . import _lib
 from ._lib import check, ptr
-from .layers import (_K_OK, _TABLE_OPTIMIZERS, _Workspace, _need_cuda, _stream, linear_opt_struct,
-                     table_opt_struct,
-                     resolve_linear_optimizer)
+from .layers import (_CLIP_MAX_FIELDS, _K_OK, _TABLE_OPTIMIZERS, _Workspace, _need_cuda, _stream,
+                     linear_opt_struct, table_opt_struct, resolve_linear_optimizer)
 
 
 class ShardPlan:
@@ -62,6 +61,13 @@ class ShardPlan:
     def shard_of(self, full):
         """This rank's rows of a full [n_rows, ...] array (numpy or torch)."""
         return full[self.rank::self.world_size]
+
+    def local_field_offset(self, rank=None):
+        """[F + 1]: the first local row of each field on `rank`, then its local row count.  Local row l is global row
+        l * G + rank, so a field's rows on one rank are contiguous; a field with fewer rows than G may have none."""
+        r = self.rank if rank is None else rank
+        G = self.world_size
+        return [max(0, (x - r + G - 1) // G) for x in self.field_offset + [self.n_rows]]
 
 
 class StageTrace:
@@ -102,7 +108,7 @@ class PeerExchange:
     and the barrier is a no-op: the same kernels run.  `barrier(p, channel)` is a device-side cross-rank barrier on
     the current stream; a lost barrier traps after BARRIER_TIMEOUT_MS instead of spinning forever."""
 
-    def __init__(self, group, world, rank, K, n_dense, seg_cap, u_cap, device, n_buf=2):
+    def __init__(self, group, world, rank, K, n_dense, seg_cap, u_cap, device, n_buf=2, norm_bytes=0):
         L = _lib.lib()
         self.world, self.rank, self.K, self.n_dense = world, rank, K, n_dense
         self.seg_cap, self.u_cap = int(seg_cap), int(u_cap)
@@ -111,25 +117,37 @@ class PeerExchange:
             lay = _lib.PeerLayout()
             check(L.dir_peer_layout_init(world, rank, K, n_dense, self.seg_cap, self.u_cap, _lib.ctypes.byref(lay)),
                   "dir_peer_layout_init")
-            nbytes = int(lay.total_bytes)
-            if world > 1:
-                import torch.distributed._symmetric_memory as symm_mem
-                buf = symm_mem.empty(nbytes, dtype=torch.uint8, device=device)
-                h = symm_mem.rendezvous(buf, group if group is not None else dist.group.WORLD)
-                base = torch.tensor(list(h.buffer_ptrs), dtype=torch.int64, device=device)
-            else:
-                buf = torch.empty(nbytes, dtype=torch.uint8, device=device)
-                h = None
-                base = torch.tensor([buf.data_ptr()], dtype=torch.int64, device=device)
-            buf.zero_()
+            buf, h, base = self._symmetric(group, world, int(lay.total_bytes), torch.uint8, device)
             lay.peer_base, lay.local = base.data_ptr(), buf.data_ptr()
             self.layouts.append(lay)
             self.bufs.append(buf)
             self.handles.append(h)
             self.peer_base.append(base)
+        # clip_norm: one small norm buffer per exchange buffer ([G][F][kClipSlices][2] doubles), each with a barrier of
+        # its own (its own symmetric allocation)
+        self.norm_bufs, self.norm_handles, self.norm_peers = [], [], []
+        for _ in range(n_buf if norm_bytes else 0):
+            buf, h, base = self._symmetric(group, world, norm_bytes // 8, torch.float64, device)
+            self.norm_bufs.append(buf)
+            self.norm_handles.append(h)
+            self.norm_peers.append(base)
         if world > 1:
             torch.cuda.synchronize(device)
             dist.barrier(group)                      # nobody stores into a buffer its owner is still zeroing
+
+    @staticmethod
+    def _symmetric(group, world, n, dtype, device):
+        """(zeroed buffer, symmetric-memory handle or None, device array of the G ranks' addresses)"""
+        if world > 1:
+            import torch.distributed._symmetric_memory as symm_mem
+            buf = symm_mem.empty(n, dtype=dtype, device=device)
+            h = symm_mem.rendezvous(buf, group if group is not None else dist.group.WORLD)
+            base = torch.tensor(list(h.buffer_ptrs), dtype=torch.int64, device=device)
+        else:
+            buf, h = torch.empty(n, dtype=dtype, device=device), None
+            base = torch.tensor([buf.data_ptr()], dtype=torch.int64, device=device)
+        buf.zero_()
+        return buf, h, base
 
     def ref(self, p):
         return _lib.ctypes.byref(self.layouts[p])
@@ -147,6 +165,11 @@ class PeerExchange:
     def barrier(self, p, channel=0):
         if self.handles[p] is not None:
             self.handles[p].barrier(channel=channel, timeout_ms=BARRIER_TIMEOUT_MS)
+
+    def norm_barrier(self, p):
+        """Every rank has stored its column partials into norm buffer p."""
+        if self.norm_handles[p] is not None:
+            self.norm_handles[p].barrier(channel=0, timeout_ms=BARRIER_TIMEOUT_MS)
 
 
 class ShardedLookups:
@@ -296,6 +319,11 @@ class ShardedEmbeddingFM(torch.nn.Module):
     replicated parameter: all-reduce its gradient like any dense parameter.
 
     `max_batch` sizes the exchange buffers.  `presort` may run at most one batch ahead of `forward`.
+
+    clip_norm: tf.clip_by_norm of every column's gradient before the update, as `EmbeddingFM(clip_norm=...)` applies it
+    (DeepCrossNetwork.py:282-289): one factor per column, over the column's per-row sums of the GLOBAL batch (every
+    rank's requests of a row merged).  Each owner reduces its rows per column and the ranks exchange the partials
+    (a few KB) over peer memory, so the step still replays from one CUDA graph.  SGD / Adagrad, one micro-batch.
     """
 
     def __init__(self, field_size: int, embedding_size: int, rows_per_field: Sequence[int],
@@ -305,11 +333,23 @@ class ShardedEmbeddingFM(torch.nn.Module):
                  linear_lr: Optional[float] = None, l1_regularization_strength: float = 0.0,
                  l2_regularization_strength: float = 0.0, init: str = "trunc_normal", micro_batches: int = 1,
                  replicate_onerow: bool = True, max_entries: Optional[int] = None, optimizer_l1: float = 0.0,
-                 optimizer_l2: float = 0.0, device="cuda"):
+                 optimizer_l2: float = 0.0, clip_norm: Optional[float] = None, device="cuda"):
         super().__init__()
         if micro_batches not in (1, 2):
             raise ValueError("micro_batches must be 1 or 2")
         self.micro_batches = int(micro_batches)
+        if clip_norm is not None and not clip_norm > 0:
+            raise ValueError("clip_norm must be > 0 (or None)")
+        self.clip_norm = None if clip_norm is None else float(clip_norm)
+        if self.clip_norm is not None:
+            if field_size > _CLIP_MAX_FIELDS:
+                raise ValueError("clip_norm supports at most %d fields (one clip factor per column), got field_size=%d"
+                                 % (_CLIP_MAX_FIELDS, field_size))
+            if str(optimizer).lower() == "proximal_adagrad":
+                raise ValueError("clip_norm is not available with proximal_adagrad")
+            if self.micro_batches != 1:
+                # the owner merges two buffers in one update: the norm pass would have to merge them as well
+                raise ValueError("clip_norm needs micro_batches=1")
         if field_size <= 0:
             raise ValueError("empty columns.")                      # deepFM.py:104-105
         if embedding_size not in _K_OK:
@@ -386,7 +426,17 @@ class ShardedEmbeddingFM(torch.nn.Module):
         if self.micro_batches == 2 and world > 32:
             raise ValueError("two micro-batches need world_size <= 32")
         n_buf = 2 * self.micro_batches          # two parities (consecutive steps alternate) x micro-batches
-        self.px = PeerExchange(process_group, world, rank, K, self.n_dense, seg_cap, u_cap, dev, n_buf)
+        L = _lib.lib()
+        clip = self.clip_norm is not None
+        self.px = PeerExchange(process_group, world, rank, K, self.n_dense, seg_cap, u_cap, dev, n_buf,
+                               norm_bytes=world * L.dir_field_sqnorms_bytes(field_size) if clip else 0)
+        # clip_norm: the columns' first local rows, the per-arrival squares (one scratch: steps run in stream order)
+        # and the combined partials of the last step ([F][kClipSlices][2], the same on every rank)
+        self.register_buffer("local_field_offset", torch.tensor(self.plan.local_field_offset(), dtype=torch.int64,
+                                                                device=dev) if clip else None)
+        self._clip_sq = torch.empty(2 * world * seg_cap, dtype=torch.float64, device=dev) if clip else None
+        self.register_buffer("clip_partials", torch.zeros(L.dir_field_sqnorms_bytes(field_size) // 8,
+                                                          dtype=torch.float64, device=dev) if clip else None)
         # who asked for which of my rows: one cell per (local row, requester), tagged with the buffer's epoch
         self.slot = [torch.zeros(cap * world, dtype=torch.int32, device=dev) for _ in range(n_buf)]
         self.slot_epoch = [torch.zeros(2, dtype=torch.int32, device=dev) for _ in range(n_buf)]
@@ -575,6 +625,9 @@ class ShardedEmbeddingFM(torch.nn.Module):
         adagrad = self.optimizer != "sgd"
         px.barrier(handles[-1].buf, 0)
         tr.mark("bwd.barrier")
+        if self.clip_norm is not None:
+            self._owner_step_clipped(h0)
+            return
         check(L.dir_shard_owner_update(
             px.ref(p), ptr(self.slot[p]), ptr(self.table), ptr(self.accum) if adagrad else None,
             self.row_stride, ptr(self.w1) if self.first_order else None,
@@ -599,6 +652,43 @@ class ShardedEmbeddingFM(torch.nn.Module):
                 self._n_unique2.data_ptr() + 8 * h0.parity if self.plan.rank == 0 else None, st),
                 "dir_shard_dense_apply")
             tr.mark("bwd.dense_apply")
+
+    def _owner_step_clipped(self, h):
+        """tf.clip_by_norm per column (one exchange buffer): the owner's per-column partials of the merged sums to every
+        rank, a barrier, then the update scaled by the rank-order combined factors; the one-row replicas clip their
+        own sums.  A step's norm buffer is written again only two steps later, by a norm pass that follows that step's
+        grads barrier, which every rank reaches only after it has combined this step's partials (same stream)."""
+        L = _lib.lib()
+        st = _stream()
+        px, p, F = self.px, h.buf, self.field_size
+        adagrad = self.optimizer != "sgd"
+        check(L.dir_shard_owner_sqnorms(px.ref(p), ptr(self.slot[p]), ptr(self.slot_epoch[p]), self.n_rows,
+                                        ptr(self.local_field_offset), F, int(self.first_order), ptr(self._clip_sq),
+                                        ptr(px.norm_peers[p]), st), "dir_shard_owner_sqnorms")
+        self.trace.mark("bwd.sqnorms")
+        px.norm_barrier(p)
+        self.trace.mark("bwd.norm_barrier")
+        check(L.dir_shard_owner_update_clipped(
+            px.ref(p), ptr(self.slot[p]), ptr(self.table), ptr(self.accum) if adagrad else None, self.row_stride,
+            ptr(self.w1) if self.first_order else None, ptr(self.w1_accum) if self.first_order else None,
+            self.lin_stride, self.n_rows, ptr(self.slot_epoch[p]), _TABLE_OPTIMIZERS[self.optimizer], self.lr,
+            linear_opt_struct(self), ptr(self.local_field_offset), F, ptr(px.norm_bufs[p]), ptr(self.clip_partials),
+            self.clip_norm, self._n_unique2.data_ptr() + 8 * h.parity, st), "dir_shard_owner_update_clipped")
+        self._last_parity = h.parity
+        self.trace.mark("bwd.owner_update")
+        if self.n_dense:
+            check(L.dir_shard_dense_apply_clipped(
+                px.ref(p), ptr(self.dense_table), ptr(self.dense_accum) if adagrad else None,
+                self.row_stride, ptr(self.dense_lin) if self.first_order else None,
+                ptr(self.dense_lin_acc) if self.first_order else None, _TABLE_OPTIMIZERS[self.optimizer],
+                self.lr, self.dense_linear_opt(), ptr(self.table), ptr(self.accum) if adagrad else None,
+                self.row_stride, ptr(self.w1) if self.first_order else None,
+                ptr(self.w1_accum) if self.first_order else None,
+                ptr(self.lin_z) if (self.first_order and self.lin_z is not None) else None,
+                self.lin_stride, ptr(self.dense_shard_row), self.clip_norm,
+                self._n_unique2.data_ptr() + 8 * h.parity if self.plan.rank == 0 else None, st),
+                "dir_shard_dense_apply_clipped")
+            self.trace.mark("bwd.dense_apply")
 
     def finish_step(self, handle_a, handle_b):
         """After the backward of both micro-batches of a batch (run with `defer_update=True`): the one owner update

@@ -376,6 +376,34 @@ int dir_shard_dense_apply(const dir_peer_layout* layout, float* dense_table, flo
                           int64_t shard_row_stride, float* shard_lin, float* shard_lin_accum,
                           float* shard_lin_z, int64_t shard_lin_stride, const int64_t* shard_row,
                           const dir_peer_layout* layout_b, int64_t* n_unique_inout, dir_stream_t stream);
+/* tf.clip_by_norm of every column's gradient on the row-sharded tables (models/DeepCrossNetwork/DeepCrossNetwork.py:
+ * 282-289), one factor per column over its MERGED per-row sums (every rank's requests of a row added as the owner
+ * update adds them).  One buffer (one exchange buffer; no second micro-batch), after the grads barrier:
+ *   dir_shard_owner_sqnorms         per leading arrival (sum g^2, g1^2) in fp64 -> sq_scratch[G * seg_cap][2], then
+ *                                   per column and slice -> norm[rank][F][kClipSlices][2] of EVERY rank; norm_peers
+ *                                   is a device array of the G ranks' norm buffers ([G][F][16][2] doubles each)
+ *   ---- barrier ----
+ *   dir_shard_owner_update_clipped  partials[F][16][2] = sum over q of norm[q] in rank order (the same on every rank),
+ *                                   then the owner update with each merged sum scaled by clip / max(||G_f||, clip)
+ *                                   (the first-order sums by their own column factor)
+ *   dir_shard_dense_apply_clipped   the replicated one-row fields: each a column of one row, clipped by its own sum
+ * local_field_offset[F+1]: the first local row of each column on this rank (ascending), then n_local_rows.
+ * with_g1: the g1 sums are live (first-order weights trained).  SGD or Adagrad only (tables and replicas). */
+int dir_shard_owner_sqnorms(const dir_peer_layout* layout, const uint32_t* slot, const uint32_t* slot_epoch,
+                            int64_t n_local_rows, const int64_t* local_field_offset, int F, int with_g1,
+                            double* sq_scratch, const uint64_t* norm_peers, dir_stream_t stream);
+int dir_shard_owner_update_clipped(const dir_peer_layout* layout, const uint32_t* slot, float* table, float* accum,
+                                   int64_t row_stride, float* lin, float* lin_accum, int64_t lin_stride,
+                                   int64_t n_local_rows, const uint32_t* slot_epoch, int optimizer, float lr,
+                                   const dir_linear_opt* linear_opt, const int64_t* local_field_offset, int F,
+                                   const double* norm, double* partials, float clip_norm, int64_t* n_unique_inout,
+                                   dir_stream_t stream);
+int dir_shard_dense_apply_clipped(const dir_peer_layout* layout, float* dense_table, float* dense_accum,
+                                  int64_t row_stride, float* dense_lin, float* dense_lin_accum, int optimizer,
+                                  float lr, const dir_linear_opt* linear_opt, float* shard_table, float* shard_accum,
+                                  int64_t shard_row_stride, float* shard_lin, float* shard_lin_accum,
+                                  float* shard_lin_z, int64_t shard_lin_stride, const int64_t* shard_row,
+                                  float clip_norm, int64_t* n_unique_inout, dir_stream_t stream);
 /* cfg4-sized tables are filled on the device: value(global row, k) from a counter hash of (seed, row, k) --
  * a sum of four 16-bit uniforms, centred and scaled to standard deviation `sd` (|value| < 3.47 sd) -- so any row
  * can be reproduced on the host without the table (oracle/deepctr_oracle.counter_rows).  Fills
