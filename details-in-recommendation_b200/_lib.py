@@ -111,6 +111,9 @@ SIGNATURES = {
     "dir_shard_dense_apply_clipped": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int,
                                               c_float, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
                                               c_void_p, c_int64, c_void_p, c_float, c_void_p, c_void_p]),
+    "dir_shard_owner_apply_adam": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p,
+                                           c_void_p, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_float,
+                                           c_void_p, c_void_p, c_void_p]),
     "dir_table_init_counter": (c_int, [c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_int64, c_uint64, c_float,
                                        c_void_p]),
     "dir_embed_bag_fm_fwd": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p,

@@ -11,58 +11,26 @@
 // adding the gradient where the row has one.  The clip_by_norm factor of a column comes from dir_field_sqnorms'
 // partials exactly as in dir_rows_apply_clipped (clip.cu).  A row whose m and v are zero and that has no gradient
 // does not move (T - 0 / eps == T bit for bit), so its stores are skipped.
-#include "common.cuh"
-#include "update.cuh"
+#include "adam.cuh"
 
 namespace dir {
 
-constexpr int kAdamTile = 1024;        // table rows per tile (one shared-memory map of distinct-row indices)
-constexpr int kAdamThreads = 256;
-constexpr int kAdamUnroll = 2;         // float4 chunks each thread loads before it stores any
-
-// first u in [0, n) with a[u] >= key (a ascending), by one warp: 32 probes per round, so ~log32(n) rounds
-__device__ __forceinline__ int64_t warp_lower_bound(const uint32_t* __restrict__ a, int64_t n, uint64_t key) {
-  const int lane = threadIdx.x & 31;
-  int64_t lo = 0, hi = n;   // the answer lies in [lo, hi]
-  while (lo < hi) {
-    const int64_t step = (hi - lo + 31) / 32;
-    const int64_t p = lo + (int64_t)lane * step;
-    const bool less = p < hi && (uint64_t)__ldg(a + p) < key;
-    const int c = __popc(__ballot_sync(0xffffffffu, less));   // probes below key: a prefix of the lanes
-    if (c == 0) break;
-    const int64_t nhi = lo + (int64_t)c * step;
-    lo = lo + (int64_t)(c - 1) * step + 1;
-    hi = nhi < hi ? nhi : hi;
+// Src of adam_tile: the gradient of distinct row uu at gu + uu * gu_stride, clipped by its column's factor
+struct UniqueGrad {
+  const float* __restrict__ gu;
+  int64_t gu_stride;
+  bool clipped;
+  const int64_t* s_off;
+  int F;
+  float clip;
+  const float* s_den;
+  __device__ __forceinline__ float4 load(int uu, int sub, int64_t) const {
+    return __ldg(reinterpret_cast<const float4*>(gu + (int64_t)uu * gu_stride) + sub);
   }
-  return lo;
-}
-
-struct AdamStep {
-  float lr_t, b1, b2, omb1, omb2, eps;  // omb = 1 - beta, in fp32 as TF evaluates it
+  __device__ __forceinline__ void scale(float4& g, int64_t row) const {
+    if (clipped) clip4(g, clip, s_den[field_of(s_off, F, (uint64_t)row)]);
+  }
 };
-
-// one component: decay, add the gradient if the row has one, update T.  IEEE sqrt and divide; no contraction.
-__device__ __forceinline__ void adam1(float& t, float& m, float& v, float g, bool has_g, const AdamStep& s) {
-  m = __fmul_rn(m, s.b1);
-  v = __fmul_rn(v, s.b2);
-  if (has_g) {
-    m = __fadd_rn(m, __fmul_rn(g, s.omb1));
-    v = __fadd_rn(v, __fmul_rn(__fmul_rn(g, g), s.omb2));
-  }
-  t = __fsub_rn(t, __fdiv_rn(__fmul_rn(s.lr_t, m), __fadd_rn(__fsqrt_rn(v), s.eps)));
-}
-
-__device__ __forceinline__ bool zero4(const float4& a) { return a.x == 0.f && a.y == 0.f && a.z == 0.f && a.w == 0.f; }
-
-// last field whose offset <= row
-__device__ __forceinline__ int field_of(const int64_t* s_off, int F, uint64_t row) {
-  int lo = 0, hi = F;
-  while (hi - lo > 1) {
-    const int mid = (lo + hi) >> 1;
-    if ((uint64_t)s_off[mid] <= row) lo = mid; else hi = mid;
-  }
-  return lo;
-}
 
 template <int LPR>
 __global__ void __launch_bounds__(kAdamThreads, 4)
@@ -85,16 +53,7 @@ rows_apply_adam_kernel(float* table, int64_t row_stride, int64_t n_rows, float* 
     U = U < 0 ? 0 : (U > n_capacity ? n_capacity : U);
   }
   if (n_unique_out && blockIdx.x == 0 && threadIdx.x == 0) *n_unique_out = U;
-  AdamStep s;
-  {
-    const float p1 = beta_power[0], p2 = beta_power[1];
-    s.lr_t = __fdiv_rn(__fmul_rn(lr, __fsqrt_rn(__fsub_rn(1.f, p2))), __fsub_rn(1.f, p1));
-    s.b1 = b1;
-    s.b2 = b2;
-    s.omb1 = __fsub_rn(1.f, b1);
-    s.omb2 = __fsub_rn(1.f, b2);
-    s.eps = eps;
-  }
+  const AdamStep s = adam_step(lr, b1, b2, eps, beta_power);
   const int warp = threadIdx.x >> 5;
   const int64_t n_tiles = (n_rows + kAdamTile - 1) / kAdamTile;
   for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -109,49 +68,7 @@ rows_apply_adam_kernel(float* table, int64_t row_stride, int64_t n_rows, float* 
     const int64_t ulo = s_range[0], uhi = s_range[1];
     for (int64_t u = ulo + threadIdx.x; u < uhi; u += blockDim.x) s_map[__ldg(urows + u) - r0] = (int32_t)u;
     __syncthreads();
-    const int n_chunks = (int)(r1 - r0) * LPR;
-    for (int c0 = threadIdx.x; c0 < n_chunks; c0 += kAdamThreads * kAdamUnroll) {
-      float4 T[kAdamUnroll], M[kAdamUnroll], V[kAdamUnroll], G[kAdamUnroll];
-      int uu[kAdamUnroll];
-#pragma unroll
-      for (int j = 0; j < kAdamUnroll; ++j) {
-        const int c = c0 + j * kAdamThreads;
-        uu[j] = -1;
-        if (c < n_chunks) {
-          const int r = c / LPR, sub = c % LPR;
-          const float* p = table + (r0 + r) * row_stride + sub * 4;
-          T[j] = *reinterpret_cast<const float4*>(p);
-          M[j] = *reinterpret_cast<const float4*>(p + K);
-          V[j] = *reinterpret_cast<const float4*>(p + 2 * K);
-          uu[j] = s_map[r];
-          if (uu[j] >= 0) G[j] = __ldg(reinterpret_cast<const float4*>(gu + (int64_t)uu[j] * gu_stride) + sub);
-        }
-      }
-#pragma unroll
-      for (int j = 0; j < kAdamUnroll; ++j) {
-        const int c = c0 + j * kAdamThreads;
-        if (c >= n_chunks) continue;
-        const bool has_g = uu[j] >= 0;
-        if (!has_g && zero4(M[j]) && zero4(V[j])) continue;   // T, m, v stay as they are, bit for bit
-        const int r = c / LPR, sub = c % LPR;
-        float4 g = has_g ? G[j] : make_float4(0.f, 0.f, 0.f, 0.f);
-        if (has_g && clipped) {
-          const float den = s_den[field_of(s_off, F, (uint64_t)(r0 + r))];
-          g.x = clip1(g.x, clip, den);
-          g.y = clip1(g.y, clip, den);
-          g.z = clip1(g.z, clip, den);
-          g.w = clip1(g.w, clip, den);
-        }
-        adam1(T[j].x, M[j].x, V[j].x, g.x, has_g, s);
-        adam1(T[j].y, M[j].y, V[j].y, g.y, has_g, s);
-        adam1(T[j].z, M[j].z, V[j].z, g.z, has_g, s);
-        adam1(T[j].w, M[j].w, V[j].w, g.w, has_g, s);
-        float* p = table + (r0 + r) * row_stride + sub * 4;
-        *reinterpret_cast<float4*>(p) = T[j];
-        *reinterpret_cast<float4*>(p + K) = M[j];
-        *reinterpret_cast<float4*>(p + 2 * K) = V[j];
-      }
-    }
+    adam_tile<LPR>(table, row_stride, r0, r1, s_map, s, UniqueGrad{gu, gu_stride, clipped, s_off, F, clip, s_den});
     if (lin != nullptr) {                 // first-order weights of the tile's rows that have a gradient
       for (int64_t u = ulo + threadIdx.x; u < uhi; u += blockDim.x) {
         const uint64_t row = __ldg(urows + u);
@@ -171,6 +88,10 @@ rows_apply_adam_kernel(float* table, int64_t row_stride, int64_t n_rows, float* 
 __global__ void adam_advance_powers_kernel(float* beta_power, float b1, float b2) {
   beta_power[0] = __fmul_rn(beta_power[0], b1);
   beta_power[1] = __fmul_rn(beta_power[1], b2);
+}
+
+void adam_advance_powers(float* beta_power, float b1, float b2, cudaStream_t st) {
+  adam_advance_powers_kernel<<<1, 1, 0, st>>>(beta_power, b1, b2);
 }
 
 }  // namespace dir

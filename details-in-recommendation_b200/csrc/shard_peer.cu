@@ -31,6 +31,11 @@
 //                                                         order, the same update with each sum scaled
 //   dir_shard_dense_apply_clipped   replicated one-row fields, each clipped by its own sum
 //
+// With optimizer='adam' (TF's Adam decays every row's moments), the owner half after the grads barrier (and, with a
+// clip, the norm pass and its barrier) is one sweep; every field goes through the exchange (no replicated rows)
+//                                                       dir_shard_owner_apply_adam  every local row decayed, the
+//                                                         requesters' sums merged in rank order where a row has them
+//
 // The owner never sorts: a requester sends each row at most once, so slot[row][q] (one cell per local row and
 // requester, written without atomics) tells an arrival whether an earlier rank asked for the same row; the first
 // one merges.  Deterministic: no floating-point atomics, sums in rank order.  A cell is (epoch << 24) | (i + 1) and
@@ -39,8 +44,7 @@
 //
 // Reference: the partitioner hook around the embedding variables, models/DeepFM/deepFM.py:163-175 (under a TF
 // parameter-server cluster the variables are sharded by row and ids / IndexedSlices travel over gRPC).
-#include "common.cuh"
-#include "update.cuh"
+#include "adam.cuh"
 
 namespace dir {
 
@@ -574,6 +578,118 @@ peer_clip_combine_kernel(const double* __restrict__ norm, int G, int64_t n, doub
   part[x] = v;
 }
 
+// ---- TF's Adam on the owner (dir_shard_owner_apply_adam)
+// _apply_sparse_shared decays the moments of every row, so the owner sweeps its whole shard in tiles of kAdamTile local
+// rows, with adam.cu's tile body.  A tile's gradients come from the requesters' id segments, not from the slot map:
+// each segment is strictly ascending in local row (the norm pass relies on it too), so per requester q two warp
+// lower_bounds find q's arrivals in [r0, r1), and each arrival i stores (q << 24) | i into the tile's map with an
+// integer atomicMin: the lowest requester that asked for a row leads it, the leader rule of peer_owner_update_kernel.
+// (2G searches per tile; reading the slot map densely would cost 4G bytes for every row.)  The merged sum starts from
+// the leader's and adds the later requesters whose slot cell carries the current epoch, in rank order with __fadd_rn:
+// the sum peer_owner_update_kernel applies and peer_owner_sqnorm_kernel squares, bit for bit.
+template <int LPR>
+struct PeerMergedGrad {
+  const float4* gb;    // the exchange buffer's g [G][seg_cap][K]
+  const float* g1b;    // and g1 [G][seg_cap]
+  const uint32_t* slot;
+  int64_t seg_cap;
+  uint32_t tag;
+  int G;
+  bool clipped;
+  const int64_t* s_off;
+  int F;
+  float clip;
+  const float* s_den;
+  __device__ __forceinline__ float4 load(int key, int sub, int64_t row) const {
+    const int q = key >> 24;
+    float4 g = __ldg(gb + ((int64_t)q * seg_cap + (key & 0xffffff)) * LPR + sub);
+    for (int p = q + 1; p < G; ++p) {
+      const uint32_t c = __ldg(slot + row * G + p);
+      if ((c >> 24) != tag) continue;
+      const float4 o = __ldg(gb + ((int64_t)p * seg_cap + ((c & 0xffffffu) - 1u)) * LPR + sub);
+      g.x = __fadd_rn(g.x, o.x);
+      g.y = __fadd_rn(g.y, o.y);
+      g.z = __fadd_rn(g.z, o.z);
+      g.w = __fadd_rn(g.w, o.w);
+    }
+    return g;
+  }
+  __device__ __forceinline__ float load_g1(int key, int64_t row) const {
+    const int q = key >> 24;
+    float g1 = __ldg(g1b + (int64_t)q * seg_cap + (key & 0xffffff));
+    for (int p = q + 1; p < G; ++p) {
+      const uint32_t c = __ldg(slot + row * G + p);
+      if ((c >> 24) == tag) g1 = __fadd_rn(g1, __ldg(g1b + (int64_t)p * seg_cap + ((c & 0xffffffu) - 1u)));
+    }
+    return g1;
+  }
+  __device__ __forceinline__ void scale(float4& g, int64_t row) const {
+    if (clipped) clip4(g, clip, s_den[field_of(s_off, F, (uint64_t)row)]);
+  }
+};
+
+template <int LPR>
+__global__ void __launch_bounds__(kAdamThreads, 4)
+peer_owner_adam_kernel(const dir_peer_layout L, const uint32_t* __restrict__ slot, const uint32_t* __restrict__ epoch,
+                       float* table, int64_t row_stride, int64_t n_local, float* lin, float* lin_accum,
+                       int64_t lin_stride, const LinOpt lo, const int64_t* __restrict__ field_offset, int F,
+                       const double* __restrict__ part, float clip, float lr, float b1, float b2, float eps,
+                       const float* __restrict__ beta_power, unsigned long long* n_unique) {
+  __shared__ int32_t s_map[kAdamTile];
+  __shared__ Arrivals s;
+  __shared__ int64_t s_lo[kMaxG], s_hi[kMaxG];
+  ClipSmem& cs = clip_smem();
+  const bool clipped = part != nullptr;
+  if (clipped) clip_denominators(part, field_offset, F, clip, cs.off, cs.den, cs.den1);
+  load_arrivals(L, s);                    // (its barrier also publishes the clip factors)
+  const AdamStep st = adam_step(lr, b1, b2, eps, beta_power);
+  const int G = L.G;
+  const int32_t* ids = reinterpret_cast<const int32_t*>(L.local + L.off_ids);
+  const PeerMergedGrad<LPR> src{reinterpret_cast<const float4*>(L.local + L.off_g),
+                                reinterpret_cast<const float*>(L.local + L.off_g1), slot, L.seg_cap, epoch[0], G,
+                                clipped, cs.off, F, clip, cs.den};
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  unsigned long long leaders = 0;
+  const int64_t n_tiles = (n_local + kAdamTile - 1) / kAdamTile;
+  for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const int64_t r0 = tile * kAdamTile;
+    const int64_t r1 = r0 + kAdamTile < n_local ? r0 + kAdamTile : n_local;
+    for (int t = warp; t < 2 * G; t += kAdamThreads / 32) {   // requester t / 2: first arrival >= r0 (t even), >= r1
+      const int q = t >> 1;
+      const int64_t b = warp_lower_bound(reinterpret_cast<const uint32_t*>(ids + (int64_t)q * L.seg_cap),
+                                         s.pre[q + 1] - s.pre[q], (uint64_t)((t & 1) ? r1 : r0));
+      if (lane == 0) ((t & 1) ? s_hi : s_lo)[q] = b;
+    }
+    for (int i = threadIdx.x; i < kAdamTile; i += blockDim.x) s_map[i] = -1;
+    __syncthreads();
+    for (int q = 0; q < G; ++q) {
+      const int32_t* seg = ids + (int64_t)q * L.seg_cap;
+      for (int64_t i = s_lo[q] + threadIdx.x; i < s_hi[q]; i += blockDim.x)
+        atomicMin(reinterpret_cast<unsigned*>(s_map) + (__ldg(seg + i) - r0), ((unsigned)q << 24) | (unsigned)i);
+    }
+    __syncthreads();
+    adam_tile<LPR>(table, row_stride, r0, r1, s_map, st, src);
+    for (int i = threadIdx.x; i < (int)(r1 - r0); i += blockDim.x) {
+      const int key = s_map[i];
+      if (key < 0) continue;
+      ++leaders;
+      if (lin != nullptr) {               // first-order weights: the leader's merged g1 through the linear rule
+        const int64_t row = r0 + i;
+        float g1 = src.load_g1(key, row);
+        if (clipped) g1 = clip1(g1, clip, cs.den1[field_of(cs.off, F, (uint64_t)row)]);
+        const int64_t off = row * lin_stride;
+        float n1, z1;
+        lin_load(lo, lin_accum, off, n1, z1);
+        lin_apply(lo, lin + off, lin_accum + off, lo.z + off, lin[off], n1, z1, g1);
+      }
+    }
+    __syncthreads();                      // s_map / s_lo / s_hi are rewritten by the next tile
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) leaders += __shfl_xor_sync(0xffffffffu, leaders, o);
+  if (lane == 0 && leaders && n_unique) atomicAdd(n_unique, leaders);
+}
+
 // replicated one-row fields: the G ranks' sums added in rank order, the same update applied to every replica;
 // shard_row[j] >= 0 names the row of the sharded table to mirror into (on the rank that owns it)
 struct DenseApplyArgs {
@@ -994,4 +1110,68 @@ extern "C" int dir_shard_dense_apply_clipped(const dir_peer_layout* layout, floa
                      dense_lin_accum, optimizer, lr, nullptr, linear_opt, shard_table, shard_accum, shard_row_stride,
                      shard_lin, shard_lin_accum, shard_lin_z, shard_lin_stride, shard_row, nullptr, n_unique_inout,
                      clip_norm, static_cast<cudaStream_t>(stream));
+}
+
+// ---- TF's Adam on the owner (see peer_owner_adam_kernel)
+extern "C" int dir_shard_owner_apply_adam(const dir_peer_layout* layout, const uint32_t* slot, const uint32_t* slot_epoch,
+                                          float* table, int64_t row_stride, int64_t n_local_rows, float* lin,
+                                          float* lin_accum, int64_t lin_stride, const dir_linear_opt* linear_opt,
+                                          const int64_t* local_field_offset, int F, const double* norm,
+                                          double* partials, float clip_norm, const dir_adam_opt* adam,
+                                          int64_t* n_unique_inout, dir_stream_t stream) {
+  using namespace dir;
+  if (int rc = check_layout("shard_owner_apply_adam", layout)) return rc;
+  const int K = layout->K;
+  if (layout->n_dense != 0)
+    return fail(DIR_EINVAL, "shard_owner_apply_adam: n_dense must be 0 (under Adam every field goes through the exchange)");
+  if (layout->seg_cap >= (1 << 24)) return fail(DIR_EINVAL, "shard_owner_apply_adam: seg_cap must be < 2^24");
+  if (!slot || !slot_epoch) return fail(DIR_EINVAL, "shard_owner_apply_adam: slot and slot_epoch are required");
+  if (n_local_rows <= 0 || n_local_rows >= 0xffffffffLL)
+    return fail(DIR_EINVAL, "shard_owner_apply_adam: 0 < n_local_rows < 2^32 - 1 required");
+  if (!table || row_stride < 3 * K || (row_stride & 3) || !aligned16(table))
+    return fail(DIR_EINVAL, "shard_owner_apply_adam: rows are [T | m | v]: row_stride >= 3K, a multiple of 4, table "
+                            "16-byte aligned");
+  if (!adam || !adam->beta_power) return fail(DIR_EINVAL, "shard_owner_apply_adam: adam and its beta_power are required");
+  if (!(adam->lr > 0.f)) return fail(DIR_EINVAL, "shard_owner_apply_adam: lr must be > 0");
+  if (!(adam->beta1 >= 0.f && adam->beta1 < 1.f) || !(adam->beta2 >= 0.f && adam->beta2 < 1.f))
+    return fail(DIR_EINVAL, "shard_owner_apply_adam: 0 <= beta1, beta2 < 1 required");
+  if (!(adam->epsilon > 0.f)) return fail(DIR_EINVAL, "shard_owner_apply_adam: epsilon must be > 0");
+  if (norm) {
+    if (F <= 0 || F > kClipMaxFields) return fail(DIR_EINVAL, "shard_owner_apply_adam: 0 < F <= 1024 required");
+    if (!local_field_offset) return fail(DIR_EINVAL, "shard_owner_apply_adam: the clip needs local_field_offset");
+    if (!partials) return fail(DIR_EINVAL, "shard_owner_apply_adam: the clip needs partials");
+    if (!(clip_norm > 0.f)) return fail(DIR_EINVAL, "shard_owner_apply_adam: clip_norm must be > 0");
+  }
+  LinOpt lo{DIR_OPT_SGD, 0.f, 0.f, 0.f, nullptr};
+  if (lin != nullptr) {
+    if (!linear_opt)
+      return fail(DIR_EINVAL, "shard_owner_apply_adam: lin needs linear_opt (Adam does not train first-order weights)");
+    if (int rc = resolve_lin("shard_owner_apply_adam", linear_opt, DIR_OPT_SGD, 0.f, lin, lin_accum, lo)) return rc;
+    if (lin_stride < 1) return fail(DIR_EINVAL, "shard_owner_apply_adam: lin_stride must be >= 1");
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (norm) {                             // the rank-order combine of dir_shard_owner_update_clipped
+    const int64_t n = (int64_t)F * kClipSlices * 2;
+    peer_clip_combine_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(norm, layout->G, n, partials);
+  }
+  const int64_t n_tiles = (n_local_rows + kAdamTile - 1) / kAdamTile;
+  const unsigned grid = (unsigned)(n_tiles < (int64_t)kSMs * 4 ? n_tiles : (int64_t)kSMs * 4);
+  const double* part = norm ? partials : nullptr;
+  unsigned long long* nu = reinterpret_cast<unsigned long long*>(n_unique_inout);
+  const float b1 = adam->beta1, b2 = adam->beta2;
+#define DIR_OA(LP)                                                                                                  \
+  peer_owner_adam_kernel<LP><<<grid, kAdamThreads, 0, st>>>(*layout, slot, slot_epoch, table, row_stride,          \
+                                                            n_local_rows, lin, lin_accum, lin_stride, lo,           \
+                                                            local_field_offset, F, part, clip_norm, adam->lr, b1,   \
+                                                            b2, adam->epsilon, adam->beta_power, nu)
+  switch (K / 4) {
+    case 1: DIR_OA(1); break;
+    case 2: DIR_OA(2); break;
+    case 4: DIR_OA(4); break;
+    case 8: DIR_OA(8); break;
+    default: DIR_OA(16); break;
+  }
+#undef DIR_OA
+  adam_advance_powers(adam->beta_power, b1, b2, st);
+  return launched("shard_owner_apply_adam", norm ? 3 : 2);
 }

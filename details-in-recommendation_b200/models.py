@@ -195,8 +195,10 @@ class DCN(torch.nn.Module):
     column's norm over the merged sums of the global batch, reduced across ranks on the device); by default it
     applies them unclipped, as it always has.
     optimizer='adam' is the reference's own (train.py:104-124, epsilon = adam_epsilon = 1e-4): TF's Adam on the
-    tables (`EmbeddingFM(optimizer='adam')`, every row's moments decay at every step) and `TFAdam` on the dense
-    parameters.  Single-GPU layer only.
+    tables (`EmbeddingFM(optimizer='adam')`, or `ShardedEmbeddingFM(optimizer='adam')` with sharded=True, where each
+    owner sweeps its own shard; every row's moments decay at every step) and `TFAdam` on the dense parameters.  With
+    sharded=True and clip_sharded_tables=True that is the reference's full rule across GPUs: every column's table
+    gradient clipped, then Adam.
     """
 
     def __init__(self, field_size: int, embedding_size: int, rows_per_field: Sequence[int],
@@ -211,8 +213,6 @@ class DCN(torch.nn.Module):
         if clip_norm and (clip_sharded_tables or not sharded):
             layer_kw = dict(layer_kw, clip_norm=clip_norm)      # every column's gradient is clipped too (:284)
         if self.optimizer == "adam":
-            if sharded:
-                raise ValueError("DCN(optimizer='adam') needs the single-GPU layer (sharded=False)")
             layer_kw = dict(layer_kw, optimizer_epsilon=self.adam_epsilon)
         self.embedding = _embedding_layer(sharded, field_size, embedding_size, list(rows_per_field), optimizer=optimizer,
                                           lr=learning_rate, first_order=False, device=device, **layer_kw)

@@ -40,6 +40,20 @@ def adam_apply_bytes(n_rows, K, U, first_order=False, linear_optimizer=None):
     return n_rows * 3 * R * 2 + U * (4 + R) + lin
 
 
+def shard_adam_apply_bytes(n_local, K, arrivals, G, U=None, first_order=False, linear_optimizer=None):
+    """dir_shard_owner_apply_adam on one owner: the sweep reads and writes all n_local rows [T | m | v] (3R each way);
+    each of the `arrivals` (every requester's distinct rows that reached this owner) costs its id (4 B, the tile map),
+    its gradient sum (R) and its row's slot cells (4G, the rank-order merge).  With first-order weights, per distinct
+    row U (default: arrivals) its g1 (4 B) and the weight's state as adam_apply_bytes counts it."""
+    R = 4 * K
+    U = arrivals if U is None else U
+    lin = 0
+    if first_order:
+        c = 2 if linear_optimizer == "sgd" else 4
+        lin = arrivals * 4 + U * (4 * c + (8 if linear_optimizer == "ftrl" else 0))
+    return n_local * 3 * R * 2 + arrivals * (4 + R + 4 * G) + lin
+
+
 def cross_fwd_bytes(B, d, L):
     return 2 * B * d * 4 + 2 * L * d * 4
 

@@ -27,8 +27,8 @@ import torch.distributed as dist
 
 from . import _lib
 from ._lib import check, ptr
-from .layers import (_CLIP_MAX_FIELDS, _K_OK, _TABLE_OPTIMIZERS, _Workspace, _need_cuda, _stream,
-                     linear_opt_struct, table_opt_struct, resolve_linear_optimizer)
+from .layers import (_CLIP_MAX_FIELDS, _K_OK, _LINEAR_OPTIMIZERS, _TABLE_OPTIMIZERS, _Workspace, _need_cuda,
+                     _stream, linear_opt_struct, table_opt_struct, resolve_linear_optimizer)
 
 
 class ShardPlan:
@@ -323,7 +323,18 @@ class ShardedEmbeddingFM(torch.nn.Module):
     clip_norm: tf.clip_by_norm of every column's gradient before the update, as `EmbeddingFM(clip_norm=...)` applies it
     (DeepCrossNetwork.py:282-289): one factor per column, over the column's per-row sums of the GLOBAL batch (every
     rank's requests of a row merged).  Each owner reduces its rows per column and the ranks exchange the partials
-    (a few KB) over peer memory, so the step still replays from one CUDA graph.  SGD / Adagrad, one micro-batch.
+    (a few KB) over peer memory, so the step still replays from one CUDA graph.  SGD / Adagrad / Adam, one
+    micro-batch.
+
+    optimizer='adam': [TF] tf.train.AdamOptimizer(lr, optimizer_beta1, optimizer_beta2, optimizer_epsilon) on the
+    tables, as `EmbeddingFM(optimizer='adam')` applies it (the reference's DCN optimizer,
+    models/DeepCrossNetwork/train.py:104-124).  TF's sparse apply decays the moments of EVERY row, so after the grads
+    barrier each owner sweeps its whole shard ([T | m | v] per row, `adam_m` / `adam_v`), adding the requesters'
+    merged sums where a row has them; the beta powers live on the device (`beta_power`, the same on every rank).  The
+    sweep runs every step, also when this rank's batch had no surviving lookup.  Every field goes through the
+    exchange: `replicate_onerow` is ignored under Adam (a replicated one-row field would need an Adam step of its
+    own, kept in step with the owner's sweep).  Adam does not train the first-order weights: with first_order=True a
+    linear_optimizer must be named.  One micro-batch.
     """
 
     def __init__(self, field_size: int, embedding_size: int, rows_per_field: Sequence[int],
@@ -333,11 +344,30 @@ class ShardedEmbeddingFM(torch.nn.Module):
                  linear_lr: Optional[float] = None, l1_regularization_strength: float = 0.0,
                  l2_regularization_strength: float = 0.0, init: str = "trunc_normal", micro_batches: int = 1,
                  replicate_onerow: bool = True, max_entries: Optional[int] = None, optimizer_l1: float = 0.0,
-                 optimizer_l2: float = 0.0, clip_norm: Optional[float] = None, device="cuda"):
+                 optimizer_l2: float = 0.0, clip_norm: Optional[float] = None, device="cuda",
+                 optimizer_beta1: float = 0.9, optimizer_beta2: float = 0.999, optimizer_epsilon: float = 1e-8):
         super().__init__()
         if micro_batches not in (1, 2):
             raise ValueError("micro_batches must be 1 or 2")
         self.micro_batches = int(micro_batches)
+        adam = str(optimizer).lower() == "adam"     # kept out of _TABLE_OPTIMIZERS, as in layers.py
+        if adam:
+            if self.micro_batches != 1:
+                # the owner's sweep reads one exchange buffer
+                raise ValueError("optimizer='adam' needs micro_batches=1")
+            if not lr > 0:
+                raise ValueError("adam needs lr > 0")
+            if not (0 <= optimizer_beta1 < 1 and 0 <= optimizer_beta2 < 1):
+                raise ValueError("optimizer_beta1 / optimizer_beta2 must be in [0, 1)")
+            if not optimizer_epsilon > 0:
+                raise ValueError("optimizer_epsilon must be > 0")
+            if first_order and linear_optimizer is None:
+                raise ValueError("Adam does not train first-order weights: name a linear_optimizer "
+                                 "(%s) or pass first_order=False" % ", ".join(sorted(_LINEAR_OPTIMIZERS)))
+            if linear_optimizer is None:
+                linear_lr = None
+        self.optimizer_beta1, self.optimizer_beta2 = float(optimizer_beta1), float(optimizer_beta2)
+        self.optimizer_epsilon = float(optimizer_epsilon)
         if clip_norm is not None and not clip_norm > 0:
             raise ValueError("clip_norm must be > 0 (or None)")
         self.clip_norm = None if clip_norm is None else float(clip_norm)
@@ -355,8 +385,8 @@ class ShardedEmbeddingFM(torch.nn.Module):
         if embedding_size not in _K_OK:
             raise ValueError("embedding_size must be one of %r" % (_K_OK,))
         optimizer = optimizer.lower()
-        if optimizer not in _TABLE_OPTIMIZERS:
-            raise ValueError("optimizer must be 'adagrad', 'sgd' or 'proximal_adagrad'")
+        if optimizer not in _TABLE_OPTIMIZERS and not adam:
+            raise ValueError("optimizer must be 'adagrad', 'sgd', 'proximal_adagrad' or 'adam'")
         self.optimizer_l1, self.optimizer_l2 = float(optimizer_l1), float(optimizer_l2)
         if self.optimizer_l1 < 0 or self.optimizer_l2 < 0:
             raise ValueError("optimizer_l1 / optimizer_l2 must be >= 0")
@@ -376,8 +406,8 @@ class ShardedEmbeddingFM(torch.nn.Module):
         self.optimizer, self.lr = optimizer, float(lr)
         self.first_order, self.emit_embeddings, self.check_bounds = first_order, emit_embeddings, check_bounds
         K = embedding_size
-        adagrad = optimizer != "sgd"                                # the rule keeps an accumulator next to the row
-        self.row_stride = 2 * K if adagrad else K
+        adagrad = optimizer not in ("sgd", "adam")                  # the rule keeps an accumulator next to the row
+        self.row_stride = 3 * K if adam else (2 * K if adagrad else K)
         self.lin_stride = 1
         self.n_rows = max(self.plan.cap, 1)                         # local rows allocated
         self.max_batch = int(max_batch)
@@ -392,6 +422,9 @@ class ShardedEmbeddingFM(torch.nn.Module):
         self.register_buffer("lin_z", torch.zeros((cap, 1), dtype=torch.float32, device=dev) if lin_needs_z else None)
         self.register_buffer("oob_flag", torch.zeros(1, dtype=torch.int32, device=dev))
         self.register_buffer("err_flag", torch.zeros(1, dtype=torch.int32, device=dev))
+        # Adam's (beta1_power, beta2_power), advanced on the device by every owner sweep (every rank, every step)
+        self.register_buffer("beta_power", torch.tensor([optimizer_beta1, optimizer_beta2], dtype=torch.float32,
+                                                        device=dev) if adam else None)
         self.bias = torch.nn.Parameter(torch.zeros(1, dtype=torch.float32, device=dev))
         self._anchor = torch.nn.Parameter(torch.zeros(1, dtype=torch.float32, device=dev))
         self._n_unique2 = torch.zeros(2, dtype=torch.int64, device=dev)   # per exchange buffer: rows the owner updated
@@ -410,7 +443,7 @@ class ShardedEmbeddingFM(torch.nn.Module):
             raise ValueError("the peer-memory exchange needs the nccl backend (one process per GPU)")
         # One-row (numeric) fields are replicated parameters: every sample of every rank hits the same row, so they
         # stay out of the sort and the exchange; their gradients are column sums.
-        onerow = [f for f, r in enumerate(rows) if r == 1][:64] if replicate_onerow else []
+        onerow = [f for f, r in enumerate(rows) if r == 1][:64] if replicate_onerow and not adam else []
         sparse = [f for f in range(field_size) if f not in set(onerow)]
         self.n_dense, self.n_sel = len(onerow), len(sparse)
         self.register_buffer("onerow_fields", torch.tensor(onerow or [0], dtype=torch.int32, device=dev))
@@ -448,6 +481,8 @@ class ShardedEmbeddingFM(torch.nn.Module):
                 self.init_counter(seed=1236, sd=sd)
             if adagrad:
                 self.accum.fill_(initial_accumulator_value)
+            if adam:
+                self.rows[:, K:].zero_()
             if self.lin_acc is not None:
                 self.lin_acc.fill_(initial_accumulator_value)
         if self.n_dense:
@@ -459,7 +494,17 @@ class ShardedEmbeddingFM(torch.nn.Module):
 
     @property
     def accum(self):
-        return self.rows[:, self.embedding_size:] if self.optimizer != "sgd" else None
+        return self.rows[:, self.embedding_size:] if self.optimizer not in ("sgd", "adam") else None
+
+    @property
+    def adam_m(self):
+        K = self.embedding_size
+        return self.rows[:, K:2 * K] if self.optimizer == "adam" else None
+
+    @property
+    def adam_v(self):
+        K = self.embedding_size
+        return self.rows[:, 2 * K:3 * K] if self.optimizer == "adam" else None
 
     @property
     def w1(self):
@@ -625,6 +670,9 @@ class ShardedEmbeddingFM(torch.nn.Module):
         adagrad = self.optimizer != "sgd"
         px.barrier(handles[-1].buf, 0)
         tr.mark("bwd.barrier")
+        if self.optimizer == "adam":
+            self._owner_step_adam(h0)
+            return
         if self.clip_norm is not None:
             self._owner_step_clipped(h0)
             return
@@ -652,6 +700,33 @@ class ShardedEmbeddingFM(torch.nn.Module):
                 self._n_unique2.data_ptr() + 8 * h0.parity if self.plan.rank == 0 else None, st),
                 "dir_shard_dense_apply")
             tr.mark("bwd.dense_apply")
+
+    def _owner_step_adam(self, h):
+        """TF's Adam (one exchange buffer): with clip_norm the norm pass and its barrier first, as in
+        `_owner_step_clipped`; then one sweep of this rank's shard that decays every row, adds the merged (clipped) sums
+        and advances `beta_power`."""
+        L = _lib.lib()
+        st = _stream()
+        px, p, F = self.px, h.buf, self.field_size
+        clip = self.clip_norm is not None
+        if clip:
+            check(L.dir_shard_owner_sqnorms(px.ref(p), ptr(self.slot[p]), ptr(self.slot_epoch[p]), self.n_rows,
+                                            ptr(self.local_field_offset), F, int(self.first_order), ptr(self._clip_sq),
+                                            ptr(px.norm_peers[p]), st), "dir_shard_owner_sqnorms")
+            self.trace.mark("bwd.sqnorms")
+            px.norm_barrier(p)
+            self.trace.mark("bwd.norm_barrier")
+        opt = _lib.AdamOpt(self.lr, self.optimizer_beta1, self.optimizer_beta2, self.optimizer_epsilon,
+                           self.beta_power.data_ptr())
+        check(L.dir_shard_owner_apply_adam(
+            px.ref(p), ptr(self.slot[p]), ptr(self.slot_epoch[p]), ptr(self.rows), self.row_stride, self.n_rows,
+            ptr(self.w1) if self.first_order else None, ptr(self.w1_accum) if self.first_order else None,
+            self.lin_stride, linear_opt_struct(self), ptr(self.local_field_offset) if clip else None, F,
+            ptr(px.norm_bufs[p]) if clip else None, ptr(self.clip_partials) if clip else None,
+            self.clip_norm if clip else 0.0, _lib.ctypes.byref(opt), self._n_unique2.data_ptr() + 8 * h.parity, st),
+            "dir_shard_owner_apply_adam")
+        self._last_parity = h.parity
+        self.trace.mark("bwd.owner_adam")
 
     def _owner_step_clipped(self, h):
         """tf.clip_by_norm per column (one exchange buffer): the owner's per-column partials of the merged sums to every
@@ -955,6 +1030,9 @@ class ShardedEmbeddingBagFM(ShardedEmbeddingFM):
             raise ValueError("combiner must be 'sum', 'mean' or 'sqrtn'")
         if kw.get("micro_batches", 1) != 1:
             raise ValueError("ShardedEmbeddingBagFM exchanges a batch in one piece: micro_batches must be 1")
+        if str(kw.get("optimizer", "adagrad")).lower() == "adam":
+            raise ValueError("ShardedEmbeddingBagFM does not train with adam (nor does EmbeddingBagFM): adam is an "
+                             "EmbeddingFM / ShardedEmbeddingFM option")
         super().__init__(field_size, embedding_size, rows_per_field, replicate_onerow=False,
                          max_entries=max_entries, **kw)
         self.combiner = combiner

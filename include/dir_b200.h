@@ -404,6 +404,29 @@ int dir_shard_dense_apply_clipped(const dir_peer_layout* layout, float* dense_ta
                                   int64_t shard_row_stride, float* shard_lin, float* shard_lin_accum,
                                   float* shard_lin_z, int64_t shard_lin_stride, const int64_t* shard_row,
                                   float clip_norm, int64_t* n_unique_inout, dir_stream_t stream);
+/* [TF] tf.train.AdamOptimizer on the row-sharded tables (models/DeepCrossNetwork/train.py:104-124, after
+ * clip_by_norm(., 100) of DeepCrossNetwork.py:282-289): Adam._apply_sparse_shared on this rank's shard, then
+ * Adam._finish -- dir_rows_apply_adam's step and arithmetic, with the merged sums of every requester as the gradient.
+ * After the grads barrier (and, with a clip, dir_shard_owner_sqnorms + its barrier), one sweep of all n_local_rows
+ * rows [T(K) | m(K) | v(K)] (row_stride >= 3K): every row decays, a row that some requester asked for adds the
+ * requesters' sums merged in rank order (the leader rule and order of dir_shard_owner_update, so the sum is the one
+ * the norm pass squared), rows with zero m and v and no gradient are left unwritten.  Run it every step, also when no
+ * lookup of this rank's batch survived: TF's Adam steps every row.
+ *   norm (NULL = no clip): this step's norm buffer; partials[F][16][2] receives the rank-order combine (as in
+ *   dir_shard_owner_update_clipped) and every merged sum is scaled by its column's clip_by_norm factor, looked up
+ *   from local_field_offset[F+1]
+ *   lin (may be NULL): first-order weights of the rows with a gradient, stepped by linear_opt (required with lin:
+ *   Adam does not train first-order weights) with the merged, clipped g1
+ *   adam->beta_power: DEVICE float[2], read by the sweep and advanced after it on the same stream
+ *   n_unique_inout (may be NULL) += local rows that had a gradient
+ * layout->n_dense must be 0 (under Adam every field goes through the exchange); seg_cap < 2^24.  Deterministic: no
+ * floating-point atomics, independent of the grid; one buffer (no second micro-batch). */
+int dir_shard_owner_apply_adam(const dir_peer_layout* layout, const uint32_t* slot, const uint32_t* slot_epoch,
+                               float* table, int64_t row_stride, int64_t n_local_rows, float* lin, float* lin_accum,
+                               int64_t lin_stride, const dir_linear_opt* linear_opt,
+                               const int64_t* local_field_offset, int F, const double* norm, double* partials,
+                               float clip_norm, const dir_adam_opt* adam, int64_t* n_unique_inout,
+                               dir_stream_t stream);
 /* cfg4-sized tables are filled on the device: value(global row, k) from a counter hash of (seed, row, k) --
  * a sum of four 16-bit uniforms, centred and scaled to standard deviation `sd` (|value| < 3.47 sd) -- so any row
  * can be reproduced on the host without the table (oracle/deepctr_oracle.counter_rows).  Fills
